@@ -25,6 +25,9 @@ Prints ONE JSON line (rank 0):
                the planes into a reused text ring), the reference's default call shape (ragged rows, host API), configs[4] (custom vocab,
                long documents, cold and warm)
 `--impl reference` times the reference itself (Pool over all cores) on a bounded sample of the same workload.
+`--dump-outputs DIR` writes what the last timed step left in the output planes (its last chunk) as DIR/<plane>.npy, float32:
+a fixed, seeded sample of DUMP_ROWS rows, with their global pair indices in DIR/pair_index.npy (float64), so that two builds
+can be compared output for output on the same arguments.
 """
 import argparse
 import hashlib
@@ -47,6 +50,8 @@ LO, HI = 3, 13
 NOMINAL_HBM_GBS = 8000.0          # north_star's figure; the measured copy bandwidth is the other denominator (SURVEY.md 8 d3)
 REF_SAMPLE_PAIRS = 40960           # --impl reference: pairs per step (the first pairs of the global batch)
 L2_FLUSH_BYTES = 256 << 20
+DUMP_ROWS = 16384                  # --dump-outputs: 16,384 rows x 256 x 3 planes x 4 B = 48 MiB of float32, under 64 MB in all
+DUMP_SEED = 20240601
 
 
 def env_int(name, default):
@@ -296,6 +301,19 @@ class Stream:
         return tot
 
 
+def dump_outputs(out, row0, path, max_rows=DUMP_ROWS):
+    """A fixed, seeded sample of the rows of the planes `out` (rows row0 ... of the batch) -> path/<plane>.npy as float32 (every
+    value is an integer below 2^24), and path/pair_index.npy (float64): the global pair index of each sampled row."""
+    import torch
+    m = out["input_ids"].shape[0]
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(m, size=min(m, max_rows), replace=False))
+    idx = torch.from_numpy(rows).to(out["input_ids"].device)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "pair_index.npy"), (row0 + rows).astype(np.float64))
+    for name, plane in out.items():
+        np.save(os.path.join(path, name + ".npy"), plane.index_select(0, idx).cpu().numpy().astype(np.float32))
+
+
 def timed_passes(torch, fn, reps):
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(reps)]
     for a, b in ev:
@@ -332,7 +350,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extras", action="store_true", help="skip configs[1] / [3] / [4] side measurements")
     ap.add_argument("--no-arms", action="store_true", help="skip the cold / noise arms")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a sample of the planes of the last timed step to DIR/<plane>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
     if args.impl == "reference":
         run_reference(args, rank, world)
@@ -407,6 +430,8 @@ def main():
     launches = tok.launch_count() - launches0
     dev_ms = float(sum(step_ms))
     tok.check_errors(dev)
+    if args.dump_outputs and rank == 0:                              # before anything else overwrites the reused planes
+        dump_outputs(S.calls[-1][2], d0 + S.calls[-1][5], args.dump_outputs)
 
     # ---- per-kernel durations (library-side CUDA events on the launching stream), outside the timed region ---------------
     prof_chunks = list(range(min(n_chunks, 8)))
@@ -749,4 +774,5 @@ def run_extras(torch, tok, S, dev, peak, workload, Tokenize):
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True       # the tree this runs from may be read-only, and a run leaves nothing in it
     main()

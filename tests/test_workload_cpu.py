@@ -53,11 +53,11 @@ def test_plane_digest_is_order_independent_and_sensitive():
 
 
 def test_oracle_ref_recipe_and_oracle_agree_on_the_bench_workload(oracle):
-    """oracle/_ref (the unmodified reference, made by oracle/make_ref.py where /root/reference exists) against the C oracle on
-    noisy pairs of the bench workload."""
-    from oracle import make_ref, ref_pool
-    if make_ref.make(quiet=True) is None:
-        pytest.skip("no reference checkout and no oracle/_ref here")
+    """oracle/_ref (the unmodified reference, copied there from a reference checkout by oracle/make_ref.py) against the C oracle
+    on noisy pairs of the bench workload."""
+    from oracle import ref_pool
+    if not ref_pool.available():
+        pytest.skip("oracle/_ref is absent: run oracle/make_ref.py --ref <reference checkout>")
     n, W = 1500, 40
     ta, tb = workload.generate_hashed(3, 0, n, 0, 3, 13, 0.05), workload.generate_hashed(3, 0, n, 1, 3, 13, 0.05)
     rows = ref_pool.encode_rows_single(workload.unpack(*ta), workload.unpack(*tb), W)
@@ -69,6 +69,28 @@ def test_oracle_ref_recipe_and_oracle_agree_on_the_bench_workload(oracle):
         assert orc["status"][i] == 0
         assert orc["ids"][orc["ids_off"][i]:orc["ids_off"][i + 1]].tolist() == r["input_ids"], i
         assert orc["tt"][orc["tt_off"][i]:orc["tt_off"][i + 1]].tolist() == r["token_type_ids"], i
+
+
+def test_bench_dump_outputs_is_a_fixed_sample_of_the_planes(tmp_path):
+    """bench.py --dump-outputs: the same rows every run, their values as float32, the global pair index beside them; the
+    full-size dump ([DUMP_ROWS, 256] for three planes plus three per-row arrays and the index) stays under 64 MB."""
+    import torch
+    import bench
+    rng = np.random.default_rng(1)
+    m, W = 5000, 64
+    planes = {"input_ids": torch.from_numpy(rng.integers(0, 48423, (m, W)).astype(np.int32)),
+              "attention_mask": torch.from_numpy(rng.integers(0, 2, (m, W)).astype(np.uint8)),
+              "row_status": torch.from_numpy(rng.integers(0, 2, m).astype(np.uint8))}
+    for d in ("a", "b"):
+        bench.dump_outputs(planes, 7000, str(tmp_path / d), max_rows=300)
+    idx = np.load(tmp_path / "a" / "pair_index.npy")
+    assert idx.dtype == np.float64 and len(idx) == 300 and (np.diff(idx) > 0).all() and idx[0] >= 7000 and idx[-1] < 7000 + m
+    rows = idx.astype(np.int64) - 7000
+    for name, plane in planes.items():
+        a, b = np.load(tmp_path / "a" / (name + ".npy")), np.load(tmp_path / "b" / (name + ".npy"))
+        assert a.dtype == np.float32 and np.array_equal(a, b)
+        assert np.array_equal(a, plane.numpy()[rows].astype(np.float32)), name
+    assert bench.DUMP_ROWS * (3 * bench.MAX_LEN * 4 + 3 * 4 + 8) < 64e6
 
 
 def test_custom_model_builder_roundtrip(tmp_path, oracle):
