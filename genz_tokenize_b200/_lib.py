@@ -34,6 +34,11 @@ class DevPlanes(C.Structure):
                 ("sequence_id", C.c_void_p), ("row_len", C.c_void_p), ("seq_len", C.c_void_p), ("row_status", C.c_void_p)]
 
 
+class Windows(C.Structure):
+    _fields_ = [("enc", Encoded), ("n_docs", C.c_int64), ("win_off", C.POINTER(C.c_int64)), ("win_doc", C.POINTER(C.c_int64)),
+                ("win_start", C.POINTER(C.c_int32))]
+
+
 SIGNATURES = {
     # name: (restype, argtypes)
     "genztok_create": (C.c_int, [C.c_char_p, C.c_char_p, C.POINTER(C.c_char_p), C.POINTER(C.c_int), C.c_int, C.POINTER(C.c_void_p)]),
@@ -52,6 +57,10 @@ SIGNATURES = {
     "genztok_encode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int, C.c_int, C.c_uint32, C.POINTER(Encoded)]),
     "genztok_free_encoded": (None, [C.c_void_p, C.POINTER(Encoded)]),
     "genztok_encode_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_uint32, C.POINTER(DevPlanes), C.c_void_p]),
+    "genztok_encode_windows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_uint32, C.POINTER(Windows)]),
+    "genztok_free_windows": (None, [C.c_void_p, C.POINTER(Windows)]),
+    "genztok_encode_windows_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_int32,
+                                                C.c_uint32, C.c_void_p, C.POINTER(DevPlanes), C.c_void_p, C.c_void_p, C.POINTER(C.c_int64), C.c_void_p]),
     "genztok_decode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.POINTER(Text)]),
     "genztok_free_text": (None, [C.c_void_p, C.POINTER(Text)]),
     "genztok_decode_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_int64), C.c_void_p]),

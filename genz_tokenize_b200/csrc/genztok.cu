@@ -9,6 +9,8 @@
 // and for ragged results (no padding / no truncation / max_len None or <= 0)
 //   k_rows<COUNT> -> k_bpe_pending -> k_rows<COUNT> (row list) -> k_row_lens -> k_scan_i64
 //   -> k_rows<RAGGED> -> k_post_rows.
+// Long documents as windows (window.cuh): the ragged steps up to k_rows<RAGGED> per side -> k_window_count -> k_scan_i64
+//   -> k_window_rows -> k_post_rows (row list).
 // Decode is k_decode_len (lengths, trailing pad runs) -> k_scan_i64 -> k_decode_write.
 #include <cuda_runtime.h>
 
@@ -34,6 +36,7 @@
 #include "post.cuh"
 #include "prep.cuh"
 #include "synth.cuh"
+#include "window.cuh"
 
 using namespace gzt;
 
@@ -105,6 +108,14 @@ struct DeviceCtx {
     SynthTables synth{};
     bool synth_ready = false;
     DevBuf synth_len;
+    // long documents as windows (window.cuh): token streams of the two sides, windows per document, the k_post_rows row list; the
+    // batch step 1 of genztok_encode_windows_device described, for its step 2
+    struct WinState {
+        DevBuf ids[2], off[2], count, woff, fix, doc, start;
+        struct { const void *a = nullptr, *a_off = nullptr, *b = nullptr, *b_off = nullptr, *win_off = nullptr; int64_t n = -1, a_bytes = 0, b_bytes = 0;
+                 int32_t W = 0, s = 0; } sig;
+        int64_t n_win = -1;                       // windows of that batch; -1: no step 1 to continue from
+    } win;
     // profiling
     bool profiling = false;
     std::vector<ProfEvent> events;
@@ -720,6 +731,112 @@ int encode_fixed_on_device(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Si
     return stream_leave(h, d, st);
 }
 
+// ---- long documents as windows (window.cuh) -------------------------------------------------------------
+// Token stream of one side: [bos] T [eos] of every document, untruncated, ragged at off[m+1] (the ragged pipeline with max_len
+// None, without the mask and k_post_rows).  Reads the stream's size back to size `ids` (synchronises).
+int token_stream(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& s, int64_t m, DevBuf& ids, DevBuf& off) {
+    CU(d->redo.ensure((size_t)m * 4)); CU(d->fix.ensure((size_t)m * 4));
+    CU(d->L.ensure((size_t)m * 4)); CU(d->keep.ensure((size_t)m * 4)); CU(d->out_len.ensure((size_t)m * 8)); CU(d->tail.ensure((size_t)m));
+    CU(off.ensure((size_t)(m + 1) * 8));
+    { LaunchScope ls(h, d, "k_reset_lists"); k_reset_lists<<<1, 1, 0, st>>>(d->C); }
+    RowArgs A{};
+    A.a = s; A.n_rows = m; A.L = d->L.as<int32_t>(); A.redo_list = d->redo.as<uint32_t>(); A.fix_list = d->fix.as<uint32_t>();
+    A.eos_i8 = eos_as_i8(d); A.pad_i8 = pad_as_i8(d);
+    A.D = pick_tile_docs(h, d, s.nbytes, 0, m, 0, false);
+    int rc = launch_rows<MODE_COUNT>(h, d, A, st, "k_rows_count", m);
+    if (rc) return rc;
+    rc = launch_bpe(h, d, st);
+    if (rc) return rc;
+    RowArgs R = A;
+    R.row_list = d->redo.as<uint32_t>();
+    rc = launch_rows<MODE_COUNT>(h, d, R, st, "k_rows_count_redo", std::min<int64_t>(m, (int64_t)d->sm_count * 64));
+    if (rc) return rc;
+    LenArgs LA{d->L.as<int32_t>(), m, 0, 0, 0, 0, d->keep.as<int32_t>(), d->out_len.as<int64_t>(), d->tail.as<uint8_t>(), nullptr, nullptr, nullptr};
+    { LaunchScope ls(h, d, "k_row_lens"); k_row_lens<<<(unsigned)std::min<int64_t>((m + 255) / 256, 4096), 256, 0, st>>>(LA); }
+    rc = launch_scan(h, d, st, d->out_len.as<int64_t>(), off.as<int64_t>(), m);
+    if (rc) return rc;
+    int64_t total = 0;
+    CU(cudaMemcpyAsync(&total, off.as<int64_t>() + m, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    CU(ids.ensure((size_t)total * 4 + 16));
+    { LaunchScope ls(h, d, "k_reset_lists"); k_reset_lists<<<1, 1, 0, st>>>(d->C); }
+    RowArgs E = A;
+    E.ids = ids.as<int32_t>(); E.row_off = off.as<int64_t>(); E.keep = d->keep.as<int32_t>();
+    return launch_rows<MODE_RAGGED>(h, d, E, st, "k_rows_ragged", m);
+}
+
+WinArgs window_args(DeviceCtx* d, bool pair, int64_t n, int32_t W, int32_t s) {
+    WinArgs A{};
+    A.ids_a = d->win.ids[0].as<int32_t>(); A.off_a = d->win.off[0].as<int64_t>();
+    if (pair) { A.ids_b = d->win.ids[1].as<int32_t>(); A.off_b = d->win.off[1].as<int64_t>(); }
+    A.n_docs = n; A.W = W; A.stride = s;
+    A.ctr = d->C.ctr;
+    A.eos_i8 = eos_as_i8(d); A.pad_i8 = pad_as_i8(d);
+    return A;
+}
+
+// Step 1: both token streams, the windows of every document, d_win_off[n+1] and their total (synchronises).  The caller has
+// sized the word cache for the chunk (ensure_cache) and n >= 1.
+int windows_layout(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& a, const Side* b, int64_t n, int32_t W, int32_t s, int64_t* d_win_off,
+                   int64_t* n_win) {
+    d->win.n_win = -1;                                               // the streams are about to change
+    int rc = launch_guard(h, d, st, a.nbytes + (b ? b->nbytes : 0) + 16, 0);
+    if (rc) return rc;
+    rc = token_stream(h, d, st, a, n, d->win.ids[0], d->win.off[0]);
+    if (!rc && b) rc = token_stream(h, d, st, *b, n, d->win.ids[1], d->win.off[1]);
+    if (rc) return rc;
+    d->cache_empty = false;
+    CU(d->win.count.ensure((size_t)n * 8));
+    WinArgs A = window_args(d, b != nullptr, n, W, s);
+    A.count = d->win.count.as<int64_t>();
+    { LaunchScope ls(h, d, "k_window_count"); k_window_count<<<(unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)d->sm_count * 8), 256, 0, st>>>(A); }
+    CU(cudaGetLastError());
+    rc = launch_scan(h, d, st, d->win.count.as<int64_t>(), d_win_off, n);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(n_win, d_win_off + n, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return GENZTOK_OK;
+}
+
+// Step 2: the K windows' planes and maps from the streams step 1 left (does not synchronise).  win_doc = doc_base + document.
+int windows_write(genztok_t* h, DeviceCtx* d, cudaStream_t st, bool pair, int64_t n, int32_t W, int32_t s, uint32_t flags, const int64_t* d_win_off,
+                  int64_t K, const genztok_dev_planes_t& P, int64_t* win_doc, int32_t* win_start, int64_t doc_base) {
+    if (K <= 0) return GENZTOK_OK;
+    if (K >= (1ll << 32)) return fail(h, GENZTOK_E_LIMIT, "%lld windows in one chunk", (long long)K);
+    CU(d->win.fix.ensure((size_t)K * 4));
+    { LaunchScope ls(h, d, "k_reset_lists"); k_reset_lists<<<1, 1, 0, st>>>(d->C); }
+    WinArgs A = window_args(d, pair, n, W, s);
+    A.win_off = d_win_off; A.n_win = K; A.doc_base = doc_base;
+    A.ids = P.input_ids; A.mask = P.attention_mask; A.row_len = P.row_len;
+    if (pair) {
+        A.tt = (flags & GENZTOK_WANT_TOKEN_TYPE) ? P.token_type_ids : nullptr;
+        A.seq = (flags & GENZTOK_WANT_SEQUENCE_ID) ? P.sequence_id : nullptr;
+        A.seq_len = P.seq_len; A.status = P.row_status;
+    }
+    A.win_doc = win_doc; A.win_start = win_start; A.fix_list = d->win.fix.as<uint32_t>();
+    auto aligned = [](const void* p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) == 0; };
+    const bool quad = (W & 3) == 0 && aligned(A.ids, 16) && aligned(A.mask, 4) && aligned(A.tt, 4) && aligned(A.seq, 4);
+    const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((K + 7) / 8, (int64_t)d->sm_count * 8));
+    {
+        // algorithmic bytes: the planes and per-window values written (the windows' tokens are read from the streams, mostly in L2)
+        const int64_t alg = K * (int64_t)W * (5 + (A.tt ? 1 : 0) + (A.seq ? 1 : 0)) + K * (4 + 8 + 4 + (pair ? 5 : 0));
+        LaunchScope ls(h, d, "k_window_rows", alg);
+        if (pair) { if (quad) k_window_rows<true, true><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, true><<<grid, 256, 0, st>>>(d->T, A); }
+        else { if (quad) k_window_rows<true, false><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, false><<<grid, 256, 0, st>>>(d->T, A); }
+    }
+    CU(cudaGetLastError());
+    if (pair && (A.tt || A.seq || A.seq_len || A.status)) {
+        PostArgs Q{};
+        Q.ids = P.input_ids; Q.W = W; Q.n_rows = K; Q.row_list = A.fix_list;
+        Q.has_pair = 1; Q.tt = A.tt; Q.seq = A.seq; Q.seq_len = A.seq_len; Q.status = A.status;
+        Q.has_max_len = 1; Q.max_len = W; Q.padding = 1; Q.truncation = 1; Q.eos_i8 = A.eos_i8; Q.pad_i8 = A.pad_i8;
+        LaunchScope ls(h, d, "k_post_rows_windows");
+        k_post_rows<<<d->sm_count, 256, 0, st>>>(d->T, Q, d->C.ctr + C_FIX);
+        CU(cudaGetLastError());
+    }
+    return GENZTOK_OK;
+}
+
 void* host_pool_get(genztok_t* h, size_t bytes, size_t* got = nullptr) {
     if (bytes == 0) bytes = 16;
     {
@@ -760,6 +877,7 @@ struct PinnedVec {
             const size_t want = std::max<size_t>(m * sizeof(T) + m * sizeof(T) / 2, 1 << 16);
             T* q = reinterpret_cast<T*>(host_pool_get(h, (want + 4095) & ~(size_t)4095, &got));
             if (!q) return false;
+            { std::lock_guard<std::mutex> l(h->pool_mu); h->plane_meta.erase(q); }   // (it is about to hold other data than a padded plane)
             if (n) memcpy(q, p, n * sizeof(T));
             if (p) host_pool_put(h, p, cap_bytes);
             p = q; cap_bytes = got;
@@ -847,6 +965,7 @@ void genztok_destroy(genztok_t* h) {
         if (d->over32_ev) cudaEventDestroy(d->over32_ev);
         if (d->last_done) cudaEventDestroy(d->last_done);
         d->synth_len.release();
+        for (DevBuf* b : {&d->win.ids[0], &d->win.ids[1], &d->win.off[0], &d->win.off[1], &d->win.count, &d->win.woff, &d->win.fix, &d->win.doc, &d->win.start}) b->release();
         for (auto& fb : d->flat) for (DevBuf* b : {&fb.dsb, &fb.st, &fb.tpref, &fb.cnt, &fb.wtok}) b->release();
         if (d->stream) cudaStreamDestroy(d->stream);
         delete d;
@@ -1076,6 +1195,28 @@ struct EncodePart {
     void bind(genztok_t* h) { ids.h = h; spans.h = h; mask.h = h; tt.h = h; seq.h = h; offs.h = h; soffs.h = h; }
 };
 
+// Chunk boundaries of rows [rb, re): rows [cuts[i], cuts[i+1]) with at most chunk_rows rows and max_chunk_bytes bytes; *most = the
+// largest chunk's bytes.  Returns -1, or a document that alone is larger than max_chunk_bytes.
+int64_t chunk_cuts(const genztok_t* h, const EncodeJob& J, int64_t rb, int64_t re, std::vector<int64_t>* cuts, int64_t* most) {
+    auto bytes_of = [&](int64_t a, int64_t b) { return (J.text_off[b] - J.text_off[a]) + (J.has_pair ? J.pair_off[b] - J.pair_off[a] : 0) + 64; };
+    cuts->assign(1, rb);
+    *most = 0;
+    int64_t r0 = rb;
+    while (r0 < re) {
+        int64_t r1 = std::min<int64_t>(re, r0 + h->chunk_rows);
+        if (bytes_of(r0, r1) > h->max_chunk_bytes) {
+            int64_t lo = r0 + 1, hi = r1;   // largest r1 that fits (at least one row)
+            while (lo < hi) { int64_t mid = (lo + hi + 1) / 2; if (bytes_of(r0, mid) <= h->max_chunk_bytes) lo = mid; else hi = mid - 1; }
+            r1 = lo;
+            if (bytes_of(r0, r1) > h->max_chunk_bytes) return r0;
+        }
+        cuts->push_back(r1);
+        *most = std::max<int64_t>(*most, bytes_of(r0, r1));
+        r0 = r1;
+    }
+    return -1;
+}
+
 void encode_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int64_t rb, int64_t re, EncodePart* part) {
     genztok_encoded_t* out = J.out;
     const bool has_pair = J.has_pair, has_max_len = J.has_max_len, want_spans = J.want_spans, fixed = J.fixed, want_tt = J.want_tt, want_seq = J.want_seq;
@@ -1087,32 +1228,11 @@ void encode_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int64
     CUF(cudaSetDevice(d->device));
     LaunchScope::cur_stream = st;
     const int8_t eos8 = eos_as_i8(d);
-    // chunk boundaries: rows [r0, r1) with at most chunk_rows rows and max_chunk_bytes bytes
-    std::vector<int64_t> cuts{rb};
-    {
-        int64_t r0 = rb;
-        while (r0 < re) {
-            int64_t r1 = std::min<int64_t>(re, r0 + h->chunk_rows);
-            auto bytes_of = [&](int64_t a, int64_t b) { return (J.text_off[b] - J.text_off[a]) + (has_pair ? J.pair_off[b] - J.pair_off[a] : 0) + 64; };
-            if (bytes_of(r0, r1) > h->max_chunk_bytes) {
-                int64_t lo = r0 + 1, hi = r1;   // largest r1 that fits (at least one row)
-                while (lo < hi) { int64_t mid = (lo + hi + 1) / 2; if (bytes_of(r0, mid) <= h->max_chunk_bytes) lo = mid; else hi = mid - 1; }
-                r1 = lo;
-                if (bytes_of(r0, r1) > h->max_chunk_bytes)
-                    PFAIL(GENZTOK_E_LIMIT, "document %lld is larger than max_chunk_bytes=%lld", (long long)r0, (long long)h->max_chunk_bytes)
-            }
-            cuts.push_back(r1);
-            r0 = r1;
-        }
-    }
-    {
-        int64_t most = 0;                                            // the largest chunk of this call
-        for (size_t ci = 0; ci + 1 < cuts.size(); ci++) {
-            const int64_t a0 = cuts[ci], a1 = cuts[ci + 1];
-            most = std::max<int64_t>(most, (J.text_off[a1] - J.text_off[a0]) + (has_pair ? J.pair_off[a1] - J.pair_off[a0] : 0) + 64);
-        }
-        FAIL_RC(ensure_cache(h, d, st, most));
-    }
+    std::vector<int64_t> cuts;
+    int64_t most = 0;
+    { const int64_t big = chunk_cuts(h, J, rb, re, &cuts, &most);
+      if (big >= 0) PFAIL(GENZTOK_E_LIMIT, "document %lld is larger than max_chunk_bytes=%lld", (long long)big, (long long)h->max_chunk_bytes) }
+    FAIL_RC(ensure_cache(h, d, st, most));
     unsigned long long tokens_before = 0;
     CUF(cudaMemcpyAsync(&tokens_before, d->C.ctr + C_TOKENS, 8, cudaMemcpyDeviceToHost, st));
     CUF(cudaStreamSynchronize(st));
@@ -1508,7 +1628,272 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
 }  // extern "C"
 
 namespace {
+
+// What one device collects for its documents [rb, re) of genztok_encode_windows (chunk after chunk, in document order).
+struct WindowPart {
+    int rc = GENZTOK_OK;
+    std::string err;
+    int64_t n_win = 0, tokens = 0, d2h_bytes = 0;
+    PinnedVec<int32_t> ids, row_len, seq_len, start; PinnedVec<uint8_t> mask, status; PinnedVec<int8_t> tt, seq; PinnedVec<int64_t> doc, offs;
+    void bind(genztok_t* h) { for (auto* v : {&ids, &row_len, &seq_len, &start}) v->h = h; mask.h = h; status.h = h; tt.h = h; seq.h = h; doc.h = h; offs.h = h; }
+};
+
+// Windows of documents [rb, re) on one device: per chunk the text goes up, both steps run, the planes and maps come home.
+// win_off[r] for r in (rb, re] is written relative to the part's first window.
+void windows_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int32_t stride, int64_t* win_off, int64_t rb, int64_t re, WindowPart* part) {
+    const bool has_pair = J.has_pair;
+    const int32_t W = J.max_len;
+    cudaStream_t st = d->stream;
+#define PFAIL(code, ...) { char _b[400]; snprintf(_b, sizeof _b, __VA_ARGS__); part->rc = (code); part->err = _b; cudaStreamSynchronize(st); return; }
+#define FAIL_RC(call) { int _rc = (call); if (_rc) { part->rc = _rc; { std::lock_guard<std::mutex> _l(h->err_mu); part->err = h->err; } cudaStreamSynchronize(st); return; } }
+#define CUF(call) { cudaError_t _e = (call); if (_e != cudaSuccess) PFAIL(GENZTOK_E_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(_e), __FILE__, __LINE__) }
+    CUF(cudaSetDevice(d->device));
+    LaunchScope::cur_stream = st;
+    FAIL_RC(stream_enter(h, d, st));
+    std::vector<int64_t> cuts;
+    int64_t most = 0;
+    { const int64_t big = chunk_cuts(h, J, rb, re, &cuts, &most);
+      if (big >= 0) PFAIL(GENZTOK_E_LIMIT, "document %lld is larger than max_chunk_bytes=%lld", (long long)big, (long long)h->max_chunk_bytes) }
+    FAIL_RC(ensure_cache(h, d, st, most));
+    unsigned long long tokens_before = 0;
+    CUF(cudaMemcpyAsync(&tokens_before, d->C.ctr + C_TOKENS, 8, cudaMemcpyDeviceToHost, st));
+    for (size_t ci = 0; ci + 1 < cuts.size(); ci++) {
+        const int64_t r0 = cuts[ci], r1 = cuts[ci + 1], m = r1 - r0;
+        const int64_t tb0 = J.text_off[r0], tb = J.text_off[r1] - tb0;
+        const int64_t pb0 = has_pair ? J.pair_off[r0] : 0, pb = has_pair ? J.pair_off[r1] - pb0 : 0;
+        // (as in the ragged path: offsets stay absolute, the chunk lands at dev + (tb0 & 15) behind a base pointer shifted by -tb0)
+        const int64_t ta = tb0 & 15, pa = pb0 & 15;
+        CUF(d->text.ensure((size_t)tb + 96)); CUF(d->toff.ensure((size_t)(m + 1) * 8));
+        if (tb) CUF(cudaMemcpyAsync(d->text.as<uint8_t>() + ta, J.text + tb0, (size_t)tb, cudaMemcpyHostToDevice, st));
+        CUF(cudaMemcpyAsync(d->toff.p, J.text_off + r0, (size_t)(m + 1) * 8, cudaMemcpyHostToDevice, st));
+        if (has_pair) {
+            CUF(d->pair.ensure((size_t)pb + 96)); CUF(d->poff.ensure((size_t)(m + 1) * 8));
+            if (pb) CUF(cudaMemcpyAsync(d->pair.as<uint8_t>() + pa, J.pair + pb0, (size_t)pb, cudaMemcpyHostToDevice, st));
+            CUF(cudaMemcpyAsync(d->poff.p, J.pair_off + r0, (size_t)(m + 1) * 8, cudaMemcpyHostToDevice, st));
+        }
+        Side a{d->text.as<uint8_t>() + ta - tb0, d->toff.as<int64_t>(), tb};
+        Side b{has_pair ? d->pair.as<uint8_t>() + pa - pb0 : nullptr, d->poff.as<int64_t>(), pb};
+        CUF(d->win.woff.ensure((size_t)(m + 1) * 8));
+        int64_t K = 0;
+        FAIL_RC(windows_layout(h, d, st, a, has_pair ? &b : nullptr, m, W, stride, d->win.woff.as<int64_t>(), &K));
+        const size_t tot = (size_t)K * (size_t)W;
+        CUF(d->ids.ensure(tot * 4 + 16)); CUF(d->mask.ensure(tot + 16)); CUF(d->row_len.ensure((size_t)K * 4 + 16));
+        CUF(d->win.doc.ensure((size_t)K * 8 + 16)); CUF(d->win.start.ensure((size_t)K * 4 + 16));
+        genztok_dev_planes_t P{};
+        P.input_ids = d->ids.as<int32_t>(); P.attention_mask = d->mask.as<uint8_t>(); P.row_len = d->row_len.as<int32_t>();
+        if (J.want_tt) { CUF(d->tt.ensure(tot + 16)); P.token_type_ids = d->tt.as<int8_t>(); }
+        if (J.want_seq) { CUF(d->seq.ensure(tot + 16)); P.sequence_id = d->seq.as<int8_t>(); }
+        if (has_pair) { CUF(d->seq_len.ensure((size_t)K * 4 + 16)); CUF(d->status.ensure((size_t)K + 16)); P.seq_len = d->seq_len.as<int32_t>(); P.row_status = d->status.as<uint8_t>(); }
+        FAIL_RC(windows_write(h, d, st, has_pair, m, W, stride, J.flags, d->win.woff.as<int64_t>(), K, P, d->win.doc.as<int64_t>(), d->win.start.as<int32_t>(), r0));
+        const size_t o = (size_t)part->n_win, n1 = o + (size_t)K;
+        if (ci == 0 && r1 < re) {                                    // first chunk of several: room for the part at this chunk's windows per document (+ 12 %)
+            const size_t est = (size_t)((double)K * (double)(re - rb) / (double)m * 1.125) + 64;
+            bool ok = part->ids.reserve(est * W) && part->mask.reserve(est * W) && part->row_len.reserve(est) && part->doc.reserve(est) && part->start.reserve(est);
+            if (J.want_tt) ok = ok && part->tt.reserve(est * W);
+            if (J.want_seq) ok = ok && part->seq.reserve(est * W);
+            if (has_pair) ok = ok && part->seq_len.reserve(est) && part->status.reserve(est);
+            if (!ok) PFAIL(GENZTOK_E_NOMEM, "pinned host allocation failed")
+        }
+        bool grown = part->ids.resize(n1 * W) && part->mask.resize(n1 * W) && part->row_len.resize(n1) && part->doc.resize(n1) && part->start.resize(n1) &&
+                     part->offs.resize((size_t)m + 1);
+        if (J.want_tt) grown = grown && part->tt.resize(n1 * W);
+        if (J.want_seq) grown = grown && part->seq.resize(n1 * W);
+        if (has_pair) grown = grown && part->seq_len.resize(n1) && part->status.resize(n1);
+        if (!grown) PFAIL(GENZTOK_E_NOMEM, "pinned host allocation failed")
+        if (K) {
+            CUF(cudaMemcpyAsync(part->ids.data() + o * W, P.input_ids, tot * 4, cudaMemcpyDeviceToHost, st));
+            CUF(cudaMemcpyAsync(part->mask.data() + o * W, P.attention_mask, tot, cudaMemcpyDeviceToHost, st));
+            if (J.want_tt) CUF(cudaMemcpyAsync(part->tt.data() + o * W, P.token_type_ids, tot, cudaMemcpyDeviceToHost, st));
+            if (J.want_seq) CUF(cudaMemcpyAsync(part->seq.data() + o * W, P.sequence_id, tot, cudaMemcpyDeviceToHost, st));
+            CUF(cudaMemcpyAsync(part->row_len.data() + o, P.row_len, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
+            CUF(cudaMemcpyAsync(part->doc.data() + o, d->win.doc.p, (size_t)K * 8, cudaMemcpyDeviceToHost, st));
+            CUF(cudaMemcpyAsync(part->start.data() + o, d->win.start.p, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
+            if (has_pair) {
+                CUF(cudaMemcpyAsync(part->seq_len.data() + o, P.seq_len, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
+                CUF(cudaMemcpyAsync(part->status.data() + o, P.row_status, (size_t)K, cudaMemcpyDeviceToHost, st));
+            }
+        }
+        CUF(cudaMemcpyAsync(part->offs.data(), d->win.woff.p, (size_t)(m + 1) * 8, cudaMemcpyDeviceToHost, st));
+        CUF(cudaStreamSynchronize(st));
+        part->d2h_bytes += (int64_t)tot * (5 + (J.want_tt ? 1 : 0) + (J.want_seq ? 1 : 0)) + K * (16 + (has_pair ? 5 : 0)) + (m + 1) * 8;
+        const int64_t* offs = part->offs.data();
+        for (int64_t i = 1; i <= m; i++) win_off[r0 + i] = part->n_win + offs[i];
+        part->n_win += K;
+    }
+    unsigned long long tokens_after = 0, nerr = 0;
+    CUF(cudaMemcpyAsync(&tokens_after, d->C.ctr + C_TOKENS, 8, cudaMemcpyDeviceToHost, st));
+    CUF(cudaMemcpyAsync(&nerr, d->C.ctr + C_ERR, 8, cudaMemcpyDeviceToHost, st));
+    CUF(cudaStreamSynchronize(st));
+    if (nerr) PFAIL(GENZTOK_E_CUDA, "internal error: device pipeline reported %llu inconsistencies", nerr)
+    part->tokens = (int64_t)(tokens_after - tokens_before);
+    FAIL_RC(stream_leave(h, d, st));
+#undef PFAIL
+#undef FAIL_RC
+#undef CUF
+}
+
+int check_window_args(genztok_t* h, int32_t max_len, int32_t stride, uint32_t flags) {
+    if (max_len < 3) return fail(h, GENZTOK_E_INVALID, "windows need max_len >= 3 (got %d)", max_len);
+    if (stride < 0 || stride >= max_len - 2) return fail(h, GENZTOK_E_INVALID, "windows need 0 <= stride < max_len - 2 (got stride=%d, max_len=%d)", stride, max_len);
+    if (flags & GENZTOK_WANT_SPANS) return fail(h, GENZTOK_E_INVALID, "spans are not available for windows");
+    return GENZTOK_OK;
+}
+
 }  // namespace
+
+extern "C" {
+
+int genztok_encode_windows(genztok_t* h, const uint8_t* text, const int64_t* text_off, const uint8_t* pair, const int64_t* pair_off, int64_t n,
+                           int32_t max_len, int32_t stride, uint32_t flags, genztok_windows_t* out) {
+    if (!h) return GENZTOK_E_INVALID;
+    if (!out || n < 0 || !text_off) return fail(h, GENZTOK_E_INVALID, "genztok_encode_windows: bad arguments");
+    int rc = check_window_args(h, max_len, stride, flags);
+    if (rc) return rc;
+    if (h->devs.empty()) return fail(h, GENZTOK_E_NODEVICE, "this handle was created without a CUDA device; there is no CPU path");
+    memset(out, 0, sizeof *out);
+    std::lock_guard<std::mutex> lk(h->mu);
+    EncodeJob J{};
+    J.text = text; J.text_off = text_off; J.pair = pair; J.pair_off = pair_off;
+    J.max_len = max_len; J.padding = 1; J.truncation = 1; J.flags = flags;
+    J.has_pair = pair_off != nullptr; J.has_max_len = true; J.fixed = true;
+    J.want_tt = J.has_pair && (flags & GENZTOK_WANT_TOKEN_TYPE);
+    J.want_seq = J.has_pair && (flags & GENZTOK_WANT_SEQUENCE_ID);
+    const bool has_pair = J.has_pair;
+    OutBlock* ob = new OutBlock();
+    auto bail = [&](int code) {
+        for (auto& pr : ob->pinned) host_pool_put(h, pr.first, pr.second);
+        delete ob;
+        memset(out, 0, sizeof *out);
+        return code;
+    };
+    // every result buffer leaves the pool to hold windows: what plane_meta knew of it no longer holds
+    auto take = [&](auto* p) { if (p) h->plane_meta.erase(p); return p; };
+    int64_t* win_off = take(out_alloc<int64_t>(h, ob, (size_t)n + 1));
+    if (!win_off) return bail(fail(h, GENZTOK_E_NOMEM, "pinned host allocation failed"));
+    win_off[0] = 0;
+    // shard the documents across the devices as genztok_encode does: contiguous ranges balanced by bytes
+    const int G = (int)h->devs.size();
+    const bool one = G == 1 || n < 2 * G;
+    std::vector<int64_t> dcut((size_t)G + 1, n);
+    dcut[0] = 0;
+    if (!one) {
+        auto weight = [&](int64_t r) { return text_off[r] + (has_pair ? pair_off[r] : 0) + 64 * r; };
+        const int64_t wtot = weight(n) - weight(0);
+        for (int g = 1; g < G; g++) {
+            const int64_t want = weight(0) + wtot * g / G;
+            int64_t lo = dcut[(size_t)g - 1], hi = n;
+            while (lo < hi) { int64_t mid = (lo + hi) / 2; if (weight(mid) < want) lo = mid + 1; else hi = mid; }
+            dcut[(size_t)g] = lo;
+        }
+    } else for (int g = 1; g <= G; g++) dcut[(size_t)g] = n;
+    std::vector<WindowPart> parts((size_t)G);
+    for (auto& pt : parts) pt.bind(h);
+    if (one) windows_rows_on_device(h, h->devs[0], J, stride, win_off, 0, n, &parts[0]);
+    else {
+        std::vector<std::thread> th;
+        for (int g = 0; g < G; g++)
+            th.emplace_back([&, g]() { windows_rows_on_device(h, h->devs[(size_t)g], J, stride, win_off, dcut[(size_t)g], dcut[(size_t)g + 1], &parts[(size_t)g]); });
+        for (auto& t : th) t.join();
+    }
+    for (auto& pt : parts)
+        if (pt.rc) { { std::lock_guard<std::mutex> l(h->err_mu); h->err = pt.err; } return bail(pt.rc); }
+    int64_t K = 0;
+    for (auto& pt : parts) K += pt.n_win;
+    const size_t tot = (size_t)K * (size_t)max_len;
+    genztok_encoded_t& E = out->enc;
+    E.n = K; E.total = (int64_t)tot; E.width = max_len; E.has_pair = has_pair;
+    E.input_ids = take(out_alloc<int32_t>(h, ob, tot));
+    E.attention_mask = take(out_alloc<uint8_t>(h, ob, tot));
+    E.row_len = take(out_alloc<int32_t>(h, ob, (size_t)K));
+    out->win_doc = take(out_alloc<int64_t>(h, ob, (size_t)K));
+    out->win_start = take(out_alloc<int32_t>(h, ob, (size_t)K));
+    bool ok = E.input_ids && E.attention_mask && E.row_len && out->win_doc && out->win_start;
+    if (J.want_tt) { E.token_type_ids = take(out_alloc<int8_t>(h, ob, tot)); E.tt_len = take(out_alloc<int32_t>(h, ob, (size_t)K)); ok = ok && E.token_type_ids && E.tt_len; }
+    if (J.want_seq) { E.sequence_id = take(out_alloc<int8_t>(h, ob, tot)); ok = ok && E.sequence_id; }
+    if (has_pair) { E.seq_len = take(out_alloc<int32_t>(h, ob, (size_t)K)); E.row_status = take(out_alloc<uint8_t>(h, ob, (size_t)K)); ok = ok && E.seq_len && E.row_status; }
+    if (!ok) return bail(fail(h, GENZTOK_E_NOMEM, "pinned host allocation failed"));
+    // stitch the parts in document order; their window offsets are shifted by the windows before them
+    int64_t base = 0;
+    for (int g = 0; g < G; g++) {
+        WindowPart& pt = parts[(size_t)g];
+        if (base) for (int64_t r = dcut[(size_t)g] + 1; r <= dcut[(size_t)g + 1]; r++) win_off[r] += base;
+        const size_t k = (size_t)pt.n_win, o = (size_t)base, w = (size_t)max_len;
+        if (k) {
+            memcpy(E.input_ids + o * w, pt.ids.data(), k * w * 4);
+            memcpy(E.attention_mask + o * w, pt.mask.data(), k * w);
+            memcpy(E.row_len + o, pt.row_len.data(), k * 4);
+            memcpy(out->win_doc + o, pt.doc.data(), k * 8);
+            memcpy(out->win_start + o, pt.start.data(), k * 4);
+            if (J.want_tt) memcpy(E.token_type_ids + o * w, pt.tt.data(), k * w);
+            if (J.want_seq) memcpy(E.sequence_id + o * w, pt.seq.data(), k * w);
+            if (has_pair) { memcpy(E.seq_len + o, pt.seq_len.data(), k * 4); memcpy(E.row_status + o, pt.status.data(), k); }
+        }
+        base += pt.n_win;
+        E.real_tokens += pt.tokens; E.d2h_bytes += pt.d2h_bytes;
+    }
+    if (J.want_tt) for (int64_t r = 0; r < K; r++) E.tt_len[r] = max_len;
+    E._owner = ob;
+    out->n_docs = n;
+    out->win_off = win_off;
+    return GENZTOK_OK;
+}
+
+void genztok_free_windows(genztok_t* h, genztok_windows_t* out) {
+    if (!out) return;
+    genztok_free_encoded(h, &out->enc);                              // (the maps belong to the same block)
+    memset(out, 0, sizeof *out);
+}
+
+int genztok_encode_windows_device(genztok_t* h, int dev, const uint8_t* d_text, const int64_t* d_text_off, int64_t text_bytes, const uint8_t* d_pair,
+                                  const int64_t* d_pair_off, int64_t pair_bytes, int64_t n, int32_t max_len, int32_t stride, uint32_t flags,
+                                  int64_t* d_win_off, const genztok_dev_planes_t* planes, int64_t* d_win_doc, int32_t* d_win_start, int64_t* n_windows,
+                                  void* stream) {
+    if (!h) return GENZTOK_E_INVALID;
+    if (dev < 0 || dev >= (int)h->devs.size()) return fail(h, GENZTOK_E_NODEVICE, "no such device slot %d (handle has %d)", dev, (int)h->devs.size());
+    if (n < 0 || !d_text_off || !d_win_off || (text_bytes > 0 && !d_text) || (planes == nullptr && !n_windows))
+        return fail(h, GENZTOK_E_INVALID, "genztok_encode_windows_device: bad arguments");
+    int rc = check_window_args(h, max_len, stride, flags);
+    if (rc) return rc;
+    if (((uintptr_t)d_text & 15) || ((uintptr_t)d_pair & 15)) return fail(h, GENZTOK_E_INVALID, "device text buffers must be 16-byte aligned");
+    std::lock_guard<std::mutex> lk(h->mu);
+    DeviceCtx* d = h->devs[(size_t)dev];
+    CU(cudaSetDevice(d->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : d->stream;
+    LaunchScope::cur_stream = st;
+    const bool has_pair = d_pair_off != nullptr;
+    const int64_t bytes = text_bytes + (has_pair ? pair_bytes : 0);
+    if (bytes > h->max_chunk_bytes) return fail(h, GENZTOK_E_LIMIT, "chunk of %lld bytes exceeds max_chunk_bytes=%lld", (long long)bytes, (long long)h->max_chunk_bytes);
+    DeviceCtx::WinState& S = d->win;
+    const bool same = S.n_win >= 0 && S.sig.a == d_text && S.sig.a_off == d_text_off && S.sig.b == d_pair && S.sig.b_off == d_pair_off &&
+                      S.sig.win_off == d_win_off && S.sig.n == n && S.sig.a_bytes == text_bytes && S.sig.b_bytes == (has_pair ? pair_bytes : 0) &&
+                      S.sig.W == max_len && S.sig.s == stride;
+    rc = stream_enter(h, d, st);
+    if (rc) return rc;
+    if (!planes || !same) {
+        int64_t K = 0;
+        if (n == 0) CU(cudaMemsetAsync(d_win_off, 0, 8, st));
+        else {
+            rc = ensure_cache(h, d, st, bytes + 32);
+            if (rc) return rc;
+            Side a{d_text, d_text_off, text_bytes}, b{d_pair, d_pair_off, pair_bytes};
+            rc = windows_layout(h, d, st, a, has_pair ? &b : nullptr, n, max_len, stride, d_win_off, &K);
+            if (rc) return rc;
+        }
+        S.n_win = K;
+        S.sig.a = d_text; S.sig.a_off = d_text_off; S.sig.b = d_pair; S.sig.b_off = d_pair_off; S.sig.win_off = d_win_off;
+        S.sig.n = n; S.sig.a_bytes = text_bytes; S.sig.b_bytes = has_pair ? pair_bytes : 0; S.sig.W = max_len; S.sig.s = stride;
+    }
+    if (n_windows) *n_windows = S.n_win;
+    if (planes) {
+        if (S.n_win > 0 && (!planes->input_ids || !planes->attention_mask || !planes->row_len || !d_win_doc || !d_win_start))
+            return fail(h, GENZTOK_E_INVALID, "genztok_encode_windows_device: step 2 needs input_ids, attention_mask, row_len and the two maps");
+        rc = windows_write(h, d, st, has_pair, n, max_len, stride, flags, d_win_off, S.n_win, *planes, d_win_doc, d_win_start, 0);
+        if (rc) return rc;
+    }
+    return stream_leave(h, d, st);
+}
+
+}  // extern "C"
 
 extern "C" {
 

@@ -4,8 +4,9 @@ wrapper over libgenztok.so.  Same constructor, `fromFile`, `__call__`, `encode`,
 B200 -- there is no CPU path, and a handle without a device raises.
 
 Extensions over the reference (which is one string per call): `encode_batch` / `decode_batch`
-(numpy in, numpy out through pinned host buffers) and `encode_device` / `decode_device`
-(torch CUDA tensors in and out, DLPack-exportable, nothing crosses PCIe).
+(numpy in, numpy out through pinned host buffers), `encode_device` / `decode_device`
+(torch CUDA tensors in and out, DLPack-exportable, nothing crosses PCIe) and `encode_windows` /
+`encode_windows_device` (long documents as overlapping max_len windows, every token kept).
 """
 import ctypes as C
 import operator
@@ -45,13 +46,13 @@ def _view(ptr, count, ctype, dtype, owner):
 
 
 class _EncodedOwner:
-    def __init__(self, tok, enc):
-        self.tok, self.enc = tok, enc
+    def __init__(self, tok, enc, free="genztok_free_encoded"):
+        self.tok, self.enc, self.free = tok, enc, free
 
     def __del__(self):
         try:
             if self.tok._h:
-                self.tok._lib.genztok_free_encoded(self.tok._h, C.byref(self.enc))
+                getattr(self.tok._lib, self.free)(self.tok._h, C.byref(self.enc))
         except Exception:
             pass
 
@@ -397,10 +398,13 @@ class Tokenize(object):
                                       flags, C.byref(enc))
         if rc:
             self._err(rc, "genztok_encode")
-        owner = _EncodedOwner(self, enc)
+        return self._wrap(enc, n, max_len is not None and bool(padding), _EncodedOwner(self, enc))
+
+    def _wrap(self, enc, n, pad_mode, owner):
+        """BatchEncoding of numpy views over the n rows of a genztok_encoded_t."""
         r = BatchEncoding()
         r._tok, r._n, r._width, r._has_pair = self, n, int(enc.width), bool(enc.has_pair)
-        r._pad_mode = max_len is not None and bool(padding)
+        r._pad_mode = pad_mode
         tot = int(enc.total)
         r._ids = _view(enc.input_ids, tot, C.c_int32, np.int32, owner)
         r._mask = _view(enc.attention_mask, tot, C.c_uint8, np.uint8, owner)
@@ -445,6 +449,93 @@ class Tokenize(object):
         if max_len is not None:
             max_len = operator.index(max_len)
         return self._encode_raw(texts, pair_texts, max_len, padding, truncation, flags, return_offset)
+
+    @staticmethod
+    def _window_args(max_len, stride):
+        max_len, stride = operator.index(max_len), operator.index(stride)
+        if max_len < 3:
+            raise ValueError("encode_windows needs max_len >= 3 (got %d)" % max_len)
+        if not 0 <= stride < max_len - 2:
+            raise ValueError("encode_windows needs 0 <= stride < max_len - 2 (got stride=%d, max_len=%d)" % (stride, max_len))
+        if max_len >= 2 ** 31:
+            raise OverflowError("max_len out of range")
+        return max_len, stride
+
+    def encode_windows(self, texts, pair_texts=None, max_len=512, stride=0, token_type_ids=True, sequence_id=False):
+        """Every token of long documents, as overlapping windows of max_len (HF tokenizers' return_overflowing_tokens with a
+        stride).  A single's window k holds [bos] + T[k(C-stride) : k(C-stride)+C] + [eos] with T = encode(text)[1:-1] and
+        C = max_len - 2; a pair keeps its first text whole in every window and windows the second with C = max_len - len(A) - 4
+        (one window, its encode_batch row, when C - stride < 1).  Each window is padded as encode_batch pads a row, so window 0
+        of a document equals its encode_batch(max_len=max_len) row.  Returns a BatchEncoding with the fixed-layout planes over
+        the windows plus overflow_to_sample_mapping (int64 [K]: the document of each window), window_start (int32 [K]: index
+        in T of its first content token) and window_off (int64 [n+1]: first window of each document)."""
+        max_len, stride = self._window_args(max_len, stride)
+        tb, to = texts if isinstance(texts, tuple) else pack_strings(texts)
+        n = len(to) - 1
+        flags, pbp, pop = 0, None, None
+        if pair_texts is not None:
+            pb, po = pair_texts if isinstance(pair_texts, tuple) else pack_strings(pair_texts)
+            if len(po) - 1 != n:
+                raise ValueError("texts and pair_texts differ in length")
+            pb, po = np.ascontiguousarray(pb, dtype=np.uint8), np.ascontiguousarray(po, dtype=np.int64)
+            pbp, pop = pb.ctypes.data, po.ctypes.data
+            flags = (L.WANT_TOKEN_TYPE if token_type_ids else 0) | (L.WANT_SEQUENCE_ID if sequence_id else 0)
+        tb, to = np.ascontiguousarray(tb, dtype=np.uint8), np.ascontiguousarray(to, dtype=np.int64)
+        w = L.Windows()
+        rc = self._lib.genztok_encode_windows(self._h, tb.ctypes.data, to.ctypes.data, pbp, pop, n, max_len, stride, flags, C.byref(w))
+        if rc:
+            self._err(rc, "genztok_encode_windows")
+        owner = _EncodedOwner(self, w, "genztok_free_windows")
+        K = int(w.enc.n)
+        r = self._wrap(w.enc, K, True, owner)
+        r["overflow_to_sample_mapping"] = _view(w.win_doc, K, C.c_int64, np.int64, owner)
+        r["window_start"] = _view(w.win_start, K, C.c_int32, np.int32, owner)
+        r["window_off"] = _view(w.win_off, n + 1, C.c_int64, np.int64, owner)
+        return r
+
+    def encode_windows_device(self, d_text, d_text_off, d_pair=None, d_pair_off=None, max_len=512, stride=0, token_type_ids=True,
+                              sequence_id=False, text_bytes=None, pair_bytes=None):
+        """encode_windows with everything resident on the GPU: inputs as for encode_device, outputs torch tensors on the input's
+        device written on torch's current stream (same keys as encode_windows).  The number of windows is read back between the
+        two steps (one synchronisation); the planes are then written without another."""
+        import torch
+        max_len, stride = self._window_args(max_len, stride)
+        n = d_text_off.numel() - 1
+        dev = d_text.device
+        has_pair = d_pair_off is not None
+        flags = ((L.WANT_TOKEN_TYPE if token_type_ids else 0) | (L.WANT_SEQUENCE_ID if sequence_id else 0)) if has_pair else 0
+        tbytes = d_text.numel() if text_bytes is None else text_bytes
+        pbytes = (d_pair.numel() if pair_bytes is None else pair_bytes) if has_pair else 0
+        args = (self._h, 0, d_text.data_ptr(), d_text_off.data_ptr(), tbytes, d_pair.data_ptr() if has_pair else None,
+                d_pair_off.data_ptr() if has_pair else None, pbytes, n, max_len, stride, flags)
+        st = self._torch_stream(dev)
+        win_off = torch.empty((n + 1,), dtype=torch.int64, device=dev)
+        K = C.c_int64()
+        rc = self._lib.genztok_encode_windows_device(*args, win_off.data_ptr(), None, None, None, C.byref(K), st)
+        if rc:
+            self._err(rc, "genztok_encode_windows_device")
+        K = int(K.value)
+        out = {"input_ids": torch.empty((K, max_len), dtype=torch.int32, device=dev),
+               "attention_mask": torch.empty((K, max_len), dtype=torch.uint8, device=dev),
+               "row_len": torch.empty((K,), dtype=torch.int32, device=dev)}
+        if has_pair:
+            if token_type_ids:
+                out["token_type_ids"] = torch.empty((K, max_len), dtype=torch.int8, device=dev)
+            if sequence_id:
+                out["sequence_id"] = torch.empty((K, max_len), dtype=torch.int8, device=dev)
+            out["seq_len"] = torch.empty((K,), dtype=torch.int32, device=dev)
+            out["row_status"] = torch.empty((K,), dtype=torch.uint8, device=dev)
+        out["overflow_to_sample_mapping"] = torch.empty((K,), dtype=torch.int64, device=dev)
+        out["window_start"] = torch.empty((K,), dtype=torch.int32, device=dev)
+        out["window_off"] = win_off
+        P = L.DevPlanes()
+        for k in ("input_ids", "attention_mask", "token_type_ids", "sequence_id", "row_len", "seq_len", "row_status"):
+            setattr(P, k, out[k].data_ptr() if k in out else None)
+        rc = self._lib.genztok_encode_windows_device(*args, win_off.data_ptr(), C.byref(P), out["overflow_to_sample_mapping"].data_ptr(),
+                                                     out["window_start"].data_ptr(), None, st)
+        if rc:
+            self._err(rc, "genztok_encode_windows_device")
+        return out
 
     def decode_batch(self, ids, offsets=None):
         """Decode rows of ids: a 2-D int array (fixed width), or flat ids + int64 offsets[n+1].  Returns list[str]."""

@@ -139,6 +139,36 @@ int genztok_encode_device(genztok_t *h, int dev, const uint8_t *d_text, const in
                           int64_t pair_bytes, int64_t n, int32_t max_len, uint32_t flags,
                           const genztok_dev_planes_t *planes, void *stream);
 
+/* ---- long documents as overlapping windows (HF tokenizers' return_overflowing_tokens + stride) ---- */
+/* T = encode(text)[1:-1] of L tokens (pairs: of the second text; A = the first text's, kept whole in every window).
+ * Singles: C = max_len - 2; K = 1 if L <= C, else 1 + ceil((L - C) / (C - stride)); window k is
+ * [bos] + T[k(C-stride) : k(C-stride)+C] + [eos].  Pairs: C = max_len - len(A) - 4, windows [bos] + A + [eos, eos] + B_k + [eos];
+ * when C - stride < 1 the document yields one window, its genztok_encode(max_len) row (row_status included).  Every window is
+ * then padded as tokenize.py:141-182,247-258 pad a row of max_len, so window 0 of a document equals its genztok_encode row.
+ * Requires max_len >= 3 and 0 <= stride < max_len - 2. */
+typedef struct genztok_windows {
+    genztok_encoded_t enc;  /* fixed layout: enc.n = windows, enc.width = max_len */
+    int64_t n_docs;
+    int64_t *win_off;       /* [n_docs+1] first window of each document */
+    int64_t *win_doc;       /* [enc.n] document of each window (overflow_to_sample_mapping) */
+    int32_t *win_start;     /* [enc.n] index in T of the window's first content token */
+} genztok_windows_t;
+/* Host buffers in, pinned host buffers out (chunked and sharded across the handle's devices like genztok_encode).
+ * flags: GENZTOK_WANT_TOKEN_TYPE / GENZTOK_WANT_SEQUENCE_ID for pairs. */
+int genztok_encode_windows(genztok_t *h, const uint8_t *text, const int64_t *text_off, const uint8_t *pair,
+                           const int64_t *pair_off, int64_t n, int32_t max_len, int32_t stride, uint32_t flags,
+                           genztok_windows_t *out);
+void genztok_free_windows(genztok_t *h, genztok_windows_t *out);
+/* Device form, two steps like genztok_decode_device.  Step 1 (planes == NULL): tokenises, fills d_win_off[n+1] and returns
+ * the number of windows in *n_windows (synchronises).  Step 2: writes the caller's [n_windows, max_len] planes (input_ids and
+ * attention_mask required; row_len required; token types, seq_len, row_status for pairs) and d_win_doc / d_win_start [n_windows]
+ * from what step 1 left in the handle; a step 2 for another batch (other pointers, n, max_len, stride) redoes step 1.  Text
+ * buffers 16-byte aligned, as for genztok_encode_device.  Step 2 does not synchronise. */
+int genztok_encode_windows_device(genztok_t *h, int dev, const uint8_t *d_text, const int64_t *d_text_off, int64_t text_bytes,
+                                  const uint8_t *d_pair, const int64_t *d_pair_off, int64_t pair_bytes, int64_t n, int32_t max_len,
+                                  int32_t stride, uint32_t flags, int64_t *d_win_off, const genztok_dev_planes_t *planes,
+                                  int64_t *d_win_doc, int32_t *d_win_start, int64_t *n_windows, void *stream);
+
 /* ---- decode: Tokenize.decode over a batch (tokenize.py:137-139) ------------------------------ */
 /* ids_off == NULL: n rows of `width` ids each.  Ids outside the decoder print the unk string. */
 int genztok_decode(genztok_t *h, const int32_t *ids, const int64_t *ids_off, int64_t n, int32_t width,
