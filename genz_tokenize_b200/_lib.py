@@ -8,7 +8,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 SO_PATH = os.environ.get("GENZTOK_LIB") or os.path.join(_HERE, "libgenztok.so")   # GENZTOK_LIB: try another build of the library
 
 MAX_LEN_NONE = -(2 ** 31)
-WANT_TOKEN_TYPE, WANT_SEQUENCE_ID, WANT_SPANS = 1, 2, 4
+WANT_TOKEN_TYPE, WANT_SEQUENCE_ID, WANT_SPANS, WANT_OFFSETS = 1, 2, 4, 8
 NONE, EOS_MARK, PAD_MARK = -1, -3, -4
 
 E_INVALID, E_IO, E_UTF8, E_CUDA, E_NOMEM, E_NODEVICE, E_LIMIT = -1, -2, -3, -4, -5, -6, -7
@@ -21,7 +21,8 @@ class Encoded(C.Structure):
                 ("token_type_ids", C.POINTER(C.c_int8)), ("sequence_id", C.POINTER(C.c_int8)),
                 ("tt_len", C.POINTER(C.c_int32)), ("seq_len", C.POINTER(C.c_int32)),
                 ("row_status", C.POINTER(C.c_uint8)), ("span_off", C.POINTER(C.c_int64)),
-                ("spans", C.POINTER(C.c_int32)), ("real_tokens", C.c_int64), ("_owner", C.c_void_p), ("d2h_bytes", C.c_int64)]
+                ("spans", C.POINTER(C.c_int32)), ("real_tokens", C.c_int64), ("_owner", C.c_void_p), ("d2h_bytes", C.c_int64),
+                ("offsets", C.POINTER(C.c_int32))]
 
 
 class Text(C.Structure):
@@ -31,7 +32,8 @@ class Text(C.Structure):
 
 class DevPlanes(C.Structure):
     _fields_ = [("input_ids", C.c_void_p), ("attention_mask", C.c_void_p), ("token_type_ids", C.c_void_p),
-                ("sequence_id", C.c_void_p), ("row_len", C.c_void_p), ("seq_len", C.c_void_p), ("row_status", C.c_void_p)]
+                ("sequence_id", C.c_void_p), ("row_len", C.c_void_p), ("seq_len", C.c_void_p), ("row_status", C.c_void_p),
+                ("offsets", C.c_void_p)]
 
 
 class Windows(C.Structure):

@@ -178,8 +178,46 @@ __device__ __forceinline__ int32_t sym_to_id(const DevTables& T, uint32_t s, boo
     return final_sym ? T.id_fin[s] : T.id_cont[s];
 }
 
-// One warp per pending cache slot.
-__global__ void __launch_bounds__(256) k_bpe_pending(DevTables T, WordCache C) {
+// Position of the k-th (0-based) set bit of m; m has more than k set bits.
+__device__ __forceinline__ uint32_t nth_set_bit(uint32_t m, uint32_t k) {
+    for (uint32_t t = 0; t < k; t++) m &= m - 1;
+    return (uint32_t)__ffs(m) - 1u;
+}
+
+// offset_mapping: byte length of each of the n final pieces S[0..n) of the word key[0..len), into out[0..n).  Piece i holds the
+// code points k_bpe_single reports for it (sym_ncp, less the 4 of "</w>" on the last piece; an unknown code point is one), cut
+// where bpe_symbols cuts them (at every byte that is not a continuation byte, and at byte 0).  Lane i of each group of 32
+// pieces finds the byte of its past-the-end code point by counting lead bytes from the group's first byte.  All 32 lanes
+// call this; lane i reads only S[i + 32k] (S may alias the arena entry that k_bpe_pending then converts in place).
+__device__ __noinline__ void bpe_piece_lens(const uint32_t* sym_ncp, const uint8_t* key, uint32_t len, const uint32_t* S, uint32_t n, uint16_t* out) {
+    const int lane = threadIdx.x & 31;
+    uint32_t p = 0;                                              // byte of the group's first code point
+    for (uint32_t base = 0; base < n; base += 32) {
+        const uint32_t i = base + lane;
+        uint32_t e = i < n ? (S[i] == SYM_NONE ? 1u : sym_ncp[S[i]] - (i == n - 1 ? 4u : 0u)) : 0u;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(FULL_MASK, e, o); if (lane >= o) e += t; }
+        // e: code points of the group up to my piece's end; the byte where that code point starts ends my piece
+        const uint32_t G = __shfl_sync(FULL_MASK, e, 31);
+        uint32_t be = len;                                       // (a code point past the word's last one starts at len)
+        for (uint32_t q = p, seen = 0; q < len && seen <= G; q += 32) {
+            const uint32_t j = q + lane;
+            const uint32_t m = __ballot_sync(FULL_MASK, j < len && (((key[j] & 0xC0) != 0x80) || j == 0));
+            const uint32_t c = __popc(m);
+            if (e >= seen && e < seen + c) be = q + nth_set_bit(m, e - seen);
+            seen += c;
+        }
+        uint32_t bs = __shfl_up_sync(FULL_MASK, be, 1);          // my piece starts where the one before ends
+        if (lane == 0) bs = p;
+        if (i < n) out[i] = (uint16_t)(be - bs);
+        p = __shfl_sync(FULL_MASK, be, 31);
+    }
+    __syncwarp();
+}
+
+// One warp per pending cache slot.  plen (offset_mapping; NULL when no call on this device has asked for offsets): the byte
+// length of every piece of a VAL_MULTI entry, at the index of its id in tok_arena.
+__global__ void __launch_bounds__(256) k_bpe_pending(DevTables T, WordCache C, uint16_t* plen) {
     pdl_wait(); pdl_trigger();
     __shared__ uint32_t sm_sym[8][BPE_SMEM_SYMS];
     __shared__ uint32_t sm_rank[8][BPE_SMEM_SYMS];
@@ -242,6 +280,8 @@ __global__ void __launch_bounds__(256) k_bpe_pending(DevTables T, WordCache C) {
                 if (lane == 0) off = (uint32_t)atomicAdd(&C.ctr[C_TOKS], (unsigned long long)n + 1);
                 off = __shfl_sync(FULL_MASK, off, 0);
             }
+            // piece lengths first: for a long word S is the arena entry the loop below converts in place
+            if (plen) bpe_piece_lens(T.sym_ncp, key, len, S, n, plen + off + 1);
             // (for a long word S aliases tok_arena + off + 1: each lane converts its own entries in place;
             //  no warp-level sync may sit inside this loop, its trip count differs per lane)
             for (uint32_t i = lane; i < n; i += 32) C.tok_arena[off + 1 + i] = (uint32_t)sym_to_id(T, S[i], i == n - 1);

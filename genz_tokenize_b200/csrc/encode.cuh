@@ -82,6 +82,10 @@ struct RowArgs {
     int32_t* nwA; int32_t* nwB;
     const int64_t* span_off;   // [n_rows+1] first span entry of each row
     int32_t* spans;            // [entries][2]
+    // offset_mapping (RAGGED, k_rows<..., OFFS>): [entries][2] byte (start, end) of each token in its document, aligned with ids.
+    // Only the text's tokens are written: the caller zeroes the plane first, so framing, pads and a forced </s> read (0, 0).
+    int32_t* offs;
+    const uint16_t* plen;      // byte length of every piece in the word cache, at the index of its id in tok_arena (bpe.cuh)
 };
 
 static const int WIN_LANES = 30;            // pieces whose word starts a window handles; 2 more are look-ahead
@@ -471,10 +475,13 @@ __device__ __forceinline__ void seq_words4(const SeqDesc& d, int32_t i0, int32_t
 // All 32 lanes call this.  ts->doff[0..nd] holds the side's document offsets relative to the tile base `tb`
 // (16-byte aligned), ts->dpos[] the next token position of every row.  Tokens at positions < cap (<= limit) are
 // delivered to rowbufs (FIXED) / ts->rg.dout (RAGGED); words of a row that has reached `limit` are not looked up.
-// All byte positions are 32-bit offsets from tb.
-template <int MODE, typename TokT>
+// All byte positions are 32-bit offsets from tb.  OFFS (RAGGED only): also the byte span of every delivered token in its
+// document into offs_out, beside the ids (a word's pieces tile it: their lengths are in plen, beside tok_arena).
+template <int MODE, typename TokT, bool OFFS = false>
 __device__ __forceinline__ void walk_side(const DevTables& T, const WordCache& C, const uint8_t* __restrict__ tb, TileSmem* ts, int nd,
-                                          int lane, int32_t limit, int32_t cap, TokT* rowbufs, int32_t Wp, int32_t* ids_out, bool insert_ok, int32_t* spans, bool count_words) {
+                                          int lane, int32_t limit, int32_t cap, TokT* rowbufs, int32_t Wp, int32_t* ids_out, bool insert_ok, int32_t* spans, bool count_words,
+                                          int32_t* offs_out = nullptr, const uint16_t* plen = nullptr) {
+    static_assert(!OFFS || MODE == MODE_RAGGED, "offsets are written by the ragged pass");
     const int32_t S = ts->doff[0], E = ts->doff[nd];
     if (E <= S) return;
     // documents that are empty share their start with the next one: then the per-piece start bits cannot number
@@ -545,6 +552,7 @@ __device__ __forceinline__ void walk_side(const DevTables& T, const WordCache& C
             int doc = 0x7FFF;
             uint32_t nt = 0, val = 0;
             bool pending = false;
+            int32_t wpos = 0, wlen = 0;                                  // OFFS: the word's first byte (from tb) and its length
             if (has) {
                 const uint32_t wl = ts->wlist[j];
                 const int32_t p = wbase + (int32_t)(wl & 511u);
@@ -574,6 +582,15 @@ __device__ __forceinline__ void walk_side(const DevTables& T, const WordCache& C
                         hit = cache_probe_fast(C, len, k0, k1, k2, hash_key24(k0, k1, k2, len), &val);
                     }
                     if (!hit) val = lookup_slow(C, tb, p, e_doc, insert_ok ? 1 : 0);
+                    if (OFFS) {
+                        wpos = p;
+                        if (hit) wlen = (int32_t)len;
+                        else if ((val & VAL_KIND) == VAL_SINGLE) {            // (a list of pieces carries its lengths: only a single needs the end)
+                            int32_t end = slow_word_end(tb, p + 1, e_doc);
+                            if (end < e_doc && tb[end] == 0x0A) end++;          // \S+\n?  (tokenize.py:106)
+                            wlen = end - p;
+                        }
+                    }
                     const uint32_t kind = val & VAL_KIND;
                     if (kind == VAL_SINGLE) nt = 1;
                     else if (kind == VAL_MULTI) nt = C.tok_arena[val & VAL_PAYLOAD];
@@ -628,16 +645,25 @@ __device__ __forceinline__ void walk_side(const DevTables& T, const WordCache& C
                 if (MODE == MODE_FIXED) { dsts = rowbufs + (size_t)doc * Wp; lim = cap; }
                 else { dstg = ids_out + ts->rg.dout[doc]; lim = ts->rg.dkeep[doc]; }
                 uint32_t fl = 0;
+                // OFFS: byte offsets are relative to the document's first byte (not the tile's or the chunk's)
+                int2* dsto = nullptr;
+                int32_t ob = 0;
+                if (OFFS) { dsto = reinterpret_cast<int2*>(offs_out) + ts->rg.dout[doc]; ob = wpos - ts->doff[doc]; }
                 if ((val & VAL_KIND) == VAL_SINGLE) {                     // (a list of one token is a word that is itself a special id: bpe.cuh)
                     const int32_t t = (int32_t)(val & VAL_PAYLOAD);
                     if (t <= spec_max) { if (t == T.eos || t == T.bos) fl |= F_SPECIAL; if (t == T.pad) fl |= F_PADTOK; }
-                    if (q < lim) { if (MODE == MODE_FIXED) dsts[q] = (TokT)t; else dstg[q] = t; }
+                    if (q < lim) {
+                        if (MODE == MODE_FIXED) dsts[q] = (TokT)t; else dstg[q] = t;
+                        if (OFFS) dsto[q] = make_int2(ob, ob + wlen);
+                    }
                 } else {
                     const uint32_t* src = C.tok_arena + (val & VAL_PAYLOAD) + 1;
+                    const uint16_t* pl = OFFS ? plen + (val & VAL_PAYLOAD) + 1 : nullptr;
                     for (uint32_t i = 0; i < nt && q < lim; i++, q++) {
                         const int32_t t = (int32_t)src[i];
                         if (t <= spec_max) { if (t == T.eos || t == T.bos) fl |= F_SPECIAL; if (t == T.pad) fl |= F_PADTOK; }
                         if (MODE == MODE_FIXED) dsts[q] = (TokT)t; else dstg[q] = t;
+                        if (OFFS) { const int32_t oe = ob + (int32_t)pl[i]; dsto[q] = make_int2(ob, oe); ob = oe; }
                     }
                 }
                 if (fl) atomicOr(&ts->dflag[doc], fl);
@@ -654,7 +680,8 @@ __device__ __forceinline__ void walk_side(const DevTables& T, const WordCache& C
 
 // TokT: type of the rows staged in shared memory (uint16_t when every id fits: half the footprint, twice the blocks).
 // TMA (MODE_FIXED, TokT = int32_t only): the planes are written by tensor stores from a final-form staging area (see TmaPlanes).
-template <int MODE, typename TokT, bool TMA>
+// OFFS (MODE_RAGGED): A.offs receives the tokens' byte offsets (see RowArgs); the other instantiations are unchanged by it.
+template <int MODE, typename TokT, bool TMA, bool OFFS = false>
 __global__ void __launch_bounds__(256, 4) k_rows(DevTables T, WordCache C, RowArgs A, const __grid_constant__ TmaPlanes M) {
     pdl_wait(); pdl_trigger();
     if (A.row_list && C.ctr[C_REDO] == 0) return;                   // second pass with nothing to redo (the usual case): before any set-up
@@ -725,7 +752,7 @@ __global__ void __launch_bounds__(256, 4) k_rows(DevTables T, WordCache C, RowAr
             }
         }
         __syncwarp();
-        walk_side<MODE, TokT>(T, C, A.a.bytes + tbase, ts, nd, lane, limit, cap, rowbufs, Wp, A.ids, insert_ok, A.spans, count_words);
+        walk_side<MODE, TokT, OFFS>(T, C, A.a.bytes + tbase, ts, nd, lane, limit, cap, rowbufs, Wp, A.ids, insert_ok, A.spans, count_words, A.offs, A.plen);
         if (A.has_pair) {
             // ... </s> </s> B   (tokenize.py:237-239)
             if (lane < nd) {
@@ -758,7 +785,7 @@ __global__ void __launch_bounds__(256, 4) k_rows(DevTables T, WordCache C, RowAr
             if (lane <= nd) ts->doff[lane] = (int32_t)(o64 - tbase);
             if (nd == 32 && lane == 0) ts->doff[32] = (int32_t)(p32nd - tbase);
             __syncwarp();
-            walk_side<MODE, TokT>(T, C, A.b.bytes + tbase, ts, nd, lane, limit, cap, rowbufs, Wp, A.ids, insert_ok, A.spans, count_words);
+            walk_side<MODE, TokT, OFFS>(T, C, A.b.bytes + tbase, ts, nd, lane, limit, cap, rowbufs, Wp, A.ids, insert_ok, A.spans, count_words, A.offs, A.plen);
         }
         // ---- closing </s>, row bookkeeping (one lane per row)
         if (lane < nd) {

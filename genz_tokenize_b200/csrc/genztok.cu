@@ -78,6 +78,8 @@ struct DeviceCtx {
     DevBuf ids, mask, tt, seq, row_len, seq_len, tt_len, status;   // outputs
     DevBuf L, keep, out_len, row_off, tail, redo, fix, misc, nwA, nwB, span_cnt, span_off, spans, scan_tmp, prep_out;
     DevBuf slots, key_arena, tok_arena, pending, ctr, rank_scratch;
+    DevBuf len_arena;                             // piece byte lengths beside tok_arena (offset_mapping; allocated on first use)
+    DevBuf offs;                                  // ragged pass: [total][2] token byte offsets (offset_mapping)
     DevBuf dec_lead;                              // decode: per-row description left by the length pass for the write pass
     DevBuf dec_stat;                              // decode, fixed-width rows: ids in front of the pad runs, summed by the length pass
     double dec_avg_lead = -1;                     // ... per row, once the host has read it (-1: not known for the current batch)
@@ -112,8 +114,9 @@ struct DeviceCtx {
     // batch step 1 of genztok_encode_windows_device described, for its step 2
     struct WinState {
         DevBuf ids[2], off[2], count, woff, fix, doc, start;
+        DevBuf offs[2], plane_offs;               // offset_mapping: the streams' token offsets, and the host form's [K, W, 2] plane
         struct { const void *a = nullptr, *a_off = nullptr, *b = nullptr, *b_off = nullptr, *win_off = nullptr; int64_t n = -1, a_bytes = 0, b_bytes = 0;
-                 int32_t W = 0, s = 0; } sig;
+                 int32_t W = 0, s = 0; bool offs = false; } sig;
         int64_t n_win = -1;                       // windows of that batch; -1: no step 1 to continue from
     } win;
     // profiling
@@ -294,6 +297,9 @@ int stream_leave(genztok_t* h, DeviceCtx* d, cudaStream_t st) {
     return GENZTOK_OK;
 }
 
+int launch_guard(genztok_t* h, DeviceCtx* d, cudaStream_t st, int64_t chunk_bytes, int force, uint32_t* z0 = nullptr, uint64_t n0 = 0, uint32_t* z1 = nullptr,
+                 uint64_t n1 = 0);
+
 uint64_t next_pow2(uint64_t x) { uint64_t p = 1; while (p < x) p <<= 1; return p; }
 
 // The word cache is sized for the worst case of ONE chunk (every second byte a new word), so its size follows the largest chunk this
@@ -327,9 +333,22 @@ int ensure_cache(genztok_t* h, DeviceCtx* d, cudaStream_t st, int64_t chunk_byte
     C.pending = d->pending.as<uint32_t>(); C.pending_cap = B / 2 + 64;
     C.ctr = d->ctr.as<unsigned long long>();
     C.rank_scratch = d->rank_scratch.as<uint32_t>(); C.rank_cap = B + 64;
+    if (d->len_arena.p) CU(d->len_arena.ensure((2 * B + 64) * 2));
     d->cache_ready = true;
     d->cache_empty = true;
     d->cache_bytes = B;
+    return GENZTOK_OK;
+}
+
+// offset_mapping needs the byte length of every piece of every cached word (k_bpe_pending records them once len_arena is
+// allocated).  The first call on a device that asks for offsets allocates the lengths and empties the cache, so that every word
+// cached from then on has them; a handle that never asks allocates nothing.  Call after ensure_cache.
+int ensure_piece_lens(genztok_t* h, DeviceCtx* d, cudaStream_t st) {
+    if (d->len_arena.p) return GENZTOK_OK;
+    CU(d->len_arena.ensure((size_t)d->C.tok_cap * 2));
+    int rc = launch_guard(h, d, st, 0, 1);
+    if (rc) return rc;
+    d->cache_empty = true;
     return GENZTOK_OK;
 }
 
@@ -353,7 +372,7 @@ int pick_tile_docs(genztok_t* h, const DeviceCtx* d, int64_t bytes_a, int64_t by
     return D;
 }
 
-template <int MODE, typename TokT, bool TMA>
+template <int MODE, typename TokT, bool TMA, bool OFFS = false>
 int launch_rows_t(genztok_t* h, DeviceCtx* d, const RowArgs& A, cudaStream_t st, const char* name, int64_t n_items_hint, const TmaPlanes* M) {
     const int D = A.row_list ? 1 : A.D;
     auto smem_for = [&](int w) {
@@ -364,7 +383,7 @@ int launch_rows_t(genztok_t* h, DeviceCtx* d, const RowArgs& A, cudaStream_t st,
     while (wpb > 1 && smem_for(wpb) > d->smem_optin) wpb >>= 1;
     const size_t smem = smem_for(wpb);
     if (smem > d->smem_optin) return fail(h, GENZTOK_E_LIMIT, "row of %d ids does not fit shared memory", A.W);
-    auto kern = k_rows<MODE, TokT, TMA>;
+    auto kern = k_rows<MODE, TokT, TMA, OFFS>;
     if (smem > 48 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 1;
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, wpb * 32, smem));
@@ -382,6 +401,7 @@ template <int MODE>
 int launch_rows(genztok_t* h, DeviceCtx* d, const RowArgs& A, cudaStream_t st, const char* name, int64_t n_items_hint, const TmaPlanes* M = nullptr) {
     if (MODE == MODE_FIXED && M) return launch_rows_t<MODE_FIXED, int32_t, true>(h, d, A, st, name, n_items_hint, M);
     if (MODE == MODE_FIXED && narrow_ids(d)) return launch_rows_t<MODE, uint16_t, false>(h, d, A, st, name, n_items_hint, nullptr);
+    if (MODE == MODE_RAGGED && A.offs) return launch_rows_t<MODE_RAGGED, int32_t, false, true>(h, d, A, st, name, n_items_hint, nullptr);
     return launch_rows_t<MODE, int32_t, false>(h, d, A, st, name, n_items_hint, nullptr);
 }
 
@@ -448,8 +468,7 @@ bool setup_tma(genztok_t* h, const DeviceCtx* d, const RowArgs& A, int64_t bytes
 // Can the fixed-layout kernel stage one row of W ids (one document per tile, one warp per block)?
 bool fixed_fits(const DeviceCtx* d, int32_t W) { return sizeof(TileSmem) + row_stage_bytes(d, W, 1) <= d->smem_optin; }
 
-int launch_guard(genztok_t* h, DeviceCtx* d, cudaStream_t st, int64_t chunk_bytes, int force, uint32_t* z0 = nullptr, uint64_t n0 = 0, uint32_t* z1 = nullptr,
-                 uint64_t n1 = 0) {
+int launch_guard(genztok_t* h, DeviceCtx* d, cudaStream_t st, int64_t chunk_bytes, int force, uint32_t* z0, uint64_t n0, uint32_t* z1, uint64_t n1) {
     {
         LaunchScope ls(h, d, "k_cache_guard");
         CU(launch_pdl(k_cache_guard, dim3(1), dim3(1), 0, st, d->C, (unsigned long long)(chunk_bytes / 2 + 2), (unsigned long long)(chunk_bytes + chunk_bytes / 3 + 8), (unsigned long long)(chunk_bytes + chunk_bytes / 2 + 2), force));
@@ -464,7 +483,7 @@ int launch_guard(genztok_t* h, DeviceCtx* d, cudaStream_t st, int64_t chunk_byte
 
 int launch_bpe(genztok_t* h, DeviceCtx* d, cudaStream_t st) {
     LaunchScope ls(h, d, "k_bpe_pending");
-    CU(launch_pdl(k_bpe_pending, dim3(d->sm_count * 6), dim3(256), 0, st, d->T, d->C));      // latency bound (pair-table look-ups): as many warps as fit
+    CU(launch_pdl(k_bpe_pending, dim3(d->sm_count * 6), dim3(256), 0, st, d->T, d->C, d->len_arena.as<uint16_t>()));      // latency bound (pair-table look-ups): as many warps as fit
     CU(cudaGetLastError());
     return GENZTOK_OK;
 }
@@ -733,8 +752,9 @@ int encode_fixed_on_device(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Si
 
 // ---- long documents as windows (window.cuh) -------------------------------------------------------------
 // Token stream of one side: [bos] T [eos] of every document, untruncated, ragged at off[m+1] (the ragged pipeline with max_len
-// None, without the mask and k_post_rows).  Reads the stream's size back to size `ids` (synchronises).
-int token_stream(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& s, int64_t m, DevBuf& ids, DevBuf& off) {
+// None, without the mask and k_post_rows).  Reads the stream's size back to size `ids` (synchronises).  offs: also the tokens'
+// byte offsets, aligned with ids ((0, 0) for the framing).
+int token_stream(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& s, int64_t m, DevBuf& ids, DevBuf& off, DevBuf* offs) {
     CU(d->redo.ensure((size_t)m * 4)); CU(d->fix.ensure((size_t)m * 4));
     CU(d->L.ensure((size_t)m * 4)); CU(d->keep.ensure((size_t)m * 4)); CU(d->out_len.ensure((size_t)m * 8)); CU(d->tail.ensure((size_t)m));
     CU(off.ensure((size_t)(m + 1) * 8));
@@ -762,13 +782,19 @@ int token_stream(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& s, int
     { LaunchScope ls(h, d, "k_reset_lists"); k_reset_lists<<<1, 1, 0, st>>>(d->C); }
     RowArgs E = A;
     E.ids = ids.as<int32_t>(); E.row_off = off.as<int64_t>(); E.keep = d->keep.as<int32_t>();
-    return launch_rows<MODE_RAGGED>(h, d, E, st, "k_rows_ragged", m);
+    if (offs) {
+        CU(offs->ensure((size_t)total * 8 + 16));
+        CU(cudaMemsetAsync(offs->p, 0, (size_t)total * 8, st));
+        E.offs = offs->as<int32_t>(); E.plen = d->len_arena.as<uint16_t>();
+    }
+    return launch_rows<MODE_RAGGED>(h, d, E, st, offs ? "k_rows_ragged_offsets" : "k_rows_ragged", m);
 }
 
 WinArgs window_args(DeviceCtx* d, bool pair, int64_t n, int32_t W, int32_t s) {
     WinArgs A{};
     A.ids_a = d->win.ids[0].as<int32_t>(); A.off_a = d->win.off[0].as<int64_t>();
     if (pair) { A.ids_b = d->win.ids[1].as<int32_t>(); A.off_b = d->win.off[1].as<int64_t>(); }
+    A.offs_a = d->win.offs[0].as<int2>(); A.offs_b = pair ? d->win.offs[1].as<int2>() : nullptr;
     A.n_docs = n; A.W = W; A.stride = s;
     A.ctr = d->C.ctr;
     A.eos_i8 = eos_as_i8(d); A.pad_i8 = pad_as_i8(d);
@@ -776,14 +802,16 @@ WinArgs window_args(DeviceCtx* d, bool pair, int64_t n, int32_t W, int32_t s) {
 }
 
 // Step 1: both token streams, the windows of every document, d_win_off[n+1] and their total (synchronises).  The caller has
-// sized the word cache for the chunk (ensure_cache) and n >= 1.
-int windows_layout(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& a, const Side* b, int64_t n, int32_t W, int32_t s, int64_t* d_win_off,
-                   int64_t* n_win) {
+// sized the word cache for the chunk (ensure_cache) and n >= 1.  offs: the streams carry token offsets too (offset_mapping).
+int windows_layout(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& a, const Side* b, int64_t n, int32_t W, int32_t s, bool offs,
+                   int64_t* d_win_off, int64_t* n_win) {
     d->win.n_win = -1;                                               // the streams are about to change
-    int rc = launch_guard(h, d, st, a.nbytes + (b ? b->nbytes : 0) + 16, 0);
+    int rc = offs ? ensure_piece_lens(h, d, st) : GENZTOK_OK;
     if (rc) return rc;
-    rc = token_stream(h, d, st, a, n, d->win.ids[0], d->win.off[0]);
-    if (!rc && b) rc = token_stream(h, d, st, *b, n, d->win.ids[1], d->win.off[1]);
+    rc = launch_guard(h, d, st, a.nbytes + (b ? b->nbytes : 0) + 16, 0);
+    if (rc) return rc;
+    rc = token_stream(h, d, st, a, n, d->win.ids[0], d->win.off[0], offs ? &d->win.offs[0] : nullptr);
+    if (!rc && b) rc = token_stream(h, d, st, *b, n, d->win.ids[1], d->win.off[1], offs ? &d->win.offs[1] : nullptr);
     if (rc) return rc;
     d->cache_empty = false;
     CU(d->win.count.ensure((size_t)n * 8));
@@ -799,6 +827,7 @@ int windows_layout(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& a, c
 }
 
 // Step 2: the K windows' planes and maps from the streams step 1 left (does not synchronise).  win_doc = doc_base + document.
+// With GENZTOK_WANT_OFFSETS in flags, P.offsets receives [K, W, 2] token offsets (step 1 must have run with offsets).
 int windows_write(genztok_t* h, DeviceCtx* d, cudaStream_t st, bool pair, int64_t n, int32_t W, int32_t s, uint32_t flags, const int64_t* d_win_off,
                   int64_t K, const genztok_dev_planes_t& P, int64_t* win_doc, int32_t* win_start, int64_t doc_base) {
     if (K <= 0) return GENZTOK_OK;
@@ -814,15 +843,22 @@ int windows_write(genztok_t* h, DeviceCtx* d, cudaStream_t st, bool pair, int64_
         A.seq_len = P.seq_len; A.status = P.row_status;
     }
     A.win_doc = win_doc; A.win_start = win_start; A.fix_list = d->win.fix.as<uint32_t>();
+    const bool offs = (flags & GENZTOK_WANT_OFFSETS) != 0;            // (P.offsets is read only then: older callers' structs end before it)
+    if (offs) A.offs = P.offsets;
     auto aligned = [](const void* p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) == 0; };
-    const bool quad = (W & 3) == 0 && aligned(A.ids, 16) && aligned(A.mask, 4) && aligned(A.tt, 4) && aligned(A.seq, 4);
+    const bool quad = (W & 3) == 0 && aligned(A.ids, 16) && aligned(A.mask, 4) && aligned(A.tt, 4) && aligned(A.seq, 4) && aligned(A.offs, 16);
     const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((K + 7) / 8, (int64_t)d->sm_count * 8));
     {
         // algorithmic bytes: the planes and per-window values written (the windows' tokens are read from the streams, mostly in L2)
-        const int64_t alg = K * (int64_t)W * (5 + (A.tt ? 1 : 0) + (A.seq ? 1 : 0)) + K * (4 + 8 + 4 + (pair ? 5 : 0));
-        LaunchScope ls(h, d, "k_window_rows", alg);
-        if (pair) { if (quad) k_window_rows<true, true><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, true><<<grid, 256, 0, st>>>(d->T, A); }
-        else { if (quad) k_window_rows<true, false><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, false><<<grid, 256, 0, st>>>(d->T, A); }
+        const int64_t alg = K * (int64_t)W * (5 + (A.tt ? 1 : 0) + (A.seq ? 1 : 0) + (offs ? 8 : 0)) + K * (4 + 8 + 4 + (pair ? 5 : 0));
+        LaunchScope ls(h, d, offs ? "k_window_rows_offsets" : "k_window_rows", alg);
+        if (offs) {
+            if (pair) { if (quad) k_window_rows<true, true, true><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, true, true><<<grid, 256, 0, st>>>(d->T, A); }
+            else { if (quad) k_window_rows<true, false, true><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, false, true><<<grid, 256, 0, st>>>(d->T, A); }
+        } else {
+            if (pair) { if (quad) k_window_rows<true, true><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, true><<<grid, 256, 0, st>>>(d->T, A); }
+            else { if (quad) k_window_rows<true, false><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, false><<<grid, 256, 0, st>>>(d->T, A); }
+        }
     }
     CU(cudaGetLastError());
     if (pair && (A.tt || A.seq || A.seq_len || A.status)) {
@@ -913,7 +949,7 @@ struct Mode { bool fixed; bool has_max_len; int32_t max_len; int padding, trunca
 // ================================================================================================
 extern "C" {
 
-const char* genztok_version(void) { return "genztok-b200 0.1 (sm_100a)"; }
+const char* genztok_version(void) { return "genztok-b200 0.2 (sm_100a)"; }
 
 const char* genztok_last_error(const genztok_t* h) { return h ? h->err.c_str() : g_create_err.c_str(); }
 
@@ -1141,6 +1177,7 @@ int genztok_encode_device(genztok_t* h, int dev, const uint8_t* d_text, const in
                           const int64_t* d_pair_off, int64_t pair_bytes, int64_t n, int32_t max_len, uint32_t flags,
                           const genztok_dev_planes_t* planes, void* stream) {
     if (!h) return GENZTOK_E_INVALID;
+    if (flags & GENZTOK_WANT_OFFSETS) return fail(h, GENZTOK_E_INVALID, "offsets are not available in the fixed device layout; use genztok_encode_windows_device");
     if (dev < 0 || dev >= (int)h->devs.size()) return fail(h, GENZTOK_E_NODEVICE, "no such device slot %d (handle has %d)", dev, (int)h->devs.size());
     if (!planes || !planes->input_ids || n < 0 || !d_text_off || (text_bytes > 0 && !d_text)) return fail(h, GENZTOK_E_INVALID, "genztok_encode_device: bad arguments");
     if (max_len < 1) return fail(h, GENZTOK_E_INVALID, "genztok_encode_device needs max_len >= 1 (fixed layout)");
@@ -1180,6 +1217,7 @@ struct EncodeJob {
     const uint8_t* text; const int64_t* text_off; const uint8_t* pair; const int64_t* pair_off;
     int32_t max_len; int padding, truncation; uint32_t flags;
     bool has_pair, has_max_len, want_spans, fixed, want_tt, want_seq;
+    bool want_offs;                // offset_mapping: the ragged pipeline writes token offsets beside the ids
     genztok_encoded_t* out;
     int32_t old_dirty[4];          // fixed layout: columns of the result planes (ids, mask, token types, sequence ids) that may hold something
                                    // other than padding from the buffer's last use (the width: unknown / a fresh buffer)
@@ -1189,10 +1227,10 @@ struct EncodePart {
     std::string err;
     int32_t extent = 0;            // fixed layout: columns that can differ from padding, max over this part's chunks
     int64_t d2h_bytes = 0;
-    PinnedVec<int32_t> ids, spans; PinnedVec<uint8_t> mask; PinnedVec<int8_t> tt, seq;
+    PinnedVec<int32_t> ids, spans, tok_offs; PinnedVec<uint8_t> mask; PinnedVec<int8_t> tt, seq;
     PinnedVec<int64_t> offs, soffs;   // a chunk's row / span offsets on their way home (pinned: a copy into pageable memory is staged by the driver)
     int64_t total = 0, span_total = 0, tokens = 0;
-    void bind(genztok_t* h) { ids.h = h; spans.h = h; mask.h = h; tt.h = h; seq.h = h; offs.h = h; soffs.h = h; }
+    void bind(genztok_t* h) { ids.h = h; spans.h = h; tok_offs.h = h; mask.h = h; tt.h = h; seq.h = h; offs.h = h; soffs.h = h; }
 };
 
 // Chunk boundaries of rows [rb, re): rows [cuts[i], cuts[i+1]) with at most chunk_rows rows and max_chunk_bytes bytes; *most = the
@@ -1233,6 +1271,7 @@ void encode_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int64
     { const int64_t big = chunk_cuts(h, J, rb, re, &cuts, &most);
       if (big >= 0) PFAIL(GENZTOK_E_LIMIT, "document %lld is larger than max_chunk_bytes=%lld", (long long)big, (long long)h->max_chunk_bytes) }
     FAIL_RC(ensure_cache(h, d, st, most));
+    if (J.want_offs) FAIL_RC(ensure_piece_lens(h, d, st));
     unsigned long long tokens_before = 0;
     CUF(cudaMemcpyAsync(&tokens_before, d->C.ctr + C_TOKENS, 8, cudaMemcpyDeviceToHost, st));
     CUF(cudaStreamSynchronize(st));
@@ -1413,7 +1452,12 @@ void encode_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int64
         RowArgs E = A;
         E.ids = d->ids.as<int32_t>(); E.row_off = d->row_off.as<int64_t>(); E.keep = d->keep.as<int32_t>();
         if (want_spans) { E.span_off = d->span_off.as<int64_t>(); E.spans = d->spans.as<int32_t>(); }
-        FAIL_RC(launch_rows<MODE_RAGGED>(h, d, E, st, "k_rows_ragged", m));
+        if (J.want_offs) {                                          // framing, pads and a forced </s> keep the (0, 0) of the memset
+            CUF(d->offs.ensure((size_t)total * 8 + 16));
+            CUF(cudaMemsetAsync(d->offs.p, 0, (size_t)total * 8, st));
+            E.offs = d->offs.as<int32_t>(); E.plen = d->len_arena.as<uint16_t>();
+        }
+        FAIL_RC(launch_rows<MODE_RAGGED>(h, d, E, st, J.want_offs ? "k_rows_ragged_offsets" : "k_rows_ragged", m));
         PostArgs Q{};
         Q.ids = d->ids.as<int32_t>(); Q.row_off = d->row_off.as<int64_t>(); Q.n_rows = m; Q.keep = d->keep.as<int32_t>(); Q.tail = d->tail.as<uint8_t>();
         Q.mask = d->mask.as<uint8_t>(); Q.has_pair = has_pair; Q.row_len = d->row_len.as<int32_t>();
@@ -1428,10 +1472,12 @@ void encode_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int64
             const size_t est = (size_t)((double)total * (double)(re - rb) / (double)m * 1.125) + 4096;
             bool ok = part->ids.reserve(est) && part->mask.reserve(est);
             if (has_pair) ok = ok && part->tt.reserve(est) && part->seq.reserve(est);
+            if (J.want_offs) ok = ok && part->tok_offs.reserve(2 * est);
             if (!ok) PFAIL(GENZTOK_E_NOMEM, "pinned host allocation failed")
         }
         bool grown = part->ids.resize(old + (size_t)total) && part->mask.resize(old + (size_t)total);
         if (has_pair) grown = grown && part->tt.resize(old + (size_t)total) && part->seq.resize(old + (size_t)total);
+        if (J.want_offs) grown = grown && part->tok_offs.resize(2 * (old + (size_t)total));
         grown = grown && part->offs.resize((size_t)m + 1);
         if (!grown) PFAIL(GENZTOK_E_NOMEM, "pinned host allocation failed")
         int64_t* const offs = part->offs.data();
@@ -1442,6 +1488,7 @@ void encode_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int64
                 CUF(cudaMemcpyAsync(part->tt.data() + old, d->tt.p, (size_t)total, cudaMemcpyDeviceToHost, st));
                 CUF(cudaMemcpyAsync(part->seq.data() + old, d->seq.p, (size_t)total, cudaMemcpyDeviceToHost, st));
             }
+            if (J.want_offs) CUF(cudaMemcpyAsync(part->tok_offs.data() + 2 * old, d->offs.p, (size_t)total * 8, cudaMemcpyDeviceToHost, st));
         }
         int64_t* soffs = nullptr;
         if (want_spans) {
@@ -1461,7 +1508,7 @@ void encode_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int64
             CUF(cudaMemcpyAsync(out->row_status + r0, d->status.p, (size_t)m, cudaMemcpyDeviceToHost, st));
         }
         CUF(cudaStreamSynchronize(st));
-        part->d2h_bytes += total * (has_pair ? 7 : 5) + (m + 1) * 8 + m * (has_pair ? 13 : 4) + (want_spans ? span_n * 8 + (m + 1) * 8 : 0);
+        part->d2h_bytes += total * (has_pair ? 7 : 5) + (m + 1) * 8 + m * (has_pair ? 13 : 4) + (want_spans ? span_n * 8 + (m + 1) * 8 : 0) + (J.want_offs ? total * 8 : 0);
         for (int64_t i = 1; i <= m; i++) out->row_off[r0 + i] = part->total + offs[i];      // relative to the part
         part->total += total;
         if (want_spans) { for (int64_t i = 1; i <= m; i++) out->span_off[r0 + i] = part->span_total + soffs[i]; part->span_total += span_n; }
@@ -1494,7 +1541,11 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
     J.has_pair = pair_off != nullptr;
     J.has_max_len = max_len != GENZTOK_MAX_LEN_NONE;
     J.want_spans = (flags & GENZTOK_WANT_SPANS) != 0;       // return_offset: produced by the ragged pipeline
-    J.fixed = J.has_max_len && max_len >= 1 && padding && truncation && fixed_fits(h->devs[0], max_len) && !J.want_spans;
+    J.want_offs = (flags & GENZTOK_WANT_OFFSETS) != 0;      // offset_mapping: produced by the ragged pipeline too
+    // the fixed regime; with offsets it is computed by the ragged pipeline, whose rows then all hold max_len entries, and
+    // presented in the fixed layout
+    const bool fixed_layout = J.has_max_len && max_len >= 1 && padding && truncation && fixed_fits(h->devs[0], max_len) && !J.want_spans;
+    J.fixed = fixed_layout && !J.want_offs;
     J.want_tt = J.has_pair && (flags & GENZTOK_WANT_TOKEN_TYPE);
     J.want_seq = J.has_pair && (flags & GENZTOK_WANT_SEQUENCE_ID);
     const bool has_pair = J.has_pair, fixed = J.fixed;
@@ -1506,6 +1557,17 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
         for (void* p : ob->mallocs) free(p);
         delete ob;
         memset(out, 0, sizeof *out);
+    };
+    // offsets in the fixed regime: every row of the ragged result is a padded / truncated row of max_len entries
+    auto present_fixed = [&]() -> int {
+        if (out->row_off[n] != n * (int64_t)max_len) {
+            free_nolock();
+            return fail(h, GENZTOK_E_CUDA, "internal error: fixed-regime rows do not hold max_len entries");
+        }
+        out->width = max_len; out->row_off = nullptr;
+        if (!J.want_tt) { out->token_type_ids = nullptr; out->tt_len = nullptr; }   // the planes the fixed layout leaves out
+        if (!J.want_seq) out->sequence_id = nullptr;
+        return GENZTOK_OK;
     };
 #define OOM_CHECK(p) if (!(p)) { free_nolock(); return fail(h, GENZTOK_E_NOMEM, "pinned host allocation failed"); }
     if (J.want_spans) { out->span_off = out_alloc<int64_t>(h, ob, (size_t)n + 1); OOM_CHECK(out->span_off); out->span_off[0] = 0; }
@@ -1592,6 +1654,7 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
                 out->input_ids = adopt(pt.ids); out->attention_mask = adopt(pt.mask);
                 if (has_pair) { out->token_type_ids = adopt(pt.tt); out->sequence_id = adopt(pt.seq); }
                 if (J.want_spans) out->spans = adopt(pt.spans);
+                if (J.want_offs) out->offsets = adopt(pt.tok_offs);
             }
             auto some = [&](size_t bytes) { void* q = malloc(bytes); ob->mallocs.push_back(q); return q; };   // (empty planes still get an address)
             if (!out->input_ids) out->input_ids = (int32_t*)some(16);
@@ -1599,13 +1662,16 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
             if (has_pair && !out->token_type_ids) out->token_type_ids = (int8_t*)some(16);
             if (has_pair && !out->sequence_id) out->sequence_id = (int8_t*)some(16);
             if (J.want_spans && !out->spans) out->spans = (int32_t*)some(16);
-            return GENZTOK_OK;
+            if (J.want_offs && !out->offsets) out->offsets = (int32_t*)some(16);
+            return fixed_layout ? present_fixed() : GENZTOK_OK;
         }
         int32_t* ids = (int32_t*)malloc(std::max<size_t>(ntot * 4, 16)); ob->mallocs.push_back(ids);
         uint8_t* mask = (uint8_t*)malloc(std::max<size_t>(ntot, 16)); ob->mallocs.push_back(mask);
         int8_t *tt = nullptr, *seq = nullptr; int32_t* spans = nullptr;
         if (has_pair) { tt = (int8_t*)malloc(std::max<size_t>(ntot, 16)); ob->mallocs.push_back(tt); seq = (int8_t*)malloc(std::max<size_t>(ntot, 16)); ob->mallocs.push_back(seq); }
         if (J.want_spans) { spans = (int32_t*)malloc(std::max<size_t>(stot * 4, 16)); ob->mallocs.push_back(spans); }
+        int32_t* toffs = nullptr;
+        if (J.want_offs) { toffs = (int32_t*)malloc(std::max<size_t>(ntot * 8, 16)); ob->mallocs.push_back(toffs); }
         for (int g = 0; g < G; g++) {
             EncodePart& pt = parts[(size_t)g];
             const int64_t rb = (G == 1 || n < 2 * G) ? (g == 0 ? 0 : n) : dcut[(size_t)g], re = (G == 1 || n < 2 * G) ? n : dcut[(size_t)g + 1];
@@ -1615,12 +1681,15 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
                 memcpy(ids + base, pt.ids.data(), pt.ids.size() * 4);
                 memcpy(mask + base, pt.mask.data(), pt.mask.size());
                 if (has_pair) { memcpy(tt + base, pt.tt.data(), pt.tt.size()); memcpy(seq + base, pt.seq.data(), pt.seq.size()); }
+                if (J.want_offs) memcpy(toffs + 2 * base, pt.tok_offs.data(), pt.ids.size() * 8);
             }
             if (J.want_spans && !pt.spans.empty()) memcpy(spans + 2 * sbase, pt.spans.data(), pt.spans.size() * 4);
             base += pt.total; sbase += pt.span_total;
         }
         out->total = base;
         out->input_ids = ids; out->attention_mask = mask; out->token_type_ids = tt; out->sequence_id = seq; out->spans = spans;
+        out->offsets = toffs;
+        if (fixed_layout) return present_fixed();
     }
     return GENZTOK_OK;
 }
@@ -1634,8 +1703,8 @@ struct WindowPart {
     int rc = GENZTOK_OK;
     std::string err;
     int64_t n_win = 0, tokens = 0, d2h_bytes = 0;
-    PinnedVec<int32_t> ids, row_len, seq_len, start; PinnedVec<uint8_t> mask, status; PinnedVec<int8_t> tt, seq; PinnedVec<int64_t> doc, offs;
-    void bind(genztok_t* h) { for (auto* v : {&ids, &row_len, &seq_len, &start}) v->h = h; mask.h = h; status.h = h; tt.h = h; seq.h = h; doc.h = h; offs.h = h; }
+    PinnedVec<int32_t> ids, row_len, seq_len, start, tok_offs; PinnedVec<uint8_t> mask, status; PinnedVec<int8_t> tt, seq; PinnedVec<int64_t> doc, offs;
+    void bind(genztok_t* h) { for (auto* v : {&ids, &row_len, &seq_len, &start, &tok_offs}) v->h = h; mask.h = h; status.h = h; tt.h = h; seq.h = h; doc.h = h; offs.h = h; }
 };
 
 // Windows of documents [rb, re) on one device: per chunk the text goes up, both steps run, the planes and maps come home.
@@ -1675,7 +1744,7 @@ void windows_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int3
         Side b{has_pair ? d->pair.as<uint8_t>() + pa - pb0 : nullptr, d->poff.as<int64_t>(), pb};
         CUF(d->win.woff.ensure((size_t)(m + 1) * 8));
         int64_t K = 0;
-        FAIL_RC(windows_layout(h, d, st, a, has_pair ? &b : nullptr, m, W, stride, d->win.woff.as<int64_t>(), &K));
+        FAIL_RC(windows_layout(h, d, st, a, has_pair ? &b : nullptr, m, W, stride, J.want_offs, d->win.woff.as<int64_t>(), &K));
         const size_t tot = (size_t)K * (size_t)W;
         CUF(d->ids.ensure(tot * 4 + 16)); CUF(d->mask.ensure(tot + 16)); CUF(d->row_len.ensure((size_t)K * 4 + 16));
         CUF(d->win.doc.ensure((size_t)K * 8 + 16)); CUF(d->win.start.ensure((size_t)K * 4 + 16));
@@ -1684,6 +1753,7 @@ void windows_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int3
         if (J.want_tt) { CUF(d->tt.ensure(tot + 16)); P.token_type_ids = d->tt.as<int8_t>(); }
         if (J.want_seq) { CUF(d->seq.ensure(tot + 16)); P.sequence_id = d->seq.as<int8_t>(); }
         if (has_pair) { CUF(d->seq_len.ensure((size_t)K * 4 + 16)); CUF(d->status.ensure((size_t)K + 16)); P.seq_len = d->seq_len.as<int32_t>(); P.row_status = d->status.as<uint8_t>(); }
+        if (J.want_offs) { CUF(d->win.plane_offs.ensure(tot * 8 + 16)); P.offsets = d->win.plane_offs.as<int32_t>(); }
         FAIL_RC(windows_write(h, d, st, has_pair, m, W, stride, J.flags, d->win.woff.as<int64_t>(), K, P, d->win.doc.as<int64_t>(), d->win.start.as<int32_t>(), r0));
         const size_t o = (size_t)part->n_win, n1 = o + (size_t)K;
         if (ci == 0 && r1 < re) {                                    // first chunk of several: room for the part at this chunk's windows per document (+ 12 %)
@@ -1691,6 +1761,7 @@ void windows_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int3
             bool ok = part->ids.reserve(est * W) && part->mask.reserve(est * W) && part->row_len.reserve(est) && part->doc.reserve(est) && part->start.reserve(est);
             if (J.want_tt) ok = ok && part->tt.reserve(est * W);
             if (J.want_seq) ok = ok && part->seq.reserve(est * W);
+            if (J.want_offs) ok = ok && part->tok_offs.reserve(2 * est * W);
             if (has_pair) ok = ok && part->seq_len.reserve(est) && part->status.reserve(est);
             if (!ok) PFAIL(GENZTOK_E_NOMEM, "pinned host allocation failed")
         }
@@ -1698,6 +1769,7 @@ void windows_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int3
                      part->offs.resize((size_t)m + 1);
         if (J.want_tt) grown = grown && part->tt.resize(n1 * W);
         if (J.want_seq) grown = grown && part->seq.resize(n1 * W);
+        if (J.want_offs) grown = grown && part->tok_offs.resize(2 * n1 * W);
         if (has_pair) grown = grown && part->seq_len.resize(n1) && part->status.resize(n1);
         if (!grown) PFAIL(GENZTOK_E_NOMEM, "pinned host allocation failed")
         if (K) {
@@ -1705,6 +1777,7 @@ void windows_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int3
             CUF(cudaMemcpyAsync(part->mask.data() + o * W, P.attention_mask, tot, cudaMemcpyDeviceToHost, st));
             if (J.want_tt) CUF(cudaMemcpyAsync(part->tt.data() + o * W, P.token_type_ids, tot, cudaMemcpyDeviceToHost, st));
             if (J.want_seq) CUF(cudaMemcpyAsync(part->seq.data() + o * W, P.sequence_id, tot, cudaMemcpyDeviceToHost, st));
+            if (J.want_offs) CUF(cudaMemcpyAsync(part->tok_offs.data() + 2 * o * W, P.offsets, tot * 8, cudaMemcpyDeviceToHost, st));
             CUF(cudaMemcpyAsync(part->row_len.data() + o, P.row_len, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
             CUF(cudaMemcpyAsync(part->doc.data() + o, d->win.doc.p, (size_t)K * 8, cudaMemcpyDeviceToHost, st));
             CUF(cudaMemcpyAsync(part->start.data() + o, d->win.start.p, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
@@ -1715,7 +1788,7 @@ void windows_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int3
         }
         CUF(cudaMemcpyAsync(part->offs.data(), d->win.woff.p, (size_t)(m + 1) * 8, cudaMemcpyDeviceToHost, st));
         CUF(cudaStreamSynchronize(st));
-        part->d2h_bytes += (int64_t)tot * (5 + (J.want_tt ? 1 : 0) + (J.want_seq ? 1 : 0)) + K * (16 + (has_pair ? 5 : 0)) + (m + 1) * 8;
+        part->d2h_bytes += (int64_t)tot * (5 + (J.want_tt ? 1 : 0) + (J.want_seq ? 1 : 0) + (J.want_offs ? 8 : 0)) + K * (16 + (has_pair ? 5 : 0)) + (m + 1) * 8;
         const int64_t* offs = part->offs.data();
         for (int64_t i = 1; i <= m; i++) win_off[r0 + i] = part->n_win + offs[i];
         part->n_win += K;
@@ -1756,6 +1829,7 @@ int genztok_encode_windows(genztok_t* h, const uint8_t* text, const int64_t* tex
     J.text = text; J.text_off = text_off; J.pair = pair; J.pair_off = pair_off;
     J.max_len = max_len; J.padding = 1; J.truncation = 1; J.flags = flags;
     J.has_pair = pair_off != nullptr; J.has_max_len = true; J.fixed = true;
+    J.want_offs = (flags & GENZTOK_WANT_OFFSETS) != 0;
     J.want_tt = J.has_pair && (flags & GENZTOK_WANT_TOKEN_TYPE);
     J.want_seq = J.has_pair && (flags & GENZTOK_WANT_SEQUENCE_ID);
     const bool has_pair = J.has_pair;
@@ -1810,6 +1884,7 @@ int genztok_encode_windows(genztok_t* h, const uint8_t* text, const int64_t* tex
     bool ok = E.input_ids && E.attention_mask && E.row_len && out->win_doc && out->win_start;
     if (J.want_tt) { E.token_type_ids = take(out_alloc<int8_t>(h, ob, tot)); E.tt_len = take(out_alloc<int32_t>(h, ob, (size_t)K)); ok = ok && E.token_type_ids && E.tt_len; }
     if (J.want_seq) { E.sequence_id = take(out_alloc<int8_t>(h, ob, tot)); ok = ok && E.sequence_id; }
+    if (J.want_offs) { E.offsets = take(out_alloc<int32_t>(h, ob, 2 * tot)); ok = ok && E.offsets; }
     if (has_pair) { E.seq_len = take(out_alloc<int32_t>(h, ob, (size_t)K)); E.row_status = take(out_alloc<uint8_t>(h, ob, (size_t)K)); ok = ok && E.seq_len && E.row_status; }
     if (!ok) return bail(fail(h, GENZTOK_E_NOMEM, "pinned host allocation failed"));
     // stitch the parts in document order; their window offsets are shifted by the windows before them
@@ -1826,6 +1901,7 @@ int genztok_encode_windows(genztok_t* h, const uint8_t* text, const int64_t* tex
             memcpy(out->win_start + o, pt.start.data(), k * 4);
             if (J.want_tt) memcpy(E.token_type_ids + o * w, pt.tt.data(), k * w);
             if (J.want_seq) memcpy(E.sequence_id + o * w, pt.seq.data(), k * w);
+            if (J.want_offs) memcpy(E.offsets + 2 * o * w, pt.tok_offs.data(), k * w * 8);
             if (has_pair) { memcpy(E.seq_len + o, pt.seq_len.data(), k * 4); memcpy(E.row_status + o, pt.status.data(), k); }
         }
         base += pt.n_win;
@@ -1864,9 +1940,10 @@ int genztok_encode_windows_device(genztok_t* h, int dev, const uint8_t* d_text, 
     const int64_t bytes = text_bytes + (has_pair ? pair_bytes : 0);
     if (bytes > h->max_chunk_bytes) return fail(h, GENZTOK_E_LIMIT, "chunk of %lld bytes exceeds max_chunk_bytes=%lld", (long long)bytes, (long long)h->max_chunk_bytes);
     DeviceCtx::WinState& S = d->win;
+    const bool offs = (flags & GENZTOK_WANT_OFFSETS) != 0;
     const bool same = S.n_win >= 0 && S.sig.a == d_text && S.sig.a_off == d_text_off && S.sig.b == d_pair && S.sig.b_off == d_pair_off &&
                       S.sig.win_off == d_win_off && S.sig.n == n && S.sig.a_bytes == text_bytes && S.sig.b_bytes == (has_pair ? pair_bytes : 0) &&
-                      S.sig.W == max_len && S.sig.s == stride;
+                      S.sig.W == max_len && S.sig.s == stride && S.sig.offs == offs;
     rc = stream_enter(h, d, st);
     if (rc) return rc;
     if (!planes || !same) {
@@ -1876,17 +1953,18 @@ int genztok_encode_windows_device(genztok_t* h, int dev, const uint8_t* d_text, 
             rc = ensure_cache(h, d, st, bytes + 32);
             if (rc) return rc;
             Side a{d_text, d_text_off, text_bytes}, b{d_pair, d_pair_off, pair_bytes};
-            rc = windows_layout(h, d, st, a, has_pair ? &b : nullptr, n, max_len, stride, d_win_off, &K);
+            rc = windows_layout(h, d, st, a, has_pair ? &b : nullptr, n, max_len, stride, offs, d_win_off, &K);
             if (rc) return rc;
         }
         S.n_win = K;
         S.sig.a = d_text; S.sig.a_off = d_text_off; S.sig.b = d_pair; S.sig.b_off = d_pair_off; S.sig.win_off = d_win_off;
-        S.sig.n = n; S.sig.a_bytes = text_bytes; S.sig.b_bytes = has_pair ? pair_bytes : 0; S.sig.W = max_len; S.sig.s = stride;
+        S.sig.n = n; S.sig.a_bytes = text_bytes; S.sig.b_bytes = has_pair ? pair_bytes : 0; S.sig.W = max_len; S.sig.s = stride; S.sig.offs = offs;
     }
     if (n_windows) *n_windows = S.n_win;
     if (planes) {
         if (S.n_win > 0 && (!planes->input_ids || !planes->attention_mask || !planes->row_len || !d_win_doc || !d_win_start))
             return fail(h, GENZTOK_E_INVALID, "genztok_encode_windows_device: step 2 needs input_ids, attention_mask, row_len and the two maps");
+        if (S.n_win > 0 && offs && !planes->offsets) return fail(h, GENZTOK_E_INVALID, "genztok_encode_windows_device: GENZTOK_WANT_OFFSETS needs planes->offsets");
         rc = windows_write(h, d, st, has_pair, n, max_len, stride, flags, d_win_off, S.n_win, *planes, d_win_doc, d_win_start, 0);
         if (rc) return rc;
     }

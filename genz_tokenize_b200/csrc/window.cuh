@@ -30,6 +30,10 @@ struct WinArgs {
     uint32_t* fix_list;                           // pair windows for k_post_rows (count at ctr[C_FIX])
     unsigned long long* ctr;                      // the word cache's counters: C_FIX, C_ERR, C_TOKENS
     int8_t eos_i8, pad_i8;
+    // offset_mapping (k_window_rows<..., OFFS>): byte (start, end) per token of the streams, aligned with ids_a / ids_b, and the
+    // [n_win, W, 2] plane they are cut into
+    const int2* offs_a; const int2* offs_b;
+    int32_t* offs;
 };
 
 // Windows of one document.  L: tokens of the windowed text, LA: tokens of the first text (pairs).
@@ -51,7 +55,9 @@ __global__ void __launch_bounds__(256) k_window_count(WinArgs A) {
 
 // One warp per window.  QUAD (W % 4 == 0, planes 16-byte aligned): a lane owns 4 consecutive columns and writes them with one
 // 16-byte store of ids and one 4-byte store per byte plane; the pad run needs no loads.  Otherwise a lane owns one column.
-template <bool QUAD, bool PAIR>
+// OFFS: the offsets plane too, taken from the streams where the ids are (first text, windowed slice) and (0, 0) elsewhere;
+// QUAD writes a lane's 4 columns (32 bytes) with two 16-byte stores.
+template <bool QUAD, bool PAIR, bool OFFS = false>
 __global__ void __launch_bounds__(256) k_window_rows(DevTables T, WinArgs A) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -81,6 +87,15 @@ __global__ void __launch_bounds__(256) k_window_rows(DevTables T, WinArgs A) {
         const int32_t Lr = trunc ? W : Lf;
         const int32_t* srcA = A.ids_a + oa;                           // srcA[i] = A[i - 1] for columns 1..LA
         const int32_t* srcX = (PAIR ? A.ids_b : A.ids_a) + ox + 1 + st - pb;   // srcX[i] = T[st + i - pb] for columns pb..e-1
+        const int2* osrcA = OFFS ? A.offs_a + oa : nullptr;          // the same columns of the offsets streams
+        const int2* osrcX = OFFS ? (PAIR ? A.offs_b : A.offs_a) + ox + 1 + st - pb : nullptr;
+        auto offset = [&](int32_t i) -> int2 {                       // (0, 0): <s>, </s>, pads, the </s> of a truncated row
+            if (i == 0 || (trunc && i == W - 1)) return make_int2(0, 0);
+            if (PAIR && i <= LA) return osrcA[i];
+            if (PAIR && i < pb) return make_int2(0, 0);
+            if (i < e) return osrcX[i];
+            return make_int2(0, 0);
+        };
         SeqDesc sd;
         if (PAIR) sd = seq_describe(LA, Lf, W);
         bool special = false;
@@ -106,6 +121,16 @@ __global__ void __launch_bounds__(256) k_window_rows(DevTables T, WinArgs A) {
                 }
                 st_cs128(A.ids + g0 + i0, v);
                 st_cs32(A.mask + g0 + i0, mk);
+                if (OFFS) {
+                    uint4 o0 = make_uint4(0, 0, 0, 0), o1 = o0;
+                    if (i0 < Lr) {
+                        const int2 a = offset(i0), b = offset(i0 + 1), c = offset(i0 + 2), d4 = offset(i0 + 3);
+                        o0 = make_uint4((uint32_t)a.x, (uint32_t)a.y, (uint32_t)b.x, (uint32_t)b.y);
+                        o1 = make_uint4((uint32_t)c.x, (uint32_t)c.y, (uint32_t)d4.x, (uint32_t)d4.y);
+                    }
+                    st_cs128(A.offs + 2 * (g0 + i0), o0);
+                    st_cs128(A.offs + 2 * (g0 + i0) + 4, o1);
+                }
                 if (PAIR && (A.tt || A.seq)) {
                     uint32_t ttw, sqw;
                     seq_words4(sd, i0, W, A.eos_i8, A.pad_i8, &ttw, &sqw);
@@ -118,6 +143,7 @@ __global__ void __launch_bounds__(256) k_window_rows(DevTables T, WinArgs A) {
                 const int32_t v = i < Lr ? value(i) : T.pad;
                 A.ids[g0 + i] = v;
                 A.mask[g0 + i] = (uint8_t)(v != T.pad);
+                if (OFFS) reinterpret_cast<int2*>(A.offs)[g0 + i] = i < Lr ? offset(i) : make_int2(0, 0);
                 tok_total += (uint32_t)(v != T.pad);
                 if (PAIR) {
                     const int32_t sv = i < sd.m ? seq_value(sd, i) : (int32_t)A.pad_i8;

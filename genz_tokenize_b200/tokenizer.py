@@ -6,7 +6,9 @@ B200 -- there is no CPU path, and a handle without a device raises.
 Extensions over the reference (which is one string per call): `encode_batch` / `decode_batch`
 (numpy in, numpy out through pinned host buffers), `encode_device` / `decode_device`
 (torch CUDA tensors in and out, DLPack-exportable, nothing crosses PCIe) and `encode_windows` /
-`encode_windows_device` (long documents as overlapping max_len windows, every token kept).
+`encode_windows_device` (long documents as overlapping max_len windows, every token kept).  Every encode
+form but encode_device can also return `offset_mapping` (HF's return_offsets_mapping): each token's
+(start, end) byte range in its own document's UTF-8 text, (0, 0) for tokens that are not from the text.
 """
 import ctypes as C
 import operator
@@ -328,8 +330,9 @@ class Tokenize(object):
             out.append(v)
         return np.asarray(out, dtype=np.int32).reshape(-1)
 
-    def __call__(self, text, pair_text=None, max_len=None, padding=True, truncation=True, return_offset=False, **kw):
-        """tokenize.py:184-259.  `text_pair=` is accepted as an alias of `pair_text`."""
+    def __call__(self, text, pair_text=None, max_len=None, padding=True, truncation=True, return_offset=False, return_offsets_mapping=False, **kw):
+        """tokenize.py:184-259.  `text_pair=` is accepted as an alias of `pair_text`.  return_offsets_mapping: also
+        'offset_mapping', a (start, end) byte range per token (see encode_batch)."""
         if "text_pair" in kw:
             if pair_text is not None:
                 raise TypeError("pass pair_text or text_pair, not both")
@@ -343,6 +346,8 @@ class Tokenize(object):
         if max_len is not None:
             max_len = operator.index(max_len)
         flags = (L.WANT_TOKEN_TYPE | L.WANT_SEQUENCE_ID) if pair_text is not None else 0
+        if return_offsets_mapping:
+            flags |= L.WANT_OFFSETS
         r = self._encode_raw([text], None if pair_text is None else [pair_text], max_len, padding, truncation, flags, return_offset)
         return self._row_to_dict(r, 0, return_offset)
 
@@ -360,6 +365,8 @@ class Tokenize(object):
             result['offset'] = [tuple(p) for p in r._spans[so:eo].tolist()]
         result['input_ids'] = r._ids[s:e].tolist()
         result['attention_mask'] = r._mask[s:e].tolist()
+        if r._offsets is not None:
+            result['offset_mapping'] = [tuple(p) for p in r._offsets[s:e].tolist()]
         if r._has_pair:
             if r._status[i]:
                 raise ValueError("None is not in list")                   # tokenize.py:157-159
@@ -415,6 +422,7 @@ class Tokenize(object):
         r._tt_len = _view(enc.tt_len, n, C.c_int32, np.int32, owner) if enc.tt_len else None
         r._seq_len = _view(enc.seq_len, n, C.c_int32, np.int32, owner) if enc.seq_len else None
         r._status = _view(enc.row_status, n, C.c_uint8, np.uint8, owner) if enc.row_status else None
+        r._offsets = _view(enc.offsets, 2 * tot, C.c_int32, np.int32, owner).reshape(-1, 2) if enc.offsets else None
         if enc.span_off:
             r._span_off = _view(enc.span_off, n + 1, C.c_int64, np.int64, owner)
             r._spans = _view(enc.spans, 2 * int(r._span_off[-1]), C.c_int32, np.int32, owner).reshape(-1, 2)
@@ -436,16 +444,22 @@ class Tokenize(object):
             r["row_status"] = r._status
         if enc.span_off:
             r["span_off"], r["spans"] = r._span_off, r._spans
+        if r._offsets is not None:
+            r["offset_mapping"] = r._offsets.reshape(shape + (2,))
         return r
 
     # ---- batch extensions -------------------------------------------------------------------------------
     def encode_batch(self, texts, pair_texts=None, max_len=None, padding=True, truncation=True, token_type_ids=True,
-                     sequence_id=True, return_offset=False):
+                     sequence_id=True, return_offset=False, return_offsets_mapping=False):
         """Encode n documents (or n pairs) in one call.  `texts` / `pair_texts`: list[str] or the packed
-        form (uint8 bytes, int64 offsets[n+1]).  Returns a BatchEncoding of numpy arrays over pinned memory."""
-        flags = 0
+        form (uint8 bytes, int64 offsets[n+1]).  Returns a BatchEncoding of numpy arrays over pinned memory.
+        return_offsets_mapping: also 'offset_mapping', int32 [n, max_len, 2] (fixed layout) or [total, 2] (ragged): the
+        [start, end) byte range of each token in the UTF-8 ('surrogatepass') bytes of its own document -- `texts[i]`, or
+        `pair_texts[i]` for tokens of the second text -- and (0, 0) for <s>, </s>, pads and the </s> truncation adds.
+        It changes no other output."""
+        flags = L.WANT_OFFSETS if return_offsets_mapping else 0
         if pair_texts is not None:
-            flags = (L.WANT_TOKEN_TYPE if token_type_ids else 0) | (L.WANT_SEQUENCE_ID if sequence_id else 0)
+            flags |= (L.WANT_TOKEN_TYPE if token_type_ids else 0) | (L.WANT_SEQUENCE_ID if sequence_id else 0)
         if max_len is not None:
             max_len = operator.index(max_len)
         return self._encode_raw(texts, pair_texts, max_len, padding, truncation, flags, return_offset)
@@ -461,14 +475,15 @@ class Tokenize(object):
             raise OverflowError("max_len out of range")
         return max_len, stride
 
-    def encode_windows(self, texts, pair_texts=None, max_len=512, stride=0, token_type_ids=True, sequence_id=False):
+    def encode_windows(self, texts, pair_texts=None, max_len=512, stride=0, token_type_ids=True, sequence_id=False, return_offsets_mapping=False):
         """Every token of long documents, as overlapping windows of max_len (HF tokenizers' return_overflowing_tokens with a
         stride).  A single's window k holds [bos] + T[k(C-stride) : k(C-stride)+C] + [eos] with T = encode(text)[1:-1] and
         C = max_len - 2; a pair keeps its first text whole in every window and windows the second with C = max_len - len(A) - 4
         (one window, its encode_batch row, when C - stride < 1).  Each window is padded as encode_batch pads a row, so window 0
         of a document equals its encode_batch(max_len=max_len) row.  Returns a BatchEncoding with the fixed-layout planes over
         the windows plus overflow_to_sample_mapping (int64 [K]: the document of each window), window_start (int32 [K]: index
-        in T of its first content token) and window_off (int64 [n+1]: first window of each document)."""
+        in T of its first content token) and window_off (int64 [n+1]: first window of each document).  return_offsets_mapping:
+        also 'offset_mapping', int32 [K, max_len, 2], as encode_batch gives it (a token has the same offsets in every window)."""
         max_len, stride = self._window_args(max_len, stride)
         tb, to = texts if isinstance(texts, tuple) else pack_strings(texts)
         n = len(to) - 1
@@ -480,6 +495,8 @@ class Tokenize(object):
             pb, po = np.ascontiguousarray(pb, dtype=np.uint8), np.ascontiguousarray(po, dtype=np.int64)
             pbp, pop = pb.ctypes.data, po.ctypes.data
             flags = (L.WANT_TOKEN_TYPE if token_type_ids else 0) | (L.WANT_SEQUENCE_ID if sequence_id else 0)
+        if return_offsets_mapping:
+            flags |= L.WANT_OFFSETS
         tb, to = np.ascontiguousarray(tb, dtype=np.uint8), np.ascontiguousarray(to, dtype=np.int64)
         w = L.Windows()
         rc = self._lib.genztok_encode_windows(self._h, tb.ctypes.data, to.ctypes.data, pbp, pop, n, max_len, stride, flags, C.byref(w))
@@ -494,16 +511,19 @@ class Tokenize(object):
         return r
 
     def encode_windows_device(self, d_text, d_text_off, d_pair=None, d_pair_off=None, max_len=512, stride=0, token_type_ids=True,
-                              sequence_id=False, text_bytes=None, pair_bytes=None):
+                              sequence_id=False, text_bytes=None, pair_bytes=None, return_offsets_mapping=False):
         """encode_windows with everything resident on the GPU: inputs as for encode_device, outputs torch tensors on the input's
-        device written on torch's current stream (same keys as encode_windows).  The number of windows is read back between the
-        two steps (one synchronisation); the planes are then written without another."""
+        device written on torch's current stream (same keys as encode_windows; 'offset_mapping' int32 [K, max_len, 2] with
+        return_offsets_mapping).  The number of windows is read back between the two steps (one synchronisation); the planes
+        are then written without another.  Window 0 of each document (rows window_off[:-1]) is its encode_batch row."""
         import torch
         max_len, stride = self._window_args(max_len, stride)
         n = d_text_off.numel() - 1
         dev = d_text.device
         has_pair = d_pair_off is not None
         flags = ((L.WANT_TOKEN_TYPE if token_type_ids else 0) | (L.WANT_SEQUENCE_ID if sequence_id else 0)) if has_pair else 0
+        if return_offsets_mapping:
+            flags |= L.WANT_OFFSETS
         tbytes = d_text.numel() if text_bytes is None else text_bytes
         pbytes = (d_pair.numel() if pair_bytes is None else pair_bytes) if has_pair else 0
         args = (self._h, 0, d_text.data_ptr(), d_text_off.data_ptr(), tbytes, d_pair.data_ptr() if has_pair else None,
@@ -525,12 +545,15 @@ class Tokenize(object):
                 out["sequence_id"] = torch.empty((K, max_len), dtype=torch.int8, device=dev)
             out["seq_len"] = torch.empty((K,), dtype=torch.int32, device=dev)
             out["row_status"] = torch.empty((K,), dtype=torch.uint8, device=dev)
+        if return_offsets_mapping:
+            out["offset_mapping"] = torch.empty((K, max_len, 2), dtype=torch.int32, device=dev)
         out["overflow_to_sample_mapping"] = torch.empty((K,), dtype=torch.int64, device=dev)
         out["window_start"] = torch.empty((K,), dtype=torch.int32, device=dev)
         out["window_off"] = win_off
         P = L.DevPlanes()
         for k in ("input_ids", "attention_mask", "token_type_ids", "sequence_id", "row_len", "seq_len", "row_status"):
             setattr(P, k, out[k].data_ptr() if k in out else None)
+        P.offsets = out["offset_mapping"].data_ptr() if return_offsets_mapping else None
         rc = self._lib.genztok_encode_windows_device(*args, win_off.data_ptr(), C.byref(P), out["overflow_to_sample_mapping"].data_ptr(),
                                                      out["window_start"].data_ptr(), None, st)
         if rc:

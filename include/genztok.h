@@ -43,6 +43,14 @@ extern "C" {
 #define GENZTOK_WANT_TOKEN_TYPE 1u  /* token_type_ids (tokenize.py:254-258) */
 #define GENZTOK_WANT_SEQUENCE_ID 2u /* sequence_id    (tokenize.py:253-255) */
 #define GENZTOK_WANT_SPANS 4u       /* return_offset=True word->token spans (tokenize.py:105-117,225-234) */
+/* offset_mapping (HF tokenizers' return_offsets_mapping): per token, the int32 byte range [start, end) of the text it came from,
+ * relative to the first byte of its own document (`text`, or `pair` for tokens of the second text).  The words are the matches
+ * of \S+\n?; a word's BPE pieces tile it in order (an attached \n belongs to the last piece, an <unk> piece spans its code
+ * point, a word that is a special token's text spans the word).  Tokens that do not come from the text -- <s>, </s> of the
+ * framing, the </s> </s> between a pair's texts, pads, the </s> that truncation forces -- get (0, 0); every real token spans at
+ * least one byte.  Asking for offsets changes no other output.  (Documents are limited to max_chunk_bytes <= 512 MiB, so every
+ * byte offset fits an int32.) */
+#define GENZTOK_WANT_OFFSETS 8u
 
 /* Entries of the int8 planes */
 #define GENZTOK_NONE (-1)      /* Python None */
@@ -76,6 +84,7 @@ typedef struct genztok_encoded {
     void *_owner;            /* internal */
     int64_t d2h_bytes;       /* bytes this call copied from the device to the host (fixed layout: only the columns that can differ
                               * from padding travel; a recycled result buffer already holds the padding) */
+    int32_t *offsets;        /* [total][2] (start, end) byte offsets with GENZTOK_WANT_OFFSETS, or NULL */
 } genztok_encoded_t;
 
 typedef struct genztok_text {
@@ -96,6 +105,7 @@ typedef struct genztok_dev_planes {
     int32_t *row_len;        /* [n] */
     int32_t *seq_len;        /* [n] */
     uint8_t *row_status;     /* [n] */
+    int32_t *offsets;        /* genztok_encode_windows_device: [n_windows, max_len, 2]; read only with GENZTOK_WANT_OFFSETS */
 } genztok_dev_planes_t;
 
 /* ---- lifetime: Tokenize.__init__ / Tokenize.fromFile (tokenize.py:7-42, 261-267) ------------ */
@@ -133,7 +143,9 @@ void genztok_free_encoded(genztok_t *h, genztok_encoded_t *out);
 
 /* Device buffers in, device buffers out, on `stream` (a cudaStream_t, NULL = the handle's own
  * stream) of device slot `dev` (index into device_ids).  Fixed layout only: requires
- * max_len >= 1, padding and truncation.  Asynchronous: returns after enqueueing. */
+ * max_len >= 1, padding and truncation.  Asynchronous: returns after enqueueing.
+ * GENZTOK_WANT_SPANS and GENZTOK_WANT_OFFSETS are rejected (GENZTOK_E_INVALID).  For offsets on the device use
+ * genztok_encode_windows_device: window 0 of each document (rows d_win_off[:-1]) is its genztok_encode row. */
 int genztok_encode_device(genztok_t *h, int dev, const uint8_t *d_text, const int64_t *d_text_off,
                           int64_t text_bytes, const uint8_t *d_pair, const int64_t *d_pair_off,
                           int64_t pair_bytes, int64_t n, int32_t max_len, uint32_t flags,
@@ -154,7 +166,8 @@ typedef struct genztok_windows {
     int32_t *win_start;     /* [enc.n] index in T of the window's first content token */
 } genztok_windows_t;
 /* Host buffers in, pinned host buffers out (chunked and sharded across the handle's devices like genztok_encode).
- * flags: GENZTOK_WANT_TOKEN_TYPE / GENZTOK_WANT_SEQUENCE_ID for pairs. */
+ * flags: GENZTOK_WANT_TOKEN_TYPE / GENZTOK_WANT_SEQUENCE_ID for pairs, GENZTOK_WANT_OFFSETS (enc.offsets [K, max_len, 2]: a
+ * token has the same offsets in every window that holds it). */
 int genztok_encode_windows(genztok_t *h, const uint8_t *text, const int64_t *text_off, const uint8_t *pair,
                            const int64_t *pair_off, int64_t n, int32_t max_len, int32_t stride, uint32_t flags,
                            genztok_windows_t *out);
@@ -162,7 +175,8 @@ void genztok_free_windows(genztok_t *h, genztok_windows_t *out);
 /* Device form, two steps like genztok_decode_device.  Step 1 (planes == NULL): tokenises, fills d_win_off[n+1] and returns
  * the number of windows in *n_windows (synchronises).  Step 2: writes the caller's [n_windows, max_len] planes (input_ids and
  * attention_mask required; row_len required; token types, seq_len, row_status for pairs) and d_win_doc / d_win_start [n_windows]
- * from what step 1 left in the handle; a step 2 for another batch (other pointers, n, max_len, stride) redoes step 1.  Text
+ * from what step 1 left in the handle; a step 2 for another batch (other pointers, n, max_len, stride, or GENZTOK_WANT_OFFSETS
+ * other than in step 1) redoes step 1.  With GENZTOK_WANT_OFFSETS step 2 also fills planes->offsets [n_windows, max_len, 2].  Text
  * buffers 16-byte aligned, as for genztok_encode_device.  Step 2 does not synchronise. */
 int genztok_encode_windows_device(genztok_t *h, int dev, const uint8_t *d_text, const int64_t *d_text_off, int64_t text_bytes,
                                   const uint8_t *d_pair, const int64_t *d_pair_off, int64_t pair_bytes, int64_t n, int32_t max_len,
