@@ -12,6 +12,7 @@ WANT_TOKEN_TYPE, WANT_SEQUENCE_ID, WANT_SPANS, WANT_OFFSETS = 1, 2, 4, 8
 NONE, EOS_MARK, PAD_MARK = -1, -3, -4
 
 E_INVALID, E_IO, E_UTF8, E_CUDA, E_NOMEM, E_NODEVICE, E_LIMIT = -1, -2, -3, -4, -5, -6, -7
+QA_BYTES, QA_CHARS = 0, 1
 
 
 class Encoded(C.Structure):
@@ -86,6 +87,10 @@ SIGNATURES = {
     "genztok_check_errors": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.POINTER(C.c_int64)]),
     "genztok_synth_init": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64]),
     "genztok_synth_device": (C.c_int, [C.c_void_p, C.c_int, C.c_uint64, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_uint32, C.c_void_p, C.c_void_p, C.POINTER(C.c_int64), C.c_void_p]),
+    "genztok_qa_labels_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_int32, C.c_int, C.c_void_p, C.c_int64, C.c_void_p, C.c_int,
+                                          C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "genztok_qa_best_spans_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int, C.c_void_p, C.c_int64,
+                                              C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "genztok_digest_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p]),
 }
 

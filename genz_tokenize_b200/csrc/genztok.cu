@@ -12,6 +12,7 @@
 // Long documents as windows (window.cuh): the ragged steps up to k_rows<RAGGED> per side -> k_window_count -> k_scan_i64
 //   -> k_window_rows -> k_post_rows (row list).
 // Decode is k_decode_len (lengths, trailing pad runs) -> k_scan_i64 -> k_decode_write.
+// Extractive QA over the windows' offsets (qa.cuh): [k_qa_char_to_byte ->] k_qa_labels; k_qa_spans -> k_qa_spans_docs.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -35,6 +36,7 @@
 #include "host_tables.hpp"
 #include "post.cuh"
 #include "prep.cuh"
+#include "qa.cuh"
 #include "synth.cuh"
 #include "window.cuh"
 
@@ -80,6 +82,7 @@ struct DeviceCtx {
     DevBuf slots, key_arena, tok_arena, pending, ctr, rank_scratch;
     DevBuf len_arena;                             // piece byte lengths beside tok_arena (offset_mapping; allocated on first use)
     DevBuf offs;                                  // ragged pass: [total][2] token byte offsets (offset_mapping)
+    DevBuf qa_ans, qa_win;                        // QA: byte spans converted from characters; per-window best spans
     DevBuf dec_lead;                              // decode: per-row description left by the length pass for the write pass
     DevBuf dec_stat;                              // decode, fixed-width rows: ids in front of the pad runs, summed by the length pass
     double dec_avg_lead = -1;                     // ... per row, once the host has read it (-1: not known for the current batch)
@@ -949,7 +952,7 @@ struct Mode { bool fixed; bool has_max_len; int32_t max_len; int padding, trunca
 // ================================================================================================
 extern "C" {
 
-const char* genztok_version(void) { return "genztok-b200 0.2 (sm_100a)"; }
+const char* genztok_version(void) { return "genztok-b200 0.3 (sm_100a)"; }
 
 const char* genztok_last_error(const genztok_t* h) { return h ? h->err.c_str() : g_create_err.c_str(); }
 
@@ -2419,6 +2422,96 @@ int genztok_gather_rows(genztok_t* h, int dev, int n_fields, const void* const* 
     }
     CU(cudaGetLastError());
     return GENZTOK_OK;
+}
+
+// Extractive QA (qa.cuh).  Arguments are checked before the device slot, so that a host-only handle reports them too.  The kernels
+// count inconsistent inputs in the word cache's error counter, which is created here when no encode has run on the device yet.
+static int qa_enter(genztok_t* h, int dev, void* stream, DeviceCtx** dp, cudaStream_t* stp) {
+    if (dev < 0 || dev >= (int)h->devs.size()) return fail(h, GENZTOK_E_NODEVICE, "no such device slot %d (handle has %d)", dev, (int)h->devs.size());
+    DeviceCtx* d = h->devs[(size_t)dev];
+    CU(cudaSetDevice(d->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : d->stream;
+    LaunchScope::cur_stream = st;
+    if (!d->cache_ready) { int rc = ensure_cache(h, d, st, 0); if (rc) return rc; }
+    *dp = d; *stp = st;
+    return stream_enter(h, d, st);
+}
+
+int genztok_qa_labels_device(genztok_t* h, int dev, const int32_t* d_offsets, int64_t n_windows, int32_t max_len, int has_pair, const int64_t* d_win_off,
+                             int64_t n_docs, const int64_t* d_answers, int unit, const uint8_t* d_text, const int64_t* d_text_off, int64_t text_bytes,
+                             int64_t* d_start, int64_t* d_end, void* stream) {
+    if (!h) return GENZTOK_E_INVALID;
+    if (max_len < 3) return fail(h, GENZTOK_E_INVALID, "genztok_qa_labels_device: max_len >= 3 needed (got %d)", max_len);
+    if (unit != GENZTOK_QA_BYTES && unit != GENZTOK_QA_CHARS) return fail(h, GENZTOK_E_INVALID, "genztok_qa_labels_device: unknown unit %d", unit);
+    if (n_windows < 0 || n_docs < 0 || !d_win_off || (n_windows > 0 && (!d_offsets || !d_start || !d_end)) || (n_docs > 0 && !d_answers))
+        return fail(h, GENZTOK_E_INVALID, "genztok_qa_labels_device: bad arguments");
+    if (unit == GENZTOK_QA_CHARS && (!d_text_off || text_bytes < 0 || (text_bytes > 0 && !d_text) || ((uintptr_t)d_text & 15)))
+        return fail(h, GENZTOK_E_INVALID, "genztok_qa_labels_device: characters need the text (16-byte aligned) and its offsets");
+    std::lock_guard<std::mutex> lk(h->mu);
+    DeviceCtx* d = nullptr;
+    cudaStream_t st = nullptr;
+    int rc = qa_enter(h, dev, stream, &d, &st);
+    if (rc) return rc;
+    QaArgs A{};
+    A.om = reinterpret_cast<const int2*>(d_offsets); A.K = n_windows; A.W = max_len; A.pair = has_pair ? 1 : 0;
+    A.win_off = d_win_off; A.n = n_docs; A.answers = d_answers; A.start = d_start; A.end = d_end; A.ctr = d->C.ctr;
+    if (unit == GENZTOK_QA_CHARS && n_docs > 0) {
+        CU(d->qa_ans.ensure((size_t)n_docs * 16));
+        A.text = d_text; A.text_off = d_text_off; A.text_bytes = text_bytes; A.char_answers = d_answers; A.byte_answers = d->qa_ans.as<int64_t>();
+        A.answers = A.byte_answers;
+        LaunchScope ls(h, d, "k_qa_char_to_byte", n_docs * 32 + 8 * (n_docs + 1) + text_bytes);
+        k_qa_char_to_byte<<<(unsigned)std::max<int64_t>(1, std::min<int64_t>((n_docs + 7) / 8, (int64_t)d->sm_count * 16)), 256, 0, st>>>(A);
+    }
+    if (n_windows > 0) {
+        // om entries read per window: om[0], 32-probe rounds for c1, s and e, and (pairs) the question's columns in rounds of 32
+        int64_t rounds = 1;
+        for (int64_t r = max_len; r > 32; r = (r + 31) / 32) rounds++;
+        const int64_t om_read = 8 + 3 * rounds * 32 * 4 + (has_pair ? 256 : 0);
+        LaunchScope ls(h, d, "k_qa_labels", n_windows * (8 + 16 + om_read) + n_docs * 16);
+        k_qa_labels<<<(unsigned)std::max<int64_t>(1, std::min<int64_t>((n_windows + 7) / 8, (int64_t)d->sm_count * 16)), 256, 0, st>>>(A);
+    }
+    CU(cudaGetLastError());
+    return stream_leave(h, d, st);
+}
+
+int genztok_qa_best_spans_device(genztok_t* h, int dev, const float* d_start_logits, const float* d_end_logits, const int32_t* d_offsets, int64_t n_windows,
+                                 int32_t max_len, int has_pair, const int64_t* d_win_off, int64_t n_docs, int32_t max_answer_len, float* d_score,
+                                 float* d_null_score, int64_t* d_window, int32_t* d_columns, int32_t* d_span, void* stream) {
+    if (!h) return GENZTOK_E_INVALID;
+    if (max_len < 3) return fail(h, GENZTOK_E_INVALID, "genztok_qa_best_spans_device: max_len >= 3 needed (got %d)", max_len);
+    if (max_answer_len < 1) return fail(h, GENZTOK_E_INVALID, "genztok_qa_best_spans_device: max_answer_len >= 1 needed (got %d)", max_answer_len);
+    if (n_windows < 0 || n_docs < 0 || !d_win_off || (n_windows > 0 && (!d_start_logits || !d_end_logits || !d_offsets)) ||
+        (n_docs > 0 && (!d_score || !d_null_score || !d_window || !d_columns || !d_span)))
+        return fail(h, GENZTOK_E_INVALID, "genztok_qa_best_spans_device: bad arguments");
+    std::lock_guard<std::mutex> lk(h->mu);
+    DeviceCtx* d = nullptr;
+    cudaStream_t st = nullptr;
+    int rc = qa_enter(h, dev, stream, &d, &st);
+    if (rc) return rc;
+    // a warp stages its window's two logit rows and the two block-maximum arrays: 16 bytes per column
+    const size_t per_warp = (size_t)max_len * 16;
+    if (per_warp > d->smem_optin) return fail(h, GENZTOK_E_LIMIT, "genztok_qa_best_spans_device: max_len %d needs %zu bytes of shared memory per warp (%zu available)",
+                                              max_len, per_warp, d->smem_optin);
+    const int wpb = (int)std::max<size_t>(1, std::min<size_t>(8, (48u << 10) / per_warp));
+    const size_t smem = per_warp * (size_t)wpb;
+    if (smem > (48u << 10)) CU(cudaFuncSetAttribute(k_qa_spans, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    QaArgs A{};
+    A.om = reinterpret_cast<const int2*>(d_offsets); A.K = n_windows; A.W = max_len; A.pair = has_pair ? 1 : 0;
+    A.win_off = d_win_off; A.n = n_docs; A.S = d_start_logits; A.E = d_end_logits; A.L = std::min(max_answer_len, max_len);
+    A.score = d_score; A.null_score = d_null_score; A.window = d_window; A.columns = d_columns; A.span = d_span; A.ctr = d->C.ctr;
+    CU(d->qa_win.ensure((size_t)std::max<int64_t>(n_windows, 1) * 16));
+    A.w_score = d->qa_win.as<float>(); A.w_null = A.w_score + n_windows;
+    A.w_s = reinterpret_cast<int32_t*>(A.w_null + n_windows); A.w_e = A.w_s + n_windows;
+    if (n_windows > 0) {
+        LaunchScope ls(h, d, "k_qa_spans", n_windows * (int64_t)max_len * (4 + 4 + 8));
+        k_qa_spans<<<(unsigned)std::max<int64_t>(1, std::min<int64_t>((n_windows + wpb - 1) / wpb, (int64_t)d->sm_count * 32)), 32 * wpb, smem, st>>>(A);
+    }
+    if (n_docs > 0) {
+        LaunchScope ls(h, d, "k_qa_spans_docs", 8 * (n_docs + 1) + n_docs * (4 + 4 + 8 + 8 + 8));
+        k_qa_spans_docs<<<(unsigned)std::min<int64_t>((n_docs + 255) / 256, (int64_t)d->sm_count * 8), 256, 0, st>>>(A);
+    }
+    CU(cudaGetLastError());
+    return stream_leave(h, d, st);
 }
 
 int genztok_check_errors(genztok_t* h, int dev, void* stream, int64_t* n_errors) {

@@ -9,6 +9,8 @@ Extensions over the reference (which is one string per call): `encode_batch` / `
 `encode_windows_device` (long documents as overlapping max_len windows, every token kept).  Every encode
 form but encode_device can also return `offset_mapping` (HF's return_offsets_mapping): each token's
 (start, end) byte range in its own document's UTF-8 text, (0, 0) for tokens that are not from the text.
+`qa_labels` / `qa_best_spans` turn those planes into extractive-QA training labels and read a QA model's
+start / end logits back into answer spans, on the GPU.
 """
 import ctypes as C
 import operator
@@ -103,6 +105,7 @@ class Tokenize(object):
         sp = (C.c_char_p * 5)(*[t.encode("utf-8", "surrogatepass") for t in
                                 (self.pad_token, self.bos_token, self.eos_token, self.mask_token, self.unk_token)])
         dev = (C.c_int * max(len(devices), 1))(*devices)
+        self._device_ids = list(devices)
         h = C.c_void_p()
         vocab = self.vocab_file
         if self._extra_vocab:
@@ -667,6 +670,122 @@ class Tokenize(object):
         if rc:
             self._err(rc, "genztok_decode_device")
         return out[:total.value], out_off
+
+    # ---- extractive question answering over the windows' planes ------------------------------------------------------------
+    def _qa_planes(self, enc):
+        """(torch offsets [K, W, 2], window_off [n + 1], has_pair, device, host_form) of an encode_windows(_device) result or a
+        fixed-layout encode_batch result with offsets (one window per document), on the handle's device."""
+        import torch
+        if "offset_mapping" not in enc:
+            raise ValueError("qa: the encoding has no 'offset_mapping'; encode with return_offsets_mapping=True")
+        om = enc["offset_mapping"]
+        if om.ndim != 3 or om.shape[2] != 2:
+            raise ValueError("qa: 'offset_mapping' must be the fixed [windows, max_len, 2] layout (got shape %s; ragged results "
+                             "are not supported)" % (tuple(om.shape),))
+        K, W = int(om.shape[0]), int(om.shape[1])
+        if W < 3:
+            raise ValueError("qa: max_len >= 3 needed (got %d)" % W)
+        host = not isinstance(om, torch.Tensor)
+        if host:
+            if not self._device_ids:
+                raise GenztokError("qa: this handle was created without a CUDA device; there is no CPU path")
+            dev = torch.device("cuda", self._device_ids[0])
+            om = torch.from_numpy(np.ascontiguousarray(om, dtype=np.int32)).to(dev)
+        else:
+            dev = om.device
+            om = om.to(torch.int32).contiguous()
+        wo = enc.get("window_off")
+        if wo is None:
+            wo = torch.arange(K + 1, dtype=torch.int64, device=dev)
+        else:
+            wo = (torch.from_numpy(np.ascontiguousarray(wo, dtype=np.int64)) if not isinstance(wo, torch.Tensor) else wo).to(dev, torch.int64).contiguous()
+            if wo.ndim != 1 or wo.numel() < 1:
+                raise ValueError("qa: 'window_off' must be int64 [n + 1]")
+        return om, wo, "seq_len" in enc, dev, host
+
+    @staticmethod
+    def _qa_rows(x, shape, dtype, dev, what):
+        import torch
+        t = x if isinstance(x, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(np.asarray(x)))
+        if tuple(t.shape) != tuple(shape):
+            raise ValueError("qa: %s must have shape %s (got %s)" % (what, tuple(shape), tuple(t.shape)))
+        return t.to(dev, dtype).contiguous()
+
+    def qa_labels(self, enc, answers, unit="byte", context=None):
+        """Extractive-QA training labels: (start_positions, end_positions), int64 [K], one pair per window.
+        `enc`: an encode_windows / encode_windows_device result, or a fixed-layout encode_batch result (one window per
+        document), made with return_offsets_mapping=True.  `answers`: [n, 2] spans [a0, a1) in the windowed text (`texts[d]`,
+        or `pair_texts[d]` for pairs), in bytes of its UTF-8 ('surrogatepass') form with unit="byte", in Python str indices
+        with unit="char" -- then `context` is that text: list[str], packed (bytes, offsets) or CUDA tensors (d_text 16-byte
+        aligned, d_text_off).  A window's context columns come from the offsets alone (singles: end > 0; pairs: end > 0
+        after the first (0, 0) column >= 1); its label is (first, last) of the context columns that overlap the answer when
+        they hold all of it, else (0, 0).  No answer (a1 <= a0) and spans past the end give (0, 0).  Device results stay on
+        their device on torch's current stream; numpy results are copied to the handle's device (8 bytes per column of
+        offsets) and the labels back."""
+        import torch
+        if unit not in ("byte", "char"):
+            raise ValueError("qa_labels: unit must be 'byte' or 'char' (got %r)" % (unit,))
+        om, wo, has_pair, dev, host = self._qa_planes(enc)
+        K, W = int(om.shape[0]), int(om.shape[1])
+        n = wo.numel() - 1
+        ans = self._qa_rows(answers, (n, 2), torch.int64, dev, "answers")
+        tx = toff = None
+        nb = 0
+        if unit == "char":
+            if context is None:
+                raise ValueError("qa_labels: unit='char' needs `context`, the windowed text")
+            if isinstance(context, tuple) and isinstance(context[0], torch.Tensor):
+                tx, toff = context[0], context[1].to(dev, torch.int64).contiguous()
+                nb = tx.numel()
+            else:
+                b, o = context if isinstance(context, tuple) else pack_strings(context)
+                b = np.ascontiguousarray(b, dtype=np.uint8)
+                nb = len(b)
+                tx = torch.from_numpy(np.concatenate([b, np.zeros((-nb) % 16 + 16, dtype=np.uint8)])).to(dev)
+                toff = torch.from_numpy(np.ascontiguousarray(o, dtype=np.int64)).to(dev)
+            if toff.numel() != n + 1:
+                raise ValueError("qa_labels: `context` holds %d documents, the encoding %d" % (toff.numel() - 1, n))
+        start = torch.empty((K,), dtype=torch.int64, device=dev)
+        end = torch.empty((K,), dtype=torch.int64, device=dev)
+        rc = self._lib.genztok_qa_labels_device(self._h, 0, om.data_ptr(), K, W, int(has_pair), wo.data_ptr(), n, ans.data_ptr(),
+                                                L.QA_CHARS if unit == "char" else L.QA_BYTES, tx.data_ptr() if tx is not None else None,
+                                                toff.data_ptr() if toff is not None else None, nb, start.data_ptr(), end.data_ptr(), self._torch_stream(dev))
+        if rc:
+            self._err(rc, "genztok_qa_labels_device")
+        if host:
+            return start.cpu().numpy(), end.cpu().numpy()
+        return start, end
+
+    def qa_best_spans(self, enc, start_logits, end_logits, max_answer_len=30):
+        """The best answer span per document from a QA model's start / end logits ([K, W], one row per window of `enc`, as
+        for qa_labels; not float32 is converted with .float()).  Candidates are (window i of the document, s, e) with s <= e
+        context columns of i and e - s + 1 <= max_answer_len, scored start_logits[i, s] + end_logits[i, e] (one float32 add);
+        the best is the largest score, ties to the smallest i, then s, then e, and a NaN score is never taken.  This is the
+        exact maximum over every valid pair (HF's top-20 x top-20 pre-filter can only find a lower or equal one).  Returns a
+        dict with, per document: 'score' (float32), 'null_score' (min over its windows of start_logits[i, 0] + end_logits[i, 0],
+        SQuAD v2's no-answer score), 'window' (int64 global window, -1 with no candidate), 'columns' (int32 [n, 2] (s, e)) and
+        'span' (int32 [n, 2], the answer's byte range in the document); a document without a candidate gets score -inf and
+        (0, 0).  Device results stay on their device; numpy results are copied to the handle's device and back."""
+        import torch
+        max_answer_len = operator.index(max_answer_len)
+        if max_answer_len < 1:
+            raise ValueError("qa_best_spans: max_answer_len >= 1 needed (got %d)" % max_answer_len)
+        om, wo, has_pair, dev, host = self._qa_planes(enc)
+        K, W = int(om.shape[0]), int(om.shape[1])
+        n = wo.numel() - 1
+        sl = self._qa_rows(start_logits if isinstance(start_logits, torch.Tensor) else np.asarray(start_logits, dtype=np.float32), (K, W), torch.float32, dev, "start_logits")
+        el = self._qa_rows(end_logits if isinstance(end_logits, torch.Tensor) else np.asarray(end_logits, dtype=np.float32), (K, W), torch.float32, dev, "end_logits")
+        out = {"score": torch.empty((n,), dtype=torch.float32, device=dev), "null_score": torch.empty((n,), dtype=torch.float32, device=dev),
+               "window": torch.empty((n,), dtype=torch.int64, device=dev), "columns": torch.empty((n, 2), dtype=torch.int32, device=dev),
+               "span": torch.empty((n, 2), dtype=torch.int32, device=dev)}
+        rc = self._lib.genztok_qa_best_spans_device(self._h, 0, sl.data_ptr(), el.data_ptr(), om.data_ptr(), K, W, int(has_pair), wo.data_ptr(), n,
+                                                    min(max_answer_len, 2 ** 31 - 1), out["score"].data_ptr(), out["null_score"].data_ptr(),
+                                                    out["window"].data_ptr(), out["columns"].data_ptr(), out["span"].data_ptr(), self._torch_stream(dev))
+        if rc:
+            self._err(rc, "genztok_qa_best_spans_device")
+        if host:
+            return {k: v.cpu().numpy() for k, v in out.items()}
+        return out
 
     # ---- measurement plumbing (bench.py, tests): synthetic workload on the device, plane digest, error counter -----------
     def synth_device(self, seed, doc0, n, side=0, lo=3, hi=13, noise=0.0, device=None):

@@ -269,6 +269,42 @@ int genztok_check_errors(genztok_t *h, int dev, void *stream, int64_t *n_errors)
 int genztok_gather_rows(genztok_t *h, int dev, int n_fields, const void *const *d_fields, const int64_t *row_bytes,
                         int64_t n_rows, const int64_t *d_index, int64_t n_index, void *const *d_out, void *stream);
 
+/* ---- extractive question answering over the windows' planes (the targets and outputs of the reference's QA models) ---------
+ * Both read the offset_mapping plane d_offsets [n_windows][max_len][2] of genztok_encode_windows(_device) (or of a fixed-layout
+ * genztok_encode, one window per document: d_win_off = 0, 1, ..., n) and d_win_off [n_docs + 1]; windows win_off[d] .. win_off[d+1]-1
+ * belong to document d, whose answer lives in the windowed text (the second text of pairs).
+ * Context columns of a window, from the offsets alone (token types move with a question that holds a literal </s>): singles,
+ * every column with end > 0; pairs, with z the first column >= 1 that is (0, 0), the columns after z with end > 0.  They form
+ * one range of columns, possibly empty (a pair whose question fills the row has none).
+ * Labels: with the answer [a0, a1) in bytes of the document, cols = the context columns with start < a1 and end > a0; the
+ * window's label is (cols[0], cols[-1]) when cols is not empty, start(cols[0]) <= a0 and end(cols[-1]) >= a1, else (0, 0) (the <s>
+ * column).  a1 <= a0 ("no answer") and spans past the document's end give (0, 0) in every window; an answer inside the stride
+ * overlap is labelled in every window that wholly holds it.  GENZTOK_QA_CHARS: d_answers are indices into the Python str; index
+ * k becomes the byte of the code point with index k (a code point is a byte that is not 10xxxxxx: Python's count for
+ * 'surrogatepass' UTF-8), the character count becomes the byte length, a larger index the byte length plus the excess (past
+ * the end), a negative one stays as it is.  The text (d_text 16-byte aligned and readable to a multiple of 16 bytes,
+ * d_text_off[n_docs + 1]) is what was windowed.  One launch per call (two with characters).
+ * Best spans: candidates (i, s, e) with i a window of d, s <= e context columns of i and e - s + 1 <= max_answer_len; score
+ * start_logits[i][s] + end_logits[i][e] (one float add).  The best is the largest score, ties to the smallest i, then s, then e;
+ * a NaN score is never taken.  This is the exact maximum over every valid pair (HF's top-20 x top-20 pre-filter can only find a
+ * lower or equal one).  Per document: d_score, d_window (global window index), d_columns (s, e), d_span = (start of s, end of e),
+ * the answer's byte range in the document, and d_null_score = the fminf over its windows of start_logits[i][0] + end_logits[i][0]
+ * (SQuAD v2's "no answer" score).  A document without a candidate gets window -1, score -inf, columns = span = (0, 0).  A warp
+ * stages its window's two logit rows in shared memory: max_len above the device's per-block limit / 16 bytes is GENZTOK_E_LIMIT.
+ * Two launches per call.
+ * Both are asynchronous on `stream` of device slot `dev` and bit-identical from run to run.  Offsets that break the layout and a
+ * win_off that does not fit n_windows are counted by genztok_check_errors (such windows get (0, 0) and no candidate). */
+#define GENZTOK_QA_BYTES 0
+#define GENZTOK_QA_CHARS 1
+int genztok_qa_labels_device(genztok_t *h, int dev, const int32_t *d_offsets, int64_t n_windows, int32_t max_len, int has_pair,
+                             const int64_t *d_win_off, int64_t n_docs, const int64_t *d_answers /* [n_docs][2] */, int unit,
+                             const uint8_t *d_text, const int64_t *d_text_off, int64_t text_bytes /* GENZTOK_QA_CHARS only */,
+                             int64_t *d_start, int64_t *d_end /* [n_windows] */, void *stream);
+int genztok_qa_best_spans_device(genztok_t *h, int dev, const float *d_start_logits, const float *d_end_logits /* [n_windows][max_len] */,
+                                 const int32_t *d_offsets, int64_t n_windows, int32_t max_len, int has_pair, const int64_t *d_win_off,
+                                 int64_t n_docs, int32_t max_answer_len, float *d_score, float *d_null_score, int64_t *d_window,
+                                 int32_t *d_columns /* [n_docs][2] */, int32_t *d_span /* [n_docs][2] */, void *stream);
+
 /* ---- measurement plumbing (not part of the reference's surface; used by bench.py and the tests) ------------------- */
 /* The synthetic workload of SURVEY.md 8 d2 produced on the device: the counter-based generator that
  * genz_tokenize_b200/workload.py::generate_hashed defines (same bytes).  genztok_synth_init uploads the word list
