@@ -945,7 +945,27 @@ T* out_alloc(genztok_t* h, OutBlock* ob, size_t count) {
     return reinterpret_cast<T*>(p);
 }
 
-struct Mode { bool fixed; bool has_max_len; int32_t max_len; int padding, truncation; };
+// Gives a result block's buffers back (the pinned ones to the pool) and deletes it.
+void release_block(genztok_t* h, OutBlock* ob) {
+    for (auto& pr : ob->pinned) host_pool_put(h, pr.first, pr.second);
+    for (void* p : ob->mallocs) free(p);
+    delete ob;
+}
+
+// The same for the result of a call that failed: what its pooled planes hold is unknown, so their plane_meta records go too.  (A
+// result that its owner frees keeps them: a recycled fixed-layout plane copies only the columns its record says can differ.)
+void discard_block(genztok_t* h, OutBlock* ob) {
+    for (auto& pr : ob->pinned) h->plane_meta.erase(pr.first);
+    release_block(h, ob);
+}
+
+// genztok_free_encoded / genztok_free_text
+template <class Out>
+void free_result(genztok_t* h, Out* out) {
+    if (!out || !out->_owner) return;
+    { std::lock_guard<std::mutex> lk(h->mu); release_block(h, reinterpret_cast<OutBlock*>(out->_owner)); }
+    memset(out, 0, sizeof *out);
+}
 
 }  // namespace
 
@@ -1195,19 +1215,7 @@ int genztok_encode_device(genztok_t* h, int dev, const uint8_t* d_text, const in
     return encode_fixed_on_device(h, d, st, a, d_pair_off ? &b : nullptr, n, max_len, flags, *planes);
 }
 
-void genztok_free_encoded(genztok_t* h, genztok_encoded_t* out) {
-    if (!out || !out->_owner) return;
-    OutBlock* ob = reinterpret_cast<OutBlock*>(out->_owner);
-    {
-        std::lock_guard<std::mutex> lk(h->mu);
-        for (auto& pr : ob->pinned) {
-            host_pool_put(h, pr.first, pr.second);
-        }
-    }
-    for (void* p : ob->mallocs) free(p);
-    delete ob;
-    memset(out, 0, sizeof *out);
-}
+void genztok_free_encoded(genztok_t* h, genztok_encoded_t* out) { free_result(h, out); }
 
 }  // extern "C"
 
@@ -1225,9 +1233,68 @@ struct EncodeJob {
     int32_t old_dirty[4];          // fixed layout: columns of the result planes (ids, mask, token types, sequence ids) that may hold something
                                    // other than padding from the buffer's last use (the width: unknown / a fresh buffer)
 };
-struct EncodePart {
+
+// The fields genztok_encode and genztok_encode_windows set alike.
+EncodeJob make_job(const uint8_t* text, const int64_t* text_off, const uint8_t* pair, const int64_t* pair_off, int32_t max_len, uint32_t flags) {
+    EncodeJob J{};
+    J.text = text; J.text_off = text_off; J.pair = pair; J.pair_off = pair_off;
+    J.max_len = max_len; J.flags = flags;
+    J.has_pair = pair_off != nullptr;
+    J.want_offs = (flags & GENZTOK_WANT_OFFSETS) != 0;
+    J.want_tt = J.has_pair && (flags & GENZTOK_WANT_TOKEN_TYPE);
+    J.want_seq = J.has_pair && (flags & GENZTOK_WANT_SEQUENCE_ID);
+    return J;
+}
+
+// Shard by row across the handle's G devices (SURVEY.md 8e): device g takes the rows [cuts[g], cuts[g + 1]), contiguous ranges
+// balanced by weight(r), a non-decreasing prefix over the rows; no collective.  Fewer than two rows per device all go to device 0.
+template <class Weight>
+std::vector<int64_t> shard_rows(int G, int64_t n, Weight weight) {
+    std::vector<int64_t> cuts((size_t)G + 1, n);
+    cuts[0] = 0;
+    if (G == 1 || n < 2 * G) return cuts;
+    const int64_t wtot = weight(n) - weight(0);
+    for (int g = 1; g < G; g++) {
+        const int64_t want = weight(0) + wtot * g / G;
+        int64_t lo = cuts[(size_t)g - 1], hi = n;
+        while (lo < hi) { int64_t mid = (lo + hi) / 2; if (weight(mid) < want) lo = mid + 1; else hi = mid; }
+        cuts[(size_t)g] = lo;
+    }
+    return cuts;
+}
+
+// work(g) for every device g of the shard cuts: inline when one device has all the rows, else one host thread per device.
+template <class Work>
+void run_shards(const std::vector<int64_t>& cuts, Work work) {
+    const int G = (int)cuts.size() - 1;
+    int busy = 0, only = 0;
+    for (int g = 0; g < G; g++) if (cuts[(size_t)g + 1] > cuts[(size_t)g]) { busy++; only = g; }
+    if (busy <= 1) { work(only); return; }
+    std::vector<std::thread> th;
+    for (int g = 0; g < G; g++) th.emplace_back([&, g]() { work(g); });
+    for (auto& t : th) t.join();
+}
+
+// What a device worker reports to the calling thread: its return code, and the text for genztok_last_error.
+struct PartStatus {
     int rc = GENZTOK_OK;
     std::string err;
+    int report(genztok_t* h) const { std::lock_guard<std::mutex> l(h->err_mu); h->err = err; return rc; }
+};
+
+// Failure exits of a device worker, which returns void and has `h`, its stream `st` and its `part` in scope: the part's status is set
+// and the stream drained before it returns.  FAIL_RC takes the text that a failed helper left in h->err.
+#define PFAIL(code, ...) { char _b[400]; snprintf(_b, sizeof _b, __VA_ARGS__); part->status.rc = (code); part->status.err = _b; cudaStreamSynchronize(st); return; }
+#define FAIL_RC(call) { int _rc = (call); if (_rc) { part->status.rc = _rc; { std::lock_guard<std::mutex> _l(h->err_mu); part->status.err = h->err; } cudaStreamSynchronize(st); return; } }
+#define CUF(call) { cudaError_t _e = (call); if (_e != cudaSuccess) PFAIL(GENZTOK_E_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(_e), __FILE__, __LINE__) }
+
+// Grows a part's array to m entries.  On the part's first chunk of several, `first` is the estimate for the whole part, reserved
+// beforehand so that later chunks do not move the array (0: nothing to reserve).
+template <class T>
+bool grow(PinnedVec<T>& v, size_t m, size_t first) { return (first == 0 || v.reserve(first)) && v.resize(m); }
+
+struct EncodePart {
+    PartStatus status;
     int32_t extent = 0;            // fixed layout: columns that can differ from padding, max over this part's chunks
     int64_t d2h_bytes = 0;
     PinnedVec<int32_t> ids, spans, tok_offs; PinnedVec<uint8_t> mask; PinnedVec<int8_t> tt, seq;
@@ -1258,167 +1325,174 @@ int64_t chunk_cuts(const genztok_t* h, const EncodeJob& J, int64_t rb, int64_t r
     return -1;
 }
 
-void encode_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int64_t rb, int64_t re, EncodePart* part) {
-    genztok_encoded_t* out = J.out;
-    const bool has_pair = J.has_pair, has_max_len = J.has_max_len, want_spans = J.want_spans, fixed = J.fixed, want_tt = J.want_tt, want_seq = J.want_seq;
-    const int32_t max_len = J.max_len;
-    cudaStream_t st = d->stream;
-#define PFAIL(code, ...) { char _b[400]; snprintf(_b, sizeof _b, __VA_ARGS__); part->rc = (code); part->err = _b; cudaStreamSynchronize(st); return; }
-#define FAIL_RC(call) { int _rc = (call); if (_rc) { part->rc = _rc; { std::lock_guard<std::mutex> _l(h->err_mu); part->err = h->err; } cudaStreamSynchronize(st); return; } }
-#define CUF(call) { cudaError_t _e = (call); if (_e != cudaSuccess) PFAIL(GENZTOK_E_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(_e), __FILE__, __LINE__) }
-    CUF(cudaSetDevice(d->device));
-    LaunchScope::cur_stream = st;
-    const int8_t eos8 = eos_as_i8(d);
-    std::vector<int64_t> cuts;
-    int64_t most = 0;
-    { const int64_t big = chunk_cuts(h, J, rb, re, &cuts, &most);
-      if (big >= 0) PFAIL(GENZTOK_E_LIMIT, "document %lld is larger than max_chunk_bytes=%lld", (long long)big, (long long)h->max_chunk_bytes) }
-    FAIL_RC(ensure_cache(h, d, st, most));
-    if (J.want_offs) FAIL_RC(ensure_piece_lens(h, d, st));
-    unsigned long long tokens_before = 0;
-    CUF(cudaMemcpyAsync(&tokens_before, d->C.ctr + C_TOKENS, 8, cudaMemcpyDeviceToHost, st));
-    CUF(cudaStreamSynchronize(st));
+// The rows [r0, r1) of both sides to the device on stream st, into text / toff (and pair / poff), which the caller has sized; *a and
+// *b are the sides the kernels read.  Offsets stay absolute (as in the caller's buffer): a side's bytes are copied to dev + (off[r0] & 15)
+// and its base pointer is shifted by -off[r0], so that base + 16k is 16-byte aligned, as the kernels' 16-byte loads need.
+cudaError_t upload_chunk(const EncodeJob& J, int64_t r0, int64_t r1, DevBuf& text, DevBuf& toff, DevBuf& pair, DevBuf& poff, cudaStream_t st,
+                         Side* a, Side* b) {
+    auto side = [&](const uint8_t* src, const int64_t* off, DevBuf& bytes, DevBuf& offs, Side* s) {
+        const int64_t b0 = off[r0], nb = off[r1] - b0;
+        *s = Side{bytes.as<uint8_t>() + (b0 & 15) - b0, offs.as<int64_t>(), nb};
+        cudaError_t e = nb ? cudaMemcpyAsync(bytes.as<uint8_t>() + (b0 & 15), src + b0, (size_t)nb, cudaMemcpyHostToDevice, st) : cudaSuccess;
+        return e != cudaSuccess ? e : cudaMemcpyAsync(offs.p, off + r0, (size_t)(r1 - r0 + 1) * 8, cudaMemcpyHostToDevice, st);
+    };
+    *b = Side{nullptr, poff.as<int64_t>(), 0};
+    cudaError_t e = side(J.text, J.text_off, text, toff, a);
+    return (e != cudaSuccess || !J.has_pair) ? e : side(J.pair, J.pair_off, pair, poff, b);
+}
 
-    if (fixed) {
-        // ---- fixed layout, pipelined over chunks: H2D(i + 1) | kernels(i) | D2H(i - 1) on three streams, two sets of chunk buffers.
-        // Only the columns that can differ from padding travel back: [0, max(extent of the chunk, what the pooled host plane still
-        // holds from its last use)), rounded up to 32; a fresh host plane takes whole rows once.
-        const size_t nc = cuts.size() - 1;
-        if (!d->s_in) CUF(cudaStreamCreateWithFlags(&d->s_in, cudaStreamNonBlocking));
-        if (!d->s_out) CUF(cudaStreamCreateWithFlags(&d->s_out, cudaStreamNonBlocking));
-        if (!d->h_extent) CUF(cudaHostAlloc(reinterpret_cast<void**>(&d->h_extent), 64, cudaHostAllocDefault));
-        int64_t mm = 0, mtb = 0, mpb = 0;
-        for (size_t ci = 0; ci < nc; ci++) {
-            mm = std::max(mm, cuts[ci + 1] - cuts[ci]);
-            mtb = std::max(mtb, J.text_off[cuts[ci + 1]] - J.text_off[cuts[ci]]);
-            if (has_pair) mpb = std::max(mpb, J.pair_off[cuts[ci + 1]] - J.pair_off[cuts[ci]]);
-        }
-        const size_t mtot = (size_t)mm * (size_t)max_len;
-        for (int sidx = 0; sidx < (nc > 1 ? 2 : 1); sidx++) {
-            DeviceCtx::Stage& sg = d->stage[sidx];
-            for (cudaEvent_t* e : {&sg.h2d, &sg.k, &sg.d2h}) if (!*e) CUF(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
-            CUF(sg.text.ensure((size_t)mtb + 96)); CUF(sg.toff.ensure((size_t)(mm + 1) * 8));
-            if (has_pair) { CUF(sg.pair.ensure((size_t)mpb + 96)); CUF(sg.poff.ensure((size_t)(mm + 1) * 8)); }
-            CUF(sg.ids.ensure(mtot * 4)); CUF(sg.mask.ensure(mtot)); CUF(sg.row_len.ensure((size_t)mm * 4)); CUF(sg.extent.ensure(16));
-            if (want_tt) CUF(sg.tt.ensure(mtot));
-            if (want_seq) CUF(sg.seq.ensure(mtot));
-            if (has_pair) { CUF(sg.seq_len.ensure((size_t)mm * 4)); CUF(sg.status.ensure((size_t)mm)); }
-        }
-        auto issue_h2d = [&](size_t ci) -> bool {
-            DeviceCtx::Stage& sg = d->stage[ci & 1];
-            const int64_t r0 = cuts[ci], r1 = cuts[ci + 1], m = r1 - r0;
-            const int64_t tb0 = J.text_off[r0], tb = J.text_off[r1] - tb0;
-            if (ci >= 2 && cudaStreamWaitEvent(d->s_in, sg.k, 0) != cudaSuccess) return false;      // the kernels of chunk ci - 2 have read this set's inputs
-            // Offsets stay absolute (as in the caller's buffer): the chunk is copied to dev + (tb0 & 15) and the base pointer is
-            // shifted by -tb0, so that base + 16k is 16-byte aligned, as the kernels' 16-byte loads need.
-            if (tb && cudaMemcpyAsync(sg.text.as<uint8_t>() + (tb0 & 15), J.text + tb0, (size_t)tb, cudaMemcpyHostToDevice, d->s_in) != cudaSuccess) return false;
-            if (cudaMemcpyAsync(sg.toff.p, J.text_off + r0, (size_t)(m + 1) * 8, cudaMemcpyHostToDevice, d->s_in) != cudaSuccess) return false;
-            if (has_pair) {
-                const int64_t pb0 = J.pair_off[r0], pb = J.pair_off[r1] - pb0;
-                if (pb && cudaMemcpyAsync(sg.pair.as<uint8_t>() + (pb0 & 15), J.pair + pb0, (size_t)pb, cudaMemcpyHostToDevice, d->s_in) != cudaSuccess) return false;
-                if (cudaMemcpyAsync(sg.poff.p, J.pair_off + r0, (size_t)(m + 1) * 8, cudaMemcpyHostToDevice, d->s_in) != cudaSuccess) return false;
-            }
-            return cudaEventRecord(sg.h2d, d->s_in) == cudaSuccess;
-        };
-        auto fail_sync = [&]() { cudaStreamSynchronize(d->s_in); cudaStreamSynchronize(st); cudaStreamSynchronize(d->s_out); };
-        if (nc && !issue_h2d(0)) { fail_sync(); PFAIL(GENZTOK_E_CUDA, "host to device copy failed: %s", cudaGetErrorString(cudaGetLastError())) }
-        for (size_t ci = 0; ci < nc; ci++) {
-            DeviceCtx::Stage& sg = d->stage[ci & 1];
-            const int64_t r0 = cuts[ci], r1 = cuts[ci + 1], m = r1 - r0;
-            const int64_t tb0 = J.text_off[r0], tb = J.text_off[r1] - tb0;
-            const int64_t pb0 = has_pair ? J.pair_off[r0] : 0, pb = has_pair ? J.pair_off[r1] - pb0 : 0;
-            // kernels of chunk ci: behind its inputs, and behind the copy-out of the chunk that used this set of planes before
-            CUF(cudaStreamWaitEvent(st, sg.h2d, 0));
-            if (ci >= 2) CUF(cudaStreamWaitEvent(st, sg.d2h, 0));
-            Side a{sg.text.as<uint8_t>() + (tb0 & 15) - tb0, sg.toff.as<int64_t>(), tb};
-            Side b{has_pair ? sg.pair.as<uint8_t>() + (pb0 & 15) - pb0 : nullptr, sg.poff.as<int64_t>(), pb};
-            genztok_dev_planes_t P{};
-            P.input_ids = sg.ids.as<int32_t>(); P.attention_mask = sg.mask.as<uint8_t>(); P.row_len = sg.row_len.as<int32_t>();
-            if (want_tt) P.token_type_ids = sg.tt.as<int8_t>();
-            if (want_seq) P.sequence_id = sg.seq.as<int8_t>();
-            if (has_pair) { P.seq_len = sg.seq_len.as<int32_t>(); P.row_status = sg.status.as<uint8_t>(); }
-            { int _rc = encode_fixed_on_device(h, d, st, a, has_pair ? &b : nullptr, m, max_len, J.flags, P);
-              if (_rc) { part->rc = _rc; { std::lock_guard<std::mutex> _l(h->err_mu); part->err = h->err; } fail_sync(); return; } }
-            CUF(cudaMemsetAsync(sg.extent.p, 0, 4, st));
-            { LaunchScope ls(h, d, "k_row_extent");
-              k_row_extent<<<(unsigned)std::min<int64_t>((m + 255) / 256, (int64_t)d->sm_count * 4), 256, 0, st>>>(P.row_len, has_pair ? P.seq_len : nullptr, m, sg.extent.as<int32_t>()); }
-            CUF(cudaMemcpyAsync(d->h_extent + (ci & 1), sg.extent.p, 4, cudaMemcpyDeviceToHost, st));
-            CUF(cudaEventRecord(sg.k, st));
-            // the next chunk's inputs travel while these kernels run
-            if (ci + 1 < nc && !issue_h2d(ci + 1)) { fail_sync(); PFAIL(GENZTOK_E_CUDA, "host to device copy failed: %s", cudaGetErrorString(cudaGetLastError())) }
-            // copy-out of chunk ci: the host learns the extent (the only wait of this loop), then the trimmed planes go on their own stream
-            CUF(cudaEventSynchronize(sg.k));
-            const int32_t kc = std::min<int32_t>(max_len, std::max<int32_t>(d->h_extent[ci & 1], 1));
-            part->extent = std::max(part->extent, kc);
-            CUF(cudaStreamWaitEvent(d->s_out, sg.k, 0));
-            const size_t o0 = (size_t)r0 * (size_t)max_len;
-            CopyOutArgs CO{};
-            CO.m = m;
-            auto copy_plane = [&](void* host, const void* dev, size_t elt, int32_t old_dirty) -> cudaError_t {
-                // whole 64-byte lines of host memory for the one-byte planes too (a partial line is a read-modify-write for the host)
-                const int32_t rnd = elt == 1 ? (int32_t)std::max<int64_t>(32, h->copy_round) : 32;
-                const int32_t cols = std::min<int32_t>(max_len, (std::max(kc, old_dirty) + rnd - 1) / rnd * rnd);
-                part->d2h_bytes += (int64_t)m * cols * (int64_t)elt;
-                uint8_t* dst = reinterpret_cast<uint8_t*>(host) + o0 * elt;
-                if (cols >= max_len) return cudaMemcpyAsync(dst, dev, (size_t)m * (size_t)max_len * elt, cudaMemcpyDeviceToHost, d->s_out);
-                void* dmap = nullptr;                                     // trimmed rows: stores of a kernel into the mapped host plane
-                if (!h->no_copy_kernel && ((size_t)max_len * elt) % 16 == 0 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0 &&
-                    cudaHostGetDevicePointer(&dmap, dst, 0) == cudaSuccess && dmap) {
-                    CO.p[CO.n_planes++] = CopyOutPlane{reinterpret_cast<const uint8_t*>(dev), reinterpret_cast<uint8_t*>(dmap), (uint32_t)(max_len * elt), (uint32_t)(cols * elt)};
-                    return cudaSuccess;
-                }
-                cudaGetLastError();
-                return cudaMemcpy2DAsync(dst, (size_t)max_len * elt, dev, (size_t)max_len * elt, (size_t)cols * elt, (size_t)m, cudaMemcpyDeviceToHost, d->s_out);
-            };
-            CUF(copy_plane(out->input_ids, sg.ids.p, 4, J.old_dirty[0]));
-            CUF(copy_plane(out->attention_mask, sg.mask.p, 1, J.old_dirty[1]));
-            if (want_tt) CUF(copy_plane(out->token_type_ids, sg.tt.p, 1, J.old_dirty[2]));
-            if (want_seq) CUF(copy_plane(out->sequence_id, sg.seq.p, 1, J.old_dirty[3]));
-            if (CO.n_planes) {
-                LaunchScope::cur_stream = d->s_out;
-                { LaunchScope ls(h, d, "k_copy_out"); k_copy_out<<<(unsigned)std::max<int64_t>(1, h->copy_blocks), 256, 0, d->s_out>>>(CO); }
-                LaunchScope::cur_stream = st;
-                CUF(cudaGetLastError());
-            }
-            CUF(cudaMemcpyAsync(out->row_len + r0, sg.row_len.p, (size_t)m * 4, cudaMemcpyDeviceToHost, d->s_out));
-            part->d2h_bytes += m * 4;
-            if (has_pair) {
-                CUF(cudaMemcpyAsync(out->seq_len + r0, sg.seq_len.p, (size_t)m * 4, cudaMemcpyDeviceToHost, d->s_out));
-                CUF(cudaMemcpyAsync(out->row_status + r0, sg.status.p, (size_t)m, cudaMemcpyDeviceToHost, d->s_out));
-                part->d2h_bytes += m * 5;
-            }
-            CUF(cudaEventRecord(sg.d2h, d->s_out));
-        }
-        CUF(cudaStreamSynchronize(d->s_out));
-        unsigned long long tokens_after = 0, nerr = 0;
+// The devices' rows of a host-buffer encode or windows call, part g on device g: the frame around chunks(d, cuts, part), which issues
+// the chunks of the part's rows on d->stream and leaves a failure in the part's status.  A part is ordered behind the previous user of
+// the device context's shared work areas (stream_enter) before anything touches them; the word cache is sized for its largest chunk;
+// the token and error counters are read around its chunks.
+template <class Part, class Chunks>
+void run_parts(genztok_t* h, const EncodeJob& J, const std::vector<int64_t>& dcut, std::vector<Part>& parts, Chunks chunks) {
+    for (auto& pt : parts) pt.bind(h);
+    run_shards(dcut, [&](int g) {
+        DeviceCtx* d = h->devs[(size_t)g];
+        Part* part = &parts[(size_t)g];
+        cudaStream_t st = d->stream;
+        CUF(cudaSetDevice(d->device));
+        LaunchScope::cur_stream = st;
+        FAIL_RC(stream_enter(h, d, st));
+        std::vector<int64_t> cuts;
+        int64_t most = 0;
+        { const int64_t big = chunk_cuts(h, J, dcut[(size_t)g], dcut[(size_t)g + 1], &cuts, &most);
+          if (big >= 0) PFAIL(GENZTOK_E_LIMIT, "document %lld is larger than max_chunk_bytes=%lld", (long long)big, (long long)h->max_chunk_bytes) }
+        FAIL_RC(ensure_cache(h, d, st, most));
+        if (J.want_offs) FAIL_RC(ensure_piece_lens(h, d, st));
+        unsigned long long tokens_before = 0, tokens_after = 0, nerr = 0;
+        CUF(cudaMemcpyAsync(&tokens_before, d->C.ctr + C_TOKENS, 8, cudaMemcpyDeviceToHost, st));
+        CUF(cudaStreamSynchronize(st));
+        chunks(d, cuts, part);
+        if (part->status.rc) return;
         CUF(cudaMemcpyAsync(&tokens_after, d->C.ctr + C_TOKENS, 8, cudaMemcpyDeviceToHost, st));
         CUF(cudaMemcpyAsync(&nerr, d->C.ctr + C_ERR, 8, cudaMemcpyDeviceToHost, st));
         CUF(cudaStreamSynchronize(st));
         if (nerr) PFAIL(GENZTOK_E_CUDA, "internal error: device pipeline reported %llu inconsistencies", nerr)
         part->tokens = (int64_t)(tokens_after - tokens_before);
-        return;
-    }
+        FAIL_RC(stream_leave(h, d, st));
+    });
+}
 
+// Fixed layout, pipelined over chunks: H2D(i + 1) | kernels(i) | D2H(i - 1) on three streams, two sets of chunk buffers.
+// Only the columns that can differ from padding travel back: [0, max(extent of the chunk, what the pooled host plane still
+// holds from its last use)), rounded up to 32; a fresh host plane takes whole rows once.
+void encode_fixed_chunks(genztok_t* h, DeviceCtx* d, const EncodeJob& J, const std::vector<int64_t>& cuts, EncodePart* part) {
+    cudaStream_t st = d->stream;
+    genztok_encoded_t* out = J.out;
+    const bool has_pair = J.has_pair, want_tt = J.want_tt, want_seq = J.want_seq;
+    const int32_t max_len = J.max_len;
+    const size_t nc = cuts.size() - 1;
+    if (!d->s_in) CUF(cudaStreamCreateWithFlags(&d->s_in, cudaStreamNonBlocking));
+    if (!d->s_out) CUF(cudaStreamCreateWithFlags(&d->s_out, cudaStreamNonBlocking));
+    if (!d->h_extent) CUF(cudaHostAlloc(reinterpret_cast<void**>(&d->h_extent), 64, cudaHostAllocDefault));
+    int64_t mm = 0, mtb = 0, mpb = 0;
+    for (size_t ci = 0; ci < nc; ci++) {
+        mm = std::max(mm, cuts[ci + 1] - cuts[ci]);
+        mtb = std::max(mtb, J.text_off[cuts[ci + 1]] - J.text_off[cuts[ci]]);
+        if (has_pair) mpb = std::max(mpb, J.pair_off[cuts[ci + 1]] - J.pair_off[cuts[ci]]);
+    }
+    const size_t mtot = (size_t)mm * (size_t)max_len;
+    for (int sidx = 0; sidx < (nc > 1 ? 2 : 1); sidx++) {
+        DeviceCtx::Stage& sg = d->stage[sidx];
+        for (cudaEvent_t* e : {&sg.h2d, &sg.k, &sg.d2h}) if (!*e) CUF(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+        CUF(sg.text.ensure((size_t)mtb + 96)); CUF(sg.toff.ensure((size_t)(mm + 1) * 8));
+        if (has_pair) { CUF(sg.pair.ensure((size_t)mpb + 96)); CUF(sg.poff.ensure((size_t)(mm + 1) * 8)); }
+        CUF(sg.ids.ensure(mtot * 4)); CUF(sg.mask.ensure(mtot)); CUF(sg.row_len.ensure((size_t)mm * 4)); CUF(sg.extent.ensure(16));
+        if (want_tt) CUF(sg.tt.ensure(mtot));
+        if (want_seq) CUF(sg.seq.ensure(mtot));
+        if (has_pair) { CUF(sg.seq_len.ensure((size_t)mm * 4)); CUF(sg.status.ensure((size_t)mm)); }
+    }
+    Side in_a[2], in_b[2];                                            // the sides of the chunks in the two sets
+    auto issue_h2d = [&](size_t ci) -> bool {
+        DeviceCtx::Stage& sg = d->stage[ci & 1];
+        if (ci >= 2 && cudaStreamWaitEvent(d->s_in, sg.k, 0) != cudaSuccess) return false;      // the kernels of chunk ci - 2 have read this set's inputs
+        if (upload_chunk(J, cuts[ci], cuts[ci + 1], sg.text, sg.toff, sg.pair, sg.poff, d->s_in, &in_a[ci & 1], &in_b[ci & 1]) != cudaSuccess) return false;
+        return cudaEventRecord(sg.h2d, d->s_in) == cudaSuccess;
+    };
+    auto fail_sync = [&]() { cudaStreamSynchronize(d->s_in); cudaStreamSynchronize(st); cudaStreamSynchronize(d->s_out); };
+    if (nc && !issue_h2d(0)) { fail_sync(); PFAIL(GENZTOK_E_CUDA, "host to device copy failed: %s", cudaGetErrorString(cudaGetLastError())) }
+    for (size_t ci = 0; ci < nc; ci++) {
+        DeviceCtx::Stage& sg = d->stage[ci & 1];
+        const int64_t r0 = cuts[ci], r1 = cuts[ci + 1], m = r1 - r0;
+        // kernels of chunk ci: behind its inputs, and behind the copy-out of the chunk that used this set of planes before
+        CUF(cudaStreamWaitEvent(st, sg.h2d, 0));
+        if (ci >= 2) CUF(cudaStreamWaitEvent(st, sg.d2h, 0));
+        genztok_dev_planes_t P{};
+        P.input_ids = sg.ids.as<int32_t>(); P.attention_mask = sg.mask.as<uint8_t>(); P.row_len = sg.row_len.as<int32_t>();
+        if (want_tt) P.token_type_ids = sg.tt.as<int8_t>();
+        if (want_seq) P.sequence_id = sg.seq.as<int8_t>();
+        if (has_pair) { P.seq_len = sg.seq_len.as<int32_t>(); P.row_status = sg.status.as<uint8_t>(); }
+        if (int rc = encode_fixed_on_device(h, d, st, in_a[ci & 1], has_pair ? &in_b[ci & 1] : nullptr, m, max_len, J.flags, P)) { fail_sync(); FAIL_RC(rc) }
+        CUF(cudaMemsetAsync(sg.extent.p, 0, 4, st));
+        { LaunchScope ls(h, d, "k_row_extent");
+          k_row_extent<<<(unsigned)std::min<int64_t>((m + 255) / 256, (int64_t)d->sm_count * 4), 256, 0, st>>>(P.row_len, has_pair ? P.seq_len : nullptr, m, sg.extent.as<int32_t>()); }
+        CUF(cudaMemcpyAsync(d->h_extent + (ci & 1), sg.extent.p, 4, cudaMemcpyDeviceToHost, st));
+        CUF(cudaEventRecord(sg.k, st));
+        // the next chunk's inputs travel while these kernels run
+        if (ci + 1 < nc && !issue_h2d(ci + 1)) { fail_sync(); PFAIL(GENZTOK_E_CUDA, "host to device copy failed: %s", cudaGetErrorString(cudaGetLastError())) }
+        // copy-out of chunk ci: the host learns the extent (the only wait of this loop), then the trimmed planes go on their own stream
+        CUF(cudaEventSynchronize(sg.k));
+        const int32_t kc = std::min<int32_t>(max_len, std::max<int32_t>(d->h_extent[ci & 1], 1));
+        part->extent = std::max(part->extent, kc);
+        CUF(cudaStreamWaitEvent(d->s_out, sg.k, 0));
+        const size_t o0 = (size_t)r0 * (size_t)max_len;
+        CopyOutArgs CO{};
+        CO.m = m;
+        auto copy_plane = [&](void* host, const void* dev, size_t elt, int32_t old_dirty) -> cudaError_t {
+            // whole 64-byte lines of host memory for the one-byte planes too (a partial line is a read-modify-write for the host)
+            const int32_t rnd = elt == 1 ? (int32_t)std::max<int64_t>(32, h->copy_round) : 32;
+            const int32_t cols = std::min<int32_t>(max_len, (std::max(kc, old_dirty) + rnd - 1) / rnd * rnd);
+            part->d2h_bytes += (int64_t)m * cols * (int64_t)elt;
+            uint8_t* dst = reinterpret_cast<uint8_t*>(host) + o0 * elt;
+            if (cols >= max_len) return cudaMemcpyAsync(dst, dev, (size_t)m * (size_t)max_len * elt, cudaMemcpyDeviceToHost, d->s_out);
+            void* dmap = nullptr;                                     // trimmed rows: stores of a kernel into the mapped host plane
+            if (!h->no_copy_kernel && ((size_t)max_len * elt) % 16 == 0 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0 &&
+                cudaHostGetDevicePointer(&dmap, dst, 0) == cudaSuccess && dmap) {
+                CO.p[CO.n_planes++] = CopyOutPlane{reinterpret_cast<const uint8_t*>(dev), reinterpret_cast<uint8_t*>(dmap), (uint32_t)(max_len * elt), (uint32_t)(cols * elt)};
+                return cudaSuccess;
+            }
+            cudaGetLastError();
+            return cudaMemcpy2DAsync(dst, (size_t)max_len * elt, dev, (size_t)max_len * elt, (size_t)cols * elt, (size_t)m, cudaMemcpyDeviceToHost, d->s_out);
+        };
+        CUF(copy_plane(out->input_ids, sg.ids.p, 4, J.old_dirty[0]));
+        CUF(copy_plane(out->attention_mask, sg.mask.p, 1, J.old_dirty[1]));
+        if (want_tt) CUF(copy_plane(out->token_type_ids, sg.tt.p, 1, J.old_dirty[2]));
+        if (want_seq) CUF(copy_plane(out->sequence_id, sg.seq.p, 1, J.old_dirty[3]));
+        if (CO.n_planes) {
+            LaunchScope::cur_stream = d->s_out;
+            { LaunchScope ls(h, d, "k_copy_out"); k_copy_out<<<(unsigned)std::max<int64_t>(1, h->copy_blocks), 256, 0, d->s_out>>>(CO); }
+            LaunchScope::cur_stream = st;
+            CUF(cudaGetLastError());
+        }
+        CUF(cudaMemcpyAsync(out->row_len + r0, sg.row_len.p, (size_t)m * 4, cudaMemcpyDeviceToHost, d->s_out));
+        part->d2h_bytes += m * 4;
+        if (has_pair) {
+            CUF(cudaMemcpyAsync(out->seq_len + r0, sg.seq_len.p, (size_t)m * 4, cudaMemcpyDeviceToHost, d->s_out));
+            CUF(cudaMemcpyAsync(out->row_status + r0, sg.status.p, (size_t)m, cudaMemcpyDeviceToHost, d->s_out));
+            part->d2h_bytes += m * 5;
+        }
+        CUF(cudaEventRecord(sg.d2h, d->s_out));
+    }
+    CUF(cudaStreamSynchronize(d->s_out));
+}
+
+// Ragged layout, chunk after chunk on d->stream: the planes come home into the part's pinned arrays, row offsets relative to the part.
+void encode_ragged_chunks(genztok_t* h, DeviceCtx* d, const EncodeJob& J, const std::vector<int64_t>& cuts, EncodePart* part) {
+    cudaStream_t st = d->stream;
+    genztok_encoded_t* out = J.out;
+    const bool has_pair = J.has_pair, has_max_len = J.has_max_len, want_spans = J.want_spans;
+    const int32_t max_len = J.max_len;
+    const int8_t eos8 = eos_as_i8(d);
+    const int64_t rb = cuts.front(), re = cuts.back();
     for (size_t ci = 0; ci + 1 < cuts.size(); ci++) {
         const int64_t r0 = cuts[ci], r1 = cuts[ci + 1], m = r1 - r0;
-        const int64_t tb0 = J.text_off[r0], tb = J.text_off[r1] - tb0;
-        const int64_t pb0 = has_pair ? J.pair_off[r0] : 0, pb = has_pair ? J.pair_off[r1] - pb0 : 0;
-        // Offsets stay absolute (as in the caller's buffer): the chunk is copied to dev + (tb0 & 15) and the base
-        // pointer is shifted by -tb0, so that base + 16k is 16-byte aligned, as the kernel's LDG.128 needs.
-        const int64_t ta = tb0 & 15, pa = pb0 & 15;
+        const int64_t tb = J.text_off[r1] - J.text_off[r0], pb = has_pair ? J.pair_off[r1] - J.pair_off[r0] : 0;
         CUF(d->text.ensure((size_t)tb + 96)); CUF(d->toff.ensure((size_t)(m + 1) * 8));
-        if (tb) CUF(cudaMemcpyAsync(d->text.as<uint8_t>() + ta, J.text + tb0, (size_t)tb, cudaMemcpyHostToDevice, st));
-        CUF(cudaMemcpyAsync(d->toff.p, J.text_off + r0, (size_t)(m + 1) * 8, cudaMemcpyHostToDevice, st));
-        if (has_pair) {
-            CUF(d->pair.ensure((size_t)pb + 96)); CUF(d->poff.ensure((size_t)(m + 1) * 8));
-            if (pb) CUF(cudaMemcpyAsync(d->pair.as<uint8_t>() + pa, J.pair + pb0, (size_t)pb, cudaMemcpyHostToDevice, st));
-            CUF(cudaMemcpyAsync(d->poff.p, J.pair_off + r0, (size_t)(m + 1) * 8, cudaMemcpyHostToDevice, st));
-        }
-        Side a{d->text.as<uint8_t>() + ta - tb0, d->toff.as<int64_t>(), tb};
-        Side b{has_pair ? d->pair.as<uint8_t>() + pa - pb0 : nullptr, d->poff.as<int64_t>(), pb};
-
-        // ---- ragged layout ---------------------------------------------------------------------------
-        if (tb + pb + 16 > h->max_chunk_bytes) PFAIL(GENZTOK_E_LIMIT, "chunk too large")
+        if (has_pair) { CUF(d->pair.ensure((size_t)pb + 96)); CUF(d->poff.ensure((size_t)(m + 1) * 8)); }
+        Side a, b;
+        CUF(upload_chunk(J, r0, r1, d->text, d->toff, d->pair, d->poff, st, &a, &b));
         CUF(d->redo.ensure((size_t)m * 4)); CUF(d->fix.ensure((size_t)m * 4));
         CUF(d->L.ensure((size_t)m * 4)); CUF(d->keep.ensure((size_t)m * 4)); CUF(d->out_len.ensure((size_t)m * 8));
         CUF(d->row_off.ensure((size_t)(m + 1) * 8)); CUF(d->tail.ensure((size_t)m));
@@ -1470,17 +1544,12 @@ void encode_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int64
         { LaunchScope ls(h, d, "k_post_rows"); k_post_rows<<<(unsigned)std::min<int64_t>((m + 7) / 8, (int64_t)d->sm_count * 8), 256, 0, st>>>(d->T, Q, nullptr); }
         CUF(cudaGetLastError());
         // bring the chunk home; offsets are kept relative to this device's part
-        const size_t old = part->ids.size();
-        if (old == 0 && r1 < re) {                                  // first chunk of several: room for the whole part at this chunk's tokens per row (+ 12 %)
-            const size_t est = (size_t)((double)total * (double)(re - rb) / (double)m * 1.125) + 4096;
-            bool ok = part->ids.reserve(est) && part->mask.reserve(est);
-            if (has_pair) ok = ok && part->tt.reserve(est) && part->seq.reserve(est);
-            if (J.want_offs) ok = ok && part->tok_offs.reserve(2 * est);
-            if (!ok) PFAIL(GENZTOK_E_NOMEM, "pinned host allocation failed")
-        }
-        bool grown = part->ids.resize(old + (size_t)total) && part->mask.resize(old + (size_t)total);
-        if (has_pair) grown = grown && part->tt.resize(old + (size_t)total) && part->seq.resize(old + (size_t)total);
-        if (J.want_offs) grown = grown && part->tok_offs.resize(2 * (old + (size_t)total));
+        const size_t old = part->ids.size(), nt = old + (size_t)total;
+        // first chunk of several: room for the whole part at this chunk's tokens per row (+ 12 %)
+        const size_t est = (old == 0 && r1 < re) ? (size_t)((double)total * (double)(re - rb) / (double)m * 1.125) + 4096 : 0;
+        bool grown = grow(part->ids, nt, est) && grow(part->mask, nt, est);
+        if (has_pair) grown = grown && grow(part->tt, nt, est) && grow(part->seq, nt, est);
+        if (J.want_offs) grown = grown && grow(part->tok_offs, 2 * nt, 2 * est);
         grown = grown && part->offs.resize((size_t)m + 1);
         if (!grown) PFAIL(GENZTOK_E_NOMEM, "pinned host allocation failed")
         int64_t* const offs = part->offs.data();
@@ -1516,15 +1585,6 @@ void encode_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int64
         part->total += total;
         if (want_spans) { for (int64_t i = 1; i <= m; i++) out->span_off[r0 + i] = part->span_total + soffs[i]; part->span_total += span_n; }
     }
-    unsigned long long tokens_after = 0, nerr = 0;
-    CUF(cudaMemcpyAsync(&tokens_after, d->C.ctr + C_TOKENS, 8, cudaMemcpyDeviceToHost, st));
-    CUF(cudaMemcpyAsync(&nerr, d->C.ctr + C_ERR, 8, cudaMemcpyDeviceToHost, st));
-    CUF(cudaStreamSynchronize(st));
-    if (nerr) PFAIL(GENZTOK_E_CUDA, "internal error: device pipeline reported %llu inconsistencies", nerr)
-    part->tokens = (int64_t)(tokens_after - tokens_before);
-#undef PFAIL
-#undef FAIL_RC
-#undef CUF
 }
 
 }  // namespace
@@ -1538,29 +1598,19 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
     if (h->devs.empty()) return fail(h, GENZTOK_E_NODEVICE, "this handle was created without a CUDA device; there is no CPU path");
     memset(out, 0, sizeof *out);
     std::lock_guard<std::mutex> lk(h->mu);
-    EncodeJob J{};
-    J.text = text; J.text_off = text_off; J.pair = pair; J.pair_off = pair_off;
-    J.max_len = max_len; J.padding = padding; J.truncation = truncation; J.flags = flags; J.out = out;
-    J.has_pair = pair_off != nullptr;
+    EncodeJob J = make_job(text, text_off, pair, pair_off, max_len, flags);
+    J.padding = padding; J.truncation = truncation; J.out = out;
     J.has_max_len = max_len != GENZTOK_MAX_LEN_NONE;
     J.want_spans = (flags & GENZTOK_WANT_SPANS) != 0;       // return_offset: produced by the ragged pipeline
-    J.want_offs = (flags & GENZTOK_WANT_OFFSETS) != 0;      // offset_mapping: produced by the ragged pipeline too
-    // the fixed regime; with offsets it is computed by the ragged pipeline, whose rows then all hold max_len entries, and
-    // presented in the fixed layout
+    // the fixed regime; with offsets (offset_mapping) it is computed by the ragged pipeline, whose rows then all hold max_len
+    // entries, and presented in the fixed layout
     const bool fixed_layout = J.has_max_len && max_len >= 1 && padding && truncation && fixed_fits(h->devs[0], max_len) && !J.want_spans;
     J.fixed = fixed_layout && !J.want_offs;
-    J.want_tt = J.has_pair && (flags & GENZTOK_WANT_TOKEN_TYPE);
-    J.want_seq = J.has_pair && (flags & GENZTOK_WANT_SEQUENCE_ID);
     const bool has_pair = J.has_pair, fixed = J.fixed;
     OutBlock* ob = new OutBlock();
     out->_owner = ob;
     out->n = n; out->has_pair = has_pair;
-    auto free_nolock = [&]() {
-        for (auto& pr : ob->pinned) { h->plane_meta.erase(pr.first); host_pool_put(h, pr.first, pr.second); }
-        for (void* p : ob->mallocs) free(p);
-        delete ob;
-        memset(out, 0, sizeof *out);
-    };
+    auto free_nolock = [&]() { discard_block(h, ob); memset(out, 0, sizeof *out); };
     // offsets in the fixed regime: every row of the ragged result is a padded / truncated row of max_len entries
     auto present_fixed = [&]() -> int {
         if (out->row_off[n] != n * (int64_t)max_len) {
@@ -1605,34 +1655,15 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
         if (it != h->plane_meta.end() && it->second.rows == n && it->second.width == max_len && it->second.elt == elts4[k]) J.old_dirty[k] = it->second.dirty_cols;
     }
 
-    // Shard by document across the handle's devices (SURVEY.md 8e): contiguous row ranges balanced by bytes, one host
-    // thread per device, no collective; every device writes its own rows of the result.
+    // every device writes its own rows of the result; the documents are balanced by bytes
     const int G = (int)h->devs.size();
-    std::vector<int64_t> dcut((size_t)G + 1, n);
-    dcut[0] = 0;
-    {
-        auto weight = [&](int64_t r) { return text_off[r] + (has_pair ? pair_off[r] : 0) + 64 * r; };
-        const int64_t wtot = weight(n) - weight(0);
-        for (int g = 1; g < G; g++) {
-            const int64_t want = weight(0) + wtot * g / G;
-            int64_t lo = dcut[(size_t)g - 1], hi = n;
-            while (lo < hi) { int64_t mid = (lo + hi) / 2; if (weight(mid) < want) lo = mid + 1; else hi = mid; }
-            dcut[(size_t)g] = lo;
-        }
-    }
+    const std::vector<int64_t> dcut = shard_rows(G, n, [&](int64_t r) { return text_off[r] + (has_pair ? pair_off[r] : 0) + 64 * r; });
     std::vector<EncodePart> parts((size_t)G);
-    for (auto& pt : parts) pt.bind(h);
-    if (G == 1 || n < 2 * G) {
-        if (G > 1) { for (int g = 1; g <= G; g++) dcut[(size_t)g] = n; }
-        encode_rows_on_device(h, h->devs[0], J, 0, n, &parts[0]);
-    } else {
-        std::vector<std::thread> th;
-        for (int g = 0; g < G; g++)
-            th.emplace_back([&, g]() { encode_rows_on_device(h, h->devs[(size_t)g], J, dcut[(size_t)g], dcut[(size_t)g + 1], &parts[(size_t)g]); });
-        for (auto& t : th) t.join();
-    }
+    run_parts(h, J, dcut, parts, [&](DeviceCtx* d, const std::vector<int64_t>& cuts, EncodePart* pt) {
+        if (fixed) encode_fixed_chunks(h, d, J, cuts, pt); else encode_ragged_chunks(h, d, J, cuts, pt);
+    });
     for (auto& pt : parts)
-        if (pt.rc) { free_nolock(); { std::lock_guard<std::mutex> l(h->err_mu); h->err = pt.err; } return pt.rc; }
+        if (pt.status.rc) { free_nolock(); return pt.status.report(h); }
     out->real_tokens = 0;
     out->d2h_bytes = 0;
     for (auto& pt : parts) { out->real_tokens += pt.tokens; out->d2h_bytes += pt.d2h_bytes; }
@@ -1677,7 +1708,7 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
         if (J.want_offs) { toffs = (int32_t*)malloc(std::max<size_t>(ntot * 8, 16)); ob->mallocs.push_back(toffs); }
         for (int g = 0; g < G; g++) {
             EncodePart& pt = parts[(size_t)g];
-            const int64_t rb = (G == 1 || n < 2 * G) ? (g == 0 ? 0 : n) : dcut[(size_t)g], re = (G == 1 || n < 2 * G) ? n : dcut[(size_t)g + 1];
+            const int64_t rb = dcut[(size_t)g], re = dcut[(size_t)g + 1];
             if (base) for (int64_t r = rb + 1; r <= re; r++) out->row_off[r] += base;
             if (J.want_spans && sbase) for (int64_t r = rb + 1; r <= re; r++) out->span_off[r] += sbase;
             if (!pt.ids.empty()) {
@@ -1703,48 +1734,26 @@ namespace {
 
 // What one device collects for its documents [rb, re) of genztok_encode_windows (chunk after chunk, in document order).
 struct WindowPart {
-    int rc = GENZTOK_OK;
-    std::string err;
+    PartStatus status;
     int64_t n_win = 0, tokens = 0, d2h_bytes = 0;
-    PinnedVec<int32_t> ids, row_len, seq_len, start, tok_offs; PinnedVec<uint8_t> mask, status; PinnedVec<int8_t> tt, seq; PinnedVec<int64_t> doc, offs;
-    void bind(genztok_t* h) { for (auto* v : {&ids, &row_len, &seq_len, &start, &tok_offs}) v->h = h; mask.h = h; status.h = h; tt.h = h; seq.h = h; doc.h = h; offs.h = h; }
+    PinnedVec<int32_t> ids, row_len, seq_len, start, tok_offs; PinnedVec<uint8_t> mask, row_status; PinnedVec<int8_t> tt, seq; PinnedVec<int64_t> doc, offs;
+    void bind(genztok_t* h) { for (auto* v : {&ids, &row_len, &seq_len, &start, &tok_offs}) v->h = h; mask.h = h; row_status.h = h; tt.h = h; seq.h = h; doc.h = h; offs.h = h; }
 };
 
-// Windows of documents [rb, re) on one device: per chunk the text goes up, both steps run, the planes and maps come home.
+// Windows of one device's chunks: per chunk the text goes up, both steps run, the planes and maps come home.
 // win_off[r] for r in (rb, re] is written relative to the part's first window.
-void windows_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int32_t stride, int64_t* win_off, int64_t rb, int64_t re, WindowPart* part) {
+void windows_chunks(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int32_t stride, int64_t* win_off, const std::vector<int64_t>& cuts, WindowPart* part) {
+    cudaStream_t st = d->stream;
     const bool has_pair = J.has_pair;
     const int32_t W = J.max_len;
-    cudaStream_t st = d->stream;
-#define PFAIL(code, ...) { char _b[400]; snprintf(_b, sizeof _b, __VA_ARGS__); part->rc = (code); part->err = _b; cudaStreamSynchronize(st); return; }
-#define FAIL_RC(call) { int _rc = (call); if (_rc) { part->rc = _rc; { std::lock_guard<std::mutex> _l(h->err_mu); part->err = h->err; } cudaStreamSynchronize(st); return; } }
-#define CUF(call) { cudaError_t _e = (call); if (_e != cudaSuccess) PFAIL(GENZTOK_E_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(_e), __FILE__, __LINE__) }
-    CUF(cudaSetDevice(d->device));
-    LaunchScope::cur_stream = st;
-    FAIL_RC(stream_enter(h, d, st));
-    std::vector<int64_t> cuts;
-    int64_t most = 0;
-    { const int64_t big = chunk_cuts(h, J, rb, re, &cuts, &most);
-      if (big >= 0) PFAIL(GENZTOK_E_LIMIT, "document %lld is larger than max_chunk_bytes=%lld", (long long)big, (long long)h->max_chunk_bytes) }
-    FAIL_RC(ensure_cache(h, d, st, most));
-    unsigned long long tokens_before = 0;
-    CUF(cudaMemcpyAsync(&tokens_before, d->C.ctr + C_TOKENS, 8, cudaMemcpyDeviceToHost, st));
+    const int64_t rb = cuts.front(), re = cuts.back();
     for (size_t ci = 0; ci + 1 < cuts.size(); ci++) {
         const int64_t r0 = cuts[ci], r1 = cuts[ci + 1], m = r1 - r0;
-        const int64_t tb0 = J.text_off[r0], tb = J.text_off[r1] - tb0;
-        const int64_t pb0 = has_pair ? J.pair_off[r0] : 0, pb = has_pair ? J.pair_off[r1] - pb0 : 0;
-        // (as in the ragged path: offsets stay absolute, the chunk lands at dev + (tb0 & 15) behind a base pointer shifted by -tb0)
-        const int64_t ta = tb0 & 15, pa = pb0 & 15;
+        const int64_t tb = J.text_off[r1] - J.text_off[r0], pb = has_pair ? J.pair_off[r1] - J.pair_off[r0] : 0;
         CUF(d->text.ensure((size_t)tb + 96)); CUF(d->toff.ensure((size_t)(m + 1) * 8));
-        if (tb) CUF(cudaMemcpyAsync(d->text.as<uint8_t>() + ta, J.text + tb0, (size_t)tb, cudaMemcpyHostToDevice, st));
-        CUF(cudaMemcpyAsync(d->toff.p, J.text_off + r0, (size_t)(m + 1) * 8, cudaMemcpyHostToDevice, st));
-        if (has_pair) {
-            CUF(d->pair.ensure((size_t)pb + 96)); CUF(d->poff.ensure((size_t)(m + 1) * 8));
-            if (pb) CUF(cudaMemcpyAsync(d->pair.as<uint8_t>() + pa, J.pair + pb0, (size_t)pb, cudaMemcpyHostToDevice, st));
-            CUF(cudaMemcpyAsync(d->poff.p, J.pair_off + r0, (size_t)(m + 1) * 8, cudaMemcpyHostToDevice, st));
-        }
-        Side a{d->text.as<uint8_t>() + ta - tb0, d->toff.as<int64_t>(), tb};
-        Side b{has_pair ? d->pair.as<uint8_t>() + pa - pb0 : nullptr, d->poff.as<int64_t>(), pb};
+        if (has_pair) { CUF(d->pair.ensure((size_t)pb + 96)); CUF(d->poff.ensure((size_t)(m + 1) * 8)); }
+        Side a, b;
+        CUF(upload_chunk(J, r0, r1, d->text, d->toff, d->pair, d->poff, st, &a, &b));
         CUF(d->win.woff.ensure((size_t)(m + 1) * 8));
         int64_t K = 0;
         FAIL_RC(windows_layout(h, d, st, a, has_pair ? &b : nullptr, m, W, stride, J.want_offs, d->win.woff.as<int64_t>(), &K));
@@ -1759,21 +1768,14 @@ void windows_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int3
         if (J.want_offs) { CUF(d->win.plane_offs.ensure(tot * 8 + 16)); P.offsets = d->win.plane_offs.as<int32_t>(); }
         FAIL_RC(windows_write(h, d, st, has_pair, m, W, stride, J.flags, d->win.woff.as<int64_t>(), K, P, d->win.doc.as<int64_t>(), d->win.start.as<int32_t>(), r0));
         const size_t o = (size_t)part->n_win, n1 = o + (size_t)K;
-        if (ci == 0 && r1 < re) {                                    // first chunk of several: room for the part at this chunk's windows per document (+ 12 %)
-            const size_t est = (size_t)((double)K * (double)(re - rb) / (double)m * 1.125) + 64;
-            bool ok = part->ids.reserve(est * W) && part->mask.reserve(est * W) && part->row_len.reserve(est) && part->doc.reserve(est) && part->start.reserve(est);
-            if (J.want_tt) ok = ok && part->tt.reserve(est * W);
-            if (J.want_seq) ok = ok && part->seq.reserve(est * W);
-            if (J.want_offs) ok = ok && part->tok_offs.reserve(2 * est * W);
-            if (has_pair) ok = ok && part->seq_len.reserve(est) && part->status.reserve(est);
-            if (!ok) PFAIL(GENZTOK_E_NOMEM, "pinned host allocation failed")
-        }
-        bool grown = part->ids.resize(n1 * W) && part->mask.resize(n1 * W) && part->row_len.resize(n1) && part->doc.resize(n1) && part->start.resize(n1) &&
-                     part->offs.resize((size_t)m + 1);
-        if (J.want_tt) grown = grown && part->tt.resize(n1 * W);
-        if (J.want_seq) grown = grown && part->seq.resize(n1 * W);
-        if (J.want_offs) grown = grown && part->tok_offs.resize(2 * n1 * W);
-        if (has_pair) grown = grown && part->seq_len.resize(n1) && part->status.resize(n1);
+        // first chunk of several: room for the part at this chunk's windows per document (+ 12 %)
+        const size_t est = (ci == 0 && r1 < re) ? (size_t)((double)K * (double)(re - rb) / (double)m * 1.125) + 64 : 0;
+        bool grown = grow(part->ids, n1 * W, est * W) && grow(part->mask, n1 * W, est * W) && grow(part->row_len, n1, est) && grow(part->doc, n1, est) &&
+                     grow(part->start, n1, est) && part->offs.resize((size_t)m + 1);
+        if (J.want_tt) grown = grown && grow(part->tt, n1 * W, est * W);
+        if (J.want_seq) grown = grown && grow(part->seq, n1 * W, est * W);
+        if (J.want_offs) grown = grown && grow(part->tok_offs, 2 * n1 * W, 2 * est * W);
+        if (has_pair) grown = grown && grow(part->seq_len, n1, est) && grow(part->row_status, n1, est);
         if (!grown) PFAIL(GENZTOK_E_NOMEM, "pinned host allocation failed")
         if (K) {
             CUF(cudaMemcpyAsync(part->ids.data() + o * W, P.input_ids, tot * 4, cudaMemcpyDeviceToHost, st));
@@ -1786,7 +1788,7 @@ void windows_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int3
             CUF(cudaMemcpyAsync(part->start.data() + o, d->win.start.p, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
             if (has_pair) {
                 CUF(cudaMemcpyAsync(part->seq_len.data() + o, P.seq_len, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
-                CUF(cudaMemcpyAsync(part->status.data() + o, P.row_status, (size_t)K, cudaMemcpyDeviceToHost, st));
+                CUF(cudaMemcpyAsync(part->row_status.data() + o, P.row_status, (size_t)K, cudaMemcpyDeviceToHost, st));
             }
         }
         CUF(cudaMemcpyAsync(part->offs.data(), d->win.woff.p, (size_t)(m + 1) * 8, cudaMemcpyDeviceToHost, st));
@@ -1796,16 +1798,6 @@ void windows_rows_on_device(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int3
         for (int64_t i = 1; i <= m; i++) win_off[r0 + i] = part->n_win + offs[i];
         part->n_win += K;
     }
-    unsigned long long tokens_after = 0, nerr = 0;
-    CUF(cudaMemcpyAsync(&tokens_after, d->C.ctr + C_TOKENS, 8, cudaMemcpyDeviceToHost, st));
-    CUF(cudaMemcpyAsync(&nerr, d->C.ctr + C_ERR, 8, cudaMemcpyDeviceToHost, st));
-    CUF(cudaStreamSynchronize(st));
-    if (nerr) PFAIL(GENZTOK_E_CUDA, "internal error: device pipeline reported %llu inconsistencies", nerr)
-    part->tokens = (int64_t)(tokens_after - tokens_before);
-    FAIL_RC(stream_leave(h, d, st));
-#undef PFAIL
-#undef FAIL_RC
-#undef CUF
 }
 
 int check_window_args(genztok_t* h, int32_t max_len, int32_t stride, uint32_t flags) {
@@ -1828,21 +1820,10 @@ int genztok_encode_windows(genztok_t* h, const uint8_t* text, const int64_t* tex
     if (h->devs.empty()) return fail(h, GENZTOK_E_NODEVICE, "this handle was created without a CUDA device; there is no CPU path");
     memset(out, 0, sizeof *out);
     std::lock_guard<std::mutex> lk(h->mu);
-    EncodeJob J{};
-    J.text = text; J.text_off = text_off; J.pair = pair; J.pair_off = pair_off;
-    J.max_len = max_len; J.padding = 1; J.truncation = 1; J.flags = flags;
-    J.has_pair = pair_off != nullptr; J.has_max_len = true; J.fixed = true;
-    J.want_offs = (flags & GENZTOK_WANT_OFFSETS) != 0;
-    J.want_tt = J.has_pair && (flags & GENZTOK_WANT_TOKEN_TYPE);
-    J.want_seq = J.has_pair && (flags & GENZTOK_WANT_SEQUENCE_ID);
+    EncodeJob J = make_job(text, text_off, pair, pair_off, max_len, flags);
     const bool has_pair = J.has_pair;
     OutBlock* ob = new OutBlock();
-    auto bail = [&](int code) {
-        for (auto& pr : ob->pinned) host_pool_put(h, pr.first, pr.second);
-        delete ob;
-        memset(out, 0, sizeof *out);
-        return code;
-    };
+    auto bail = [&](int code) { discard_block(h, ob); memset(out, 0, sizeof *out); return code; };
     // every result buffer leaves the pool to hold windows: what plane_meta knew of it no longer holds
     auto take = [&](auto* p) { if (p) h->plane_meta.erase(p); return p; };
     int64_t* win_off = take(out_alloc<int64_t>(h, ob, (size_t)n + 1));
@@ -1850,30 +1831,11 @@ int genztok_encode_windows(genztok_t* h, const uint8_t* text, const int64_t* tex
     win_off[0] = 0;
     // shard the documents across the devices as genztok_encode does: contiguous ranges balanced by bytes
     const int G = (int)h->devs.size();
-    const bool one = G == 1 || n < 2 * G;
-    std::vector<int64_t> dcut((size_t)G + 1, n);
-    dcut[0] = 0;
-    if (!one) {
-        auto weight = [&](int64_t r) { return text_off[r] + (has_pair ? pair_off[r] : 0) + 64 * r; };
-        const int64_t wtot = weight(n) - weight(0);
-        for (int g = 1; g < G; g++) {
-            const int64_t want = weight(0) + wtot * g / G;
-            int64_t lo = dcut[(size_t)g - 1], hi = n;
-            while (lo < hi) { int64_t mid = (lo + hi) / 2; if (weight(mid) < want) lo = mid + 1; else hi = mid; }
-            dcut[(size_t)g] = lo;
-        }
-    } else for (int g = 1; g <= G; g++) dcut[(size_t)g] = n;
+    const std::vector<int64_t> dcut = shard_rows(G, n, [&](int64_t r) { return text_off[r] + (has_pair ? pair_off[r] : 0) + 64 * r; });
     std::vector<WindowPart> parts((size_t)G);
-    for (auto& pt : parts) pt.bind(h);
-    if (one) windows_rows_on_device(h, h->devs[0], J, stride, win_off, 0, n, &parts[0]);
-    else {
-        std::vector<std::thread> th;
-        for (int g = 0; g < G; g++)
-            th.emplace_back([&, g]() { windows_rows_on_device(h, h->devs[(size_t)g], J, stride, win_off, dcut[(size_t)g], dcut[(size_t)g + 1], &parts[(size_t)g]); });
-        for (auto& t : th) t.join();
-    }
+    run_parts(h, J, dcut, parts, [&](DeviceCtx* d, const std::vector<int64_t>& cuts, WindowPart* pt) { windows_chunks(h, d, J, stride, win_off, cuts, pt); });
     for (auto& pt : parts)
-        if (pt.rc) { { std::lock_guard<std::mutex> l(h->err_mu); h->err = pt.err; } return bail(pt.rc); }
+        if (pt.status.rc) return bail(pt.status.report(h));
     int64_t K = 0;
     for (auto& pt : parts) K += pt.n_win;
     const size_t tot = (size_t)K * (size_t)max_len;
@@ -1905,7 +1867,7 @@ int genztok_encode_windows(genztok_t* h, const uint8_t* text, const int64_t* tex
             if (J.want_tt) memcpy(E.token_type_ids + o * w, pt.tt.data(), k * w);
             if (J.want_seq) memcpy(E.sequence_id + o * w, pt.seq.data(), k * w);
             if (J.want_offs) memcpy(E.offsets + 2 * o * w, pt.tok_offs.data(), k * w * 8);
-            if (has_pair) { memcpy(E.seq_len + o, pt.seq_len.data(), k * 4); memcpy(E.row_status + o, pt.status.data(), k); }
+            if (has_pair) { memcpy(E.seq_len + o, pt.seq_len.data(), k * 4); memcpy(E.row_status + o, pt.row_status.data(), k); }
         }
         base += pt.n_win;
         E.real_tokens += pt.tokens; E.d2h_bytes += pt.d2h_bytes;
@@ -1974,11 +1936,6 @@ int genztok_encode_windows_device(genztok_t* h, int dev, const uint8_t* d_text, 
     return stream_leave(h, d, st);
 }
 
-}  // extern "C"
-
-extern "C" {
-
-// ---- decode -------------------------------------------------------------------------------------------
 }  // extern "C"
 
 namespace {
@@ -2158,54 +2115,42 @@ int genztok_decode_device_into(genztok_t* h, int dev, const int32_t* d_ids, cons
     return decode_on_device(h, h->devs[(size_t)dev], d_ids, d_ids_off, n, width, d_out_off, d_bytes, total_bytes, stream, capacity);
 }
 
-void genztok_free_text(genztok_t* h, genztok_text_t* out) {
-    if (!out || !out->_owner) return;
-    OutBlock* ob = reinterpret_cast<OutBlock*>(out->_owner);
-    {
-        std::lock_guard<std::mutex> lk(h->mu);
-        for (auto& pr : ob->pinned) host_pool_put(h, pr.first, pr.second);
-    }
-    for (void* p : ob->mallocs) free(p);
-    delete ob;
-    memset(out, 0, sizeof *out);
-}
+void genztok_free_text(genztok_t* h, genztok_text_t* out) { free_result(h, out); }
 
 }  // extern "C"
 
 namespace {
 
-struct DecodePart { int rc = GENZTOK_OK; std::vector<uint8_t> bytes; std::vector<int64_t> off; };   // off: row ends relative to the part's start
+struct DecodePart { PartStatus status; std::vector<uint8_t> bytes; std::vector<int64_t> off; };   // off: row ends relative to the part's start
 
 // Rows [r0, r1) on one device, in chunks of chunk_rows: ids up, both passes, text and offsets down.
-void decode_rows_on_device(genztok_t* h, DeviceCtx* d, const int32_t* ids, const int64_t* ids_off, int32_t width, int64_t r0, int64_t r1, DecodePart* P) {
-    cudaSetDevice(d->device);
+void decode_rows_on_device(genztok_t* h, DeviceCtx* d, const int32_t* ids, const int64_t* ids_off, int32_t width, int64_t r0, int64_t r1, DecodePart* part) {
     cudaStream_t st = d->stream;
+    CUF(cudaSetDevice(d->device));
     const int64_t rows_per_chunk = std::max<int64_t>(1, h->chunk_rows);
-    P->off.reserve((size_t)(r1 - r0));
+    part->off.reserve((size_t)(r1 - r0));
     int64_t total_all = 0;
     std::vector<int64_t> offs;
-    for (int64_t c0 = r0; c0 < r1 && P->rc == GENZTOK_OK; c0 += rows_per_chunk) {
+    for (int64_t c0 = r0; c0 < r1; c0 += rows_per_chunk) {
         const int64_t c1 = std::min(r1, c0 + rows_per_chunk), m = c1 - c0;
         const int64_t i0 = ids_off ? ids_off[c0] : c0 * width, i1 = ids_off ? ids_off[c1] : c1 * width, ni = i1 - i0;
         cudaError_t e;
         if ((e = d->ids.ensure((size_t)ni * 4 + 16)) != cudaSuccess || (e = d->row_off.ensure((size_t)(m + 1) * 8)) != cudaSuccess ||
-            (e = d->toff.ensure((size_t)(m + 1) * 8)) != cudaSuccess) { P->rc = fail(h, GENZTOK_E_CUDA, "cudaMalloc: %s", cudaGetErrorString(e)); break; }
-        if (ni) cudaMemcpyAsync(d->ids.p, ids + i0, (size_t)ni * 4, cudaMemcpyHostToDevice, st);
+            (e = d->toff.ensure((size_t)(m + 1) * 8)) != cudaSuccess) PFAIL(GENZTOK_E_CUDA, "cudaMalloc: %s", cudaGetErrorString(e))
+        if (ni) CUF(cudaMemcpyAsync(d->ids.p, ids + i0, (size_t)ni * 4, cudaMemcpyHostToDevice, st));
         const int64_t* d_ioff = nullptr;
-        if (ids_off) { cudaMemcpyAsync(d->toff.p, ids_off + c0, (size_t)(m + 1) * 8, cudaMemcpyHostToDevice, st); d_ioff = d->toff.as<int64_t>(); }
+        if (ids_off) { CUF(cudaMemcpyAsync(d->toff.p, ids_off + c0, (size_t)(m + 1) * 8, cudaMemcpyHostToDevice, st)); d_ioff = d->toff.as<int64_t>(); }
         int64_t total = 0;
-        P->rc = decode_on_device(h, d, d->ids.as<int32_t>() - (ids_off ? i0 : 0), d_ioff, m, width, d->row_off.as<int64_t>(), nullptr, &total, st);
-        if (P->rc) break;
-        if ((e = d->text.ensure((size_t)total + 16)) != cudaSuccess) { P->rc = fail(h, GENZTOK_E_CUDA, "cudaMalloc: %s", cudaGetErrorString(e)); break; }
-        P->rc = decode_on_device(h, d, d->ids.as<int32_t>() - (ids_off ? i0 : 0), d_ioff, m, width, d->row_off.as<int64_t>(), d->text.as<uint8_t>(), nullptr, st);
-        if (P->rc) break;
+        FAIL_RC(decode_on_device(h, d, d->ids.as<int32_t>() - (ids_off ? i0 : 0), d_ioff, m, width, d->row_off.as<int64_t>(), nullptr, &total, st));
+        if ((e = d->text.ensure((size_t)total + 16)) != cudaSuccess) PFAIL(GENZTOK_E_CUDA, "cudaMalloc: %s", cudaGetErrorString(e))
+        FAIL_RC(decode_on_device(h, d, d->ids.as<int32_t>() - (ids_off ? i0 : 0), d_ioff, m, width, d->row_off.as<int64_t>(), d->text.as<uint8_t>(), nullptr, st));
         offs.resize((size_t)m + 1);
-        const size_t old = P->bytes.size();
-        P->bytes.resize(old + (size_t)total);
-        if (total) cudaMemcpyAsync(P->bytes.data() + old, d->text.p, (size_t)total, cudaMemcpyDeviceToHost, st);
-        cudaMemcpyAsync(offs.data(), d->row_off.p, (size_t)(m + 1) * 8, cudaMemcpyDeviceToHost, st);
-        if ((e = cudaStreamSynchronize(st)) != cudaSuccess) { P->rc = fail(h, GENZTOK_E_CUDA, "decode: %s", cudaGetErrorString(e)); break; }
-        for (int64_t i = 1; i <= m; i++) P->off.push_back(total_all + offs[(size_t)i]);
+        const size_t old = part->bytes.size();
+        part->bytes.resize(old + (size_t)total);
+        if (total) CUF(cudaMemcpyAsync(part->bytes.data() + old, d->text.p, (size_t)total, cudaMemcpyDeviceToHost, st));
+        CUF(cudaMemcpyAsync(offs.data(), d->row_off.p, (size_t)(m + 1) * 8, cudaMemcpyDeviceToHost, st));
+        if ((e = cudaStreamSynchronize(st)) != cudaSuccess) PFAIL(GENZTOK_E_CUDA, "decode: %s", cudaGetErrorString(e))
+        for (int64_t i = 1; i <= m; i++) part->off.push_back(total_all + offs[(size_t)i]);
         total_all += total;
     }
 }
@@ -2224,36 +2169,13 @@ int genztok_decode(genztok_t* h, const int32_t* ids, const int64_t* ids_off, int
     int64_t* off = out_alloc<int64_t>(h, ob, (size_t)n + 1);
     if (!off) { delete ob; return fail(h, GENZTOK_E_NOMEM, "pinned host allocation failed"); }
     off[0] = 0;
-    // Shard by row across the handle's devices (SURVEY.md 8e): contiguous row ranges balanced by ids, one host thread per
-    // device, no collective; the parts' texts are concatenated and their offsets shifted.
+    // the rows are balanced by ids; the parts' texts are concatenated and their offsets shifted
     const int G = (int)h->devs.size();
-    std::vector<int64_t> dcut((size_t)G + 1, n);
-    dcut[0] = 0;
-    if (G > 1 && n >= 2 * G) {
-        auto weight = [&](int64_t r) { return (ids_off ? ids_off[r] - ids_off[0] : r * (int64_t)width) + 16 * r; };
-        const int64_t wtot = weight(n);
-        for (int g = 1; g < G; g++) {
-            const int64_t want = wtot * g / G;
-            int64_t lo = dcut[(size_t)g - 1], hi = n;
-            while (lo < hi) { int64_t mid = (lo + hi) / 2; if (weight(mid) < want) lo = mid + 1; else hi = mid; }
-            dcut[(size_t)g] = lo;
-        }
-    }
+    const std::vector<int64_t> dcut = shard_rows(G, n, [&](int64_t r) { return (ids_off ? ids_off[r] - ids_off[0] : r * (int64_t)width) + 16 * r; });
     std::vector<DecodePart> parts((size_t)G);
-    if (G == 1 || n < 2 * G) {
-        decode_rows_on_device(h, h->devs[0], ids, ids_off, width, 0, n, &parts[0]);
-    } else {
-        std::vector<std::thread> th;
-        for (int g = 0; g < G; g++)
-            th.emplace_back([&, g]() { decode_rows_on_device(h, h->devs[(size_t)g], ids, ids_off, width, dcut[(size_t)g], dcut[(size_t)g + 1], &parts[(size_t)g]); });
-        for (auto& t : th) t.join();
-    }
+    run_shards(dcut, [&](int g) { decode_rows_on_device(h, h->devs[(size_t)g], ids, ids_off, width, dcut[(size_t)g], dcut[(size_t)g + 1], &parts[(size_t)g]); });
     for (auto& pt : parts)
-        if (pt.rc) {
-            for (auto& pr : ob->pinned) host_pool_put(h, pr.first, pr.second);
-            delete ob;
-            return pt.rc;
-        }
+        if (pt.status.rc) { discard_block(h, ob); return pt.status.report(h); }
     size_t total_all = 0;
     for (auto& pt : parts) total_all += pt.bytes.size();
     uint8_t* bytes = (uint8_t*)malloc(std::max<size_t>(total_all, 16));
@@ -2279,14 +2201,15 @@ int genztok_preprocess(genztok_t* h, int op, const uint8_t* text, const int64_t*
     CU(cudaSetDevice(d->device));
     cudaStream_t st = d->stream;
     LaunchScope::cur_stream = st;
+    int rc = stream_enter(h, d, st);                                 // (the text, offset and length buffers are the encode's too)
+    if (rc) return rc;
     OutBlock* ob = new OutBlock();
     int64_t* off = out_alloc<int64_t>(h, ob, (size_t)n + 1);
     if (!off) { delete ob; return fail(h, GENZTOK_E_NOMEM, "pinned host allocation failed"); }
     off[0] = 0;
     std::vector<uint8_t> acc;
     int64_t total_all = 0;
-    int rc = GENZTOK_OK;
-    auto bail = [&](int code) { for (auto& pr : ob->pinned) host_pool_put(h, pr.first, pr.second); delete ob; return code; };
+    auto bail = [&](int code) { discard_block(h, ob); return code; };
     int64_t r0 = 0;
     while (r0 < n) {
         int64_t r1 = std::min<int64_t>(n, r0 + h->chunk_rows);
@@ -2319,6 +2242,8 @@ int genztok_preprocess(genztok_t* h, int op, const uint8_t* text, const int64_t*
         total_all += total;
         r0 = r1;
     }
+    rc = stream_leave(h, d, st);
+    if (rc) return bail(rc);
     uint8_t* bytes = (uint8_t*)malloc(std::max<size_t>(acc.size(), 16));
     if (!acc.empty()) memcpy(bytes, acc.data(), acc.size());
     ob->mallocs.push_back(bytes);
@@ -2543,22 +2468,24 @@ int genztok_preprocess_device(genztok_t* h, int dev, int op, const uint8_t* d_te
     cudaStream_t st = stream ? (cudaStream_t)stream : d->stream;
     LaunchScope::cur_stream = st;
     const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + 7) / 8, (int64_t)d->sm_count * 8));
+    int rc = stream_enter(h, d, st);
+    if (rc) return rc;
     if (!d_out) {
         CU(d->out_len.ensure((size_t)std::max<int64_t>(n, 1) * 8));
         PrepArgs A{d_text, d_text_off, n, op, d->out_len.as<int64_t>(), nullptr, nullptr};
         if (n > 0) { LaunchScope ls(h, d, "k_prep_len"); k_prep<false><<<grid, 256, 0, st>>>(A); }
-        int rc = launch_scan(h, d, st, d->out_len.as<int64_t>(), d_out_off, n);
+        rc = launch_scan(h, d, st, d->out_len.as<int64_t>(), d_out_off, n);
         if (rc) return rc;
         if (total_bytes) {
             CU(cudaMemcpyAsync(total_bytes, d_out_off + n, 8, cudaMemcpyDeviceToHost, st));
             CU(cudaStreamSynchronize(st));
         }
-        return GENZTOK_OK;
+        return stream_leave(h, d, st);
     }
     PrepArgs A{d_text, d_text_off, n, op, nullptr, d_out_off, d_out};
     if (n > 0) { LaunchScope ls(h, d, "k_prep_write"); k_prep<true><<<grid, 256, 0, st>>>(A); }
     CU(cudaGetLastError());
-    return GENZTOK_OK;
+    return stream_leave(h, d, st);
 }
 
 // ---- helpers ----------------------------------------------------------------------------------------------
