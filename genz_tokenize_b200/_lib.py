@@ -91,6 +91,8 @@ SIGNATURES = {
                                           C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "genztok_qa_best_spans_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int, C.c_void_p, C.c_int64,
                                               C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "genztok_mlm_mask_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_double,
+                                         C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "genztok_digest_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p]),
 }
 

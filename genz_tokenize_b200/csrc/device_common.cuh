@@ -88,6 +88,14 @@ __device__ __forceinline__ void st_release_u32(uint32_t* p, uint32_t v) {
 __device__ __forceinline__ void st_cs128(void* p, uint4 v) { __stcs(reinterpret_cast<uint4*>(p), v); }
 __device__ __forceinline__ void st_cs32(void* p, uint32_t v) { __stcs(reinterpret_cast<uint32_t*>(p), v); }
 
+// splitmix64's finaliser and golden-ratio increment: the counter-based hashes of the synthetic workload, the plane digest
+// (synth.cuh) and MLM masking (mlm.cuh); genz_tokenize_b200/workload.py::_mix64 is the same function on the host.
+static const uint64_t GOLD = 0x9E3779B97F4A7C15ULL;
+__host__ __device__ __forceinline__ uint64_t mix64(uint64_t x) {
+    x ^= x >> 30; x *= 0xBF58476D1CE4E5B9ULL; x ^= x >> 27; x *= 0x94D049BB133111EBULL; x ^= x >> 31;
+    return x;
+}
+
 __device__ __forceinline__ uint32_t rotl32(uint32_t x, int r) { return (x << r) | (x >> (32 - r)); }
 __device__ __forceinline__ uint32_t fmix32(uint32_t h) {
     h ^= h >> 16; h *= 0x85ebca6bu; h ^= h >> 13; h *= 0xc2b2ae35u; h ^= h >> 16;

@@ -13,10 +13,12 @@
 //   -> k_window_rows -> k_post_rows (row list).
 // Decode is k_decode_len (lengths, trailing pad runs) -> k_scan_i64 -> k_decode_write.
 // Extractive QA over the windows' offsets (qa.cuh): [k_qa_char_to_byte ->] k_qa_labels; k_qa_spans -> k_qa_spans_docs.
+// MLM inputs and labels from an id plane (mlm.cuh): k_mlm_mask<WHOLE_WORD>.
 #include <cuda_runtime.h>
 
 #include <algorithm>
 #include <atomic>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -34,6 +36,7 @@
 #include "flat.cuh"
 #include "gather.cuh"
 #include "host_tables.hpp"
+#include "mlm.cuh"
 #include "post.cuh"
 #include "prep.cuh"
 #include "qa.cuh"
@@ -83,6 +86,8 @@ struct DeviceCtx {
     DevBuf len_arena;                             // piece byte lengths beside tok_arena (offset_mapping; allocated on first use)
     DevBuf offs;                                  // ragged pass: [total][2] token byte offsets (offset_mapping)
     DevBuf qa_ans, qa_win;                        // QA: byte spans converted from characters; per-window best spans
+    const uint32_t* mlm_cont = nullptr;           // MLM (mlm.cuh): the handle's continuation bitset and replacement ids, uploaded
+    const int32_t* mlm_repl = nullptr;            // on the first MLM call of this device
     DevBuf dec_lead;                              // decode: per-row description left by the length pass for the write pass
     DevBuf dec_stat;                              // decode, fixed-width rows: ids in front of the pad runs, summed by the length pass
     double dec_avg_lead = -1;                     // ... per row, once the host has read it (-1: not known for the current batch)
@@ -174,6 +179,11 @@ struct genztok {
     // `dirty_cols` equal to padding.  A call that reuses it copies only the columns that can differ (see encode_fixed_pipelined).
     struct PlaneMeta { int64_t rows; int32_t width, dirty_cols, elt; int32_t pad; };
     std::map<void*, PlaneMeta> plane_meta;
+    // MLM masking (mlm.cuh), built from the tables on the first MLM call: bit id of mlm_cont is set when decoder[id] ends in "@@";
+    // mlm_repl lists, ascending, the ids in the decoder that are not special
+    bool mlm_built = false;
+    std::vector<uint32_t> mlm_cont;
+    std::vector<int32_t> mlm_repl;
 };
 
 namespace {
@@ -972,7 +982,7 @@ void free_result(genztok_t* h, Out* out) {
 // ================================================================================================
 extern "C" {
 
-const char* genztok_version(void) { return "genztok-b200 0.3 (sm_100a)"; }
+const char* genztok_version(void) { return "genztok-b200 0.4 (sm_100a)"; }
 
 const char* genztok_last_error(const genztok_t* h) { return h ? h->err.c_str() : g_create_err.c_str(); }
 
@@ -2434,6 +2444,66 @@ int genztok_qa_best_spans_device(genztok_t* h, int dev, const float* d_start_log
     if (n_docs > 0) {
         LaunchScope ls(h, d, "k_qa_spans_docs", 8 * (n_docs + 1) + n_docs * (4 + 4 + 8 + 8 + 8));
         k_qa_spans_docs<<<(unsigned)std::min<int64_t>((n_docs + 255) / 256, (int64_t)d->sm_count * 8), 256, 0, st>>>(A);
+    }
+    CU(cudaGetLastError());
+    return stream_leave(h, d, st);
+}
+
+// MLM masking (mlm.cuh).  Arguments are checked before the device slot, as for the QA calls.
+static void mlm_build(genztok_t* h) {
+    if (h->mlm_built) return;
+    const HostTables& H = h->H;
+    h->mlm_cont.assign((size_t)((H.n_ids + 31) / 32), 0u);
+    h->mlm_repl.clear();
+    for (int64_t id = 0; id < H.n_ids; id++) {
+        const int64_t e = H.decoder[(size_t)id];
+        if (e < 0) continue;
+        const std::string& s = H.enc_keys[(size_t)e];
+        if (s.size() >= 2 && s.compare(s.size() - 2, 2, "@@") == 0) h->mlm_cont[(size_t)(id >> 5)] |= 1u << (id & 31);
+        if (std::find(H.special_id, H.special_id + 5, (int32_t)id) == H.special_id + 5) h->mlm_repl.push_back((int32_t)id);
+    }
+    h->mlm_built = true;
+}
+
+int genztok_mlm_mask_device(genztok_t* h, int dev, const int32_t* d_ids, int64_t n, int32_t width, const int64_t* d_row_keys, uint64_t seed,
+                            double mlm_probability, double mask_replace_prob, double random_replace_prob, int whole_word, int32_t* d_masked_ids,
+                            int64_t* d_labels, void* stream) {
+    if (!h) return GENZTOK_E_INVALID;
+    const double p = mlm_probability, a = mask_replace_prob, b = random_replace_prob;
+    for (double x : {p, a, b})
+        if (!(x >= 0.0 && x <= 1.0))
+            return fail(h, GENZTOK_E_INVALID, "genztok_mlm_mask_device: probabilities must be finite and in [0, 1] (got %g, %g, %g)", p, a, b);
+    if (a + b > 1.0) return fail(h, GENZTOK_E_INVALID, "genztok_mlm_mask_device: mask_replace_prob + random_replace_prob must be <= 1 (got %g + %g)", a, b);
+    if (n < 0 || width < 1) return fail(h, GENZTOK_E_INVALID, "genztok_mlm_mask_device: n >= 0 and width >= 1 needed (got %lld, %d)", (long long)n, width);
+    if (n > 0 && (!d_ids || !d_masked_ids || !d_labels)) return fail(h, GENZTOK_E_INVALID, "genztok_mlm_mask_device: ids, masked ids and labels are required");
+    if (n > 0 && (const void*)d_masked_ids == (const void*)d_ids)
+        return fail(h, GENZTOK_E_INVALID, "genztok_mlm_mask_device: the masked ids must not overwrite the input ids");
+    std::lock_guard<std::mutex> lk(h->mu);
+    mlm_build(h);
+    if (b > 0.0 && h->mlm_repl.empty())
+        return fail(h, GENZTOK_E_INVALID, "genztok_mlm_mask_device: random_replace_prob > 0 but the vocab has no id to draw (every id is special)");
+    if (dev < 0 || dev >= (int)h->devs.size()) return fail(h, GENZTOK_E_NODEVICE, "no such device slot %d (handle has %d)", dev, (int)h->devs.size());
+    DeviceCtx* d = h->devs[(size_t)dev];
+    CU(cudaSetDevice(d->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : d->stream;
+    LaunchScope::cur_stream = st;
+    if (!d->mlm_repl) CU(upload(d, h->mlm_repl, &d->mlm_repl));
+    if (!d->mlm_cont) CU(upload(d, h->mlm_cont, &d->mlm_cont));
+    int rc = stream_enter(h, d, st);
+    if (rc) return rc;
+    const double two32 = 4294967296.0;
+    MlmArgs A{};
+    A.ids = d_ids; A.n = n; A.W = width; A.row_keys = d_row_keys;
+    A.s0 = mix64(seed ^ MLM_K);
+    A.t_sel = (uint64_t)std::floor(p * two32); A.t_mask = (uint64_t)std::floor(a * two32); A.t_mask_rand = (uint64_t)std::floor((a + b) * two32);
+    A.cont = d->mlm_cont; A.repl = d->mlm_repl; A.m = (uint32_t)h->mlm_repl.size(); A.n_ids = d->T.n_ids;
+    A.pad = d->T.pad; A.bos = d->T.bos; A.eos = d->T.eos; A.msk = d->T.msk; A.unk = d->T.unk;
+    A.out = d_masked_ids; A.labels = d_labels;
+    if (n > 0) {
+        LaunchScope ls(h, d, whole_word ? "k_mlm_mask_words" : "k_mlm_mask_tokens", n * (int64_t)width * (4 + 4 + 8) + (d_row_keys ? 8 * n : 0));
+        const unsigned grid = (unsigned)std::min<int64_t>((n + 7) / 8, (int64_t)d->sm_count * 64);
+        if (whole_word) k_mlm_mask<true><<<grid, 256, 0, st>>>(A);
+        else k_mlm_mask<false><<<grid, 256, 0, st>>>(A);
     }
     CU(cudaGetLastError());
     return stream_leave(h, d, st);

@@ -24,11 +24,7 @@ struct SynthArgs {
     uint8_t* bytes;
 };
 
-static const uint64_t SY_GOLD = 0x9E3779B97F4A7C15ULL, SY_K_LEN = 0xA5A5A5A5A5A5A5A5ULL, SY_K_NOISE = 0xC3C3C3C3C3C3C3C3ULL;
-__host__ __device__ __forceinline__ uint64_t mix64(uint64_t x) {
-    x ^= x >> 30; x *= 0xBF58476D1CE4E5B9ULL; x ^= x >> 27; x *= 0x94D049BB133111EBULL; x ^= x >> 31;
-    return x;
-}
+static const uint64_t SY_K_LEN = 0xA5A5A5A5A5A5A5A5ULL, SY_K_NOISE = 0xC3C3C3C3C3C3C3C3ULL;
 // first index with cdf32[i] > u (numpy searchsorted side='right'), clamped to nw - 1
 __device__ __forceinline__ uint32_t synth_pick(const SynthTables& T, uint32_t u) {
     uint32_t lo = 0, hi = T.nw;
@@ -41,7 +37,7 @@ __global__ void __launch_bounds__(256) k_synth(SynthTables T, SynthArgs A) {
     const char alphabet[37] = "abcdefghijklmnopqrstuvwxyz0123456789";
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < A.n; i += (int64_t)gridDim.x * blockDim.x) {
         const uint64_t d = (uint64_t)(A.doc0 + i);
-        const uint64_t D = mix64(A.seed * SY_GOLD + 2ULL * d + (uint64_t)A.side);
+        const uint64_t D = mix64(A.seed * GOLD + 2ULL * d + (uint64_t)A.side);
         const uint32_t k = (uint32_t)A.lo + (uint32_t)(((mix64(D ^ SY_K_LEN) >> 32) * (uint64_t)(A.hi - A.lo + 1)) >> 32);
         int64_t len = 0;
         uint8_t* out = WRITE ? A.bytes + A.off[i] : nullptr;
@@ -50,7 +46,7 @@ __global__ void __launch_bounds__(256) k_synth(SynthTables T, SynthArgs A) {
             len += n;
         };
         for (uint32_t j = 0; j < k; j++) {
-            const uint64_t R = mix64(D + (uint64_t)(j + 1) * SY_GOLD);
+            const uint64_t R = mix64(D + (uint64_t)(j + 1) * GOLD);
             const uint32_t w = synth_pick(T, (uint32_t)(R >> 32));
             int kind = -1;
             uint64_t Q = 0;
@@ -92,11 +88,11 @@ __global__ void __launch_bounds__(256) k_plane_digest(DigestArgs A) {
     const int32_t W = A.W, W4 = A.W >> 2;
     uint64_t sum = 0;
     for (int64_t r = warp; r < A.n; r += n_warps) {
-        const uint64_t rk = mix64((uint64_t)(A.row0 + r) * SY_GOLD);
-        for (int32_t i = lane; i < W; i += 32) sum += mix64((rk + (uint64_t)i * SY_GOLD) ^ (uint64_t)A.ids[r * W + i]);
+        const uint64_t rk = mix64((uint64_t)(A.row0 + r) * GOLD);
+        for (int32_t i = lane; i < W; i += 32) sum += mix64((rk + (uint64_t)i * GOLD) ^ (uint64_t)A.ids[r * W + i]);
         for (int32_t i = lane; i < W4; i += 32) {
-            sum += mix64((rk + ((1ULL << 32) + (uint64_t)i) * SY_GOLD) ^ (uint64_t)A.mask[r * W4 + i]);
-            if (A.tt) sum += mix64((rk + ((2ULL << 32) + (uint64_t)i) * SY_GOLD) ^ (uint64_t)A.tt[r * W4 + i]);
+            sum += mix64((rk + ((1ULL << 32) + (uint64_t)i) * GOLD) ^ (uint64_t)A.mask[r * W4 + i]);
+            if (A.tt) sum += mix64((rk + ((2ULL << 32) + (uint64_t)i) * GOLD) ^ (uint64_t)A.tt[r * W4 + i]);
         }
     }
 #pragma unroll

@@ -10,7 +10,8 @@ Extensions over the reference (which is one string per call): `encode_batch` / `
 form but encode_device can also return `offset_mapping` (HF's return_offsets_mapping): each token's
 (start, end) byte range in its own document's UTF-8 text, (0, 0) for tokens that are not from the text.
 `qa_labels` / `qa_best_spans` turn those planes into extractive-QA training labels and read a QA model's
-start / end logits back into answer spans, on the GPU.
+start / end logits back into answer spans, on the GPU.  `mlm_mask` turns any fixed-layout id plane into masked-language-model
+inputs and labels (token or whole-word masking), on the GPU.
 """
 import ctypes as C
 import operator
@@ -786,6 +787,60 @@ class Tokenize(object):
         if host:
             return {k: v.cpu().numpy() for k, v in out.items()}
         return out
+
+    # ---- masked language modelling ---------------------------------------------------------------------------------------------
+    def mlm_mask(self, input_ids, seed, mlm_probability=0.15, whole_word=False, mask_replace_prob=0.8, random_replace_prob=0.1, row_keys=None):
+        """Masked-language-model inputs and labels from a fixed-layout id plane [n, W] (an encode_batch, encode_device,
+        encode_windows(_device) or DataCollection batch's input_ids): returns (masked_ids int32 [n, W], labels int64 [n, W]).
+        Eligible columns (ids in [0, n_ids) that are not special) are selected with probability `mlm_probability`, per token or,
+        with `whole_word`, per word (a piece whose vocab string ends in "@@" continues into the next column); a selected column
+        becomes the mask id with probability `mask_replace_prob`, a random non-special vocab id with `random_replace_prob`,
+        else keeps its id, and is labelled with its original id; every other column keeps its id and is labelled -100.  The
+        draws are a pure function of (seed, row key, row contents), row r's key being `row_keys[r]` (int64 [n]) or r: take a
+        new `seed` per epoch for dynamic masking.  include/genztok.h states the hashes.  A CUDA tensor stays on its device, on
+        torch's current stream; a numpy plane is copied to the handle's device and the results back.  Other integer dtypes are
+        converted to int32, ids outside the int32 range becoming -1 or 2^31 - 1 (ineligible either way, and so returned);
+        float, bool and complex planes raise TypeError."""
+        import torch
+        host = not isinstance(input_ids, torch.Tensor)
+        if host:
+            a = np.asarray(input_ids)
+            if a.dtype.kind not in "iu":
+                raise TypeError("mlm_mask: input_ids must hold integers (got %s)" % a.dtype)
+            if not self._device_ids:
+                raise GenztokError("mlm_mask: this handle was created without a CUDA device; there is no CPU path")
+            dev = torch.device("cuda", self._device_ids[0])
+            if a.dtype.itemsize >= 4 and a.dtype != np.int32:                # ids outside int32 can never be eligible: keep them so
+                a = np.minimum(a, 2 ** 31 - 1) if a.dtype.kind == "u" else np.clip(a, -1, 2 ** 31 - 1)
+            ids = torch.from_numpy(np.ascontiguousarray(a, dtype=np.int32)).to(dev)
+        else:
+            dev = input_ids.device
+            if input_ids.dtype not in (torch.int8, torch.int16, torch.int32, torch.int64, torch.uint8):
+                raise TypeError("mlm_mask: input_ids must hold integers (got %s)" % input_ids.dtype)
+            ids = input_ids
+            if ids.dtype == torch.int64:                                    # ids outside int32 can never be eligible: keep them so
+                ids = ids.clamp(-1, 2 ** 31 - 1)
+            ids = ids.to(torch.int32).contiguous()
+        if ids.ndim != 2:
+            raise ValueError("mlm_mask: input_ids must be a fixed-layout [n, W] plane (got shape %s)" % (tuple(ids.shape),))
+        n, W = int(ids.shape[0]), int(ids.shape[1])
+        keys = None
+        if row_keys is not None:
+            keys = row_keys if isinstance(row_keys, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(np.asarray(row_keys, dtype=np.int64)))
+            if tuple(keys.shape) != (n,):
+                raise ValueError("mlm_mask: row_keys must have shape (%d,) (got %s)" % (n, tuple(keys.shape)))
+            keys = keys.to(dev, torch.int64).contiguous()
+        out = torch.empty((n, W), dtype=torch.int32, device=dev)
+        labels = torch.empty((n, W), dtype=torch.int64, device=dev)
+        rc = self._lib.genztok_mlm_mask_device(self._h, 0, ids.data_ptr(), n, W, keys.data_ptr() if keys is not None else None,
+                                               operator.index(seed) & (2 ** 64 - 1), float(mlm_probability), float(mask_replace_prob),
+                                               float(random_replace_prob), int(bool(whole_word)), out.data_ptr(), labels.data_ptr(),
+                                               self._torch_stream(dev))
+        if rc:
+            self._err(rc, "genztok_mlm_mask_device")
+        if host:
+            return out.cpu().numpy(), labels.cpu().numpy()
+        return out, labels
 
     # ---- measurement plumbing (bench.py, tests): synthetic workload on the device, plane digest, error counter -----------
     def synth_device(self, seed, doc0, n, side=0, lo=3, hi=13, noise=0.0, device=None):

@@ -305,6 +305,37 @@ int genztok_qa_best_spans_device(genztok_t *h, int dev, const float *d_start_log
                                  int64_t n_docs, int32_t max_answer_len, float *d_score, float *d_null_score, int64_t *d_window,
                                  int32_t *d_columns /* [n_docs][2] */, int32_t *d_span /* [n_docs][2] */, void *stream);
 
+/* ---- masked-language-model inputs and labels (the pre-training recipe of the reference's RoBERTa / DistilBERT models) ------
+ * Reads a fixed-layout id plane d_ids [n][width] (any encode, window or gathered batch) and writes d_masked_ids [n][width] (int32)
+ * and d_labels [n][width] (int64): at a selected column the replaced id and the original id, everywhere else the input id and
+ * -100 (HF's DataCollatorForLanguageModeling conventions).  d_ids is not modified; d_masked_ids must not be d_ids.
+ *  - Eligible column: 0 <= id < n_ids (the size of the handle's id table) and id is none of the five special ids.  Framing, pads,
+ *    an existing mask, unk and ids the vocab does not know are never selected, so every label is -100 or a valid class index.
+ *  - Continuation id: an id in the decoder whose string ends in the two bytes "@@" (the pieces decode glues to the next piece);
+ *    no other id continues, including ids absent from the decoder and ids outside [0, n_ids).
+ *  - Group of column j: j itself; with whole_word, the largest g <= j with g == 0 or ids[r][g - 1] not a continuation id.  A group
+ *    can hold ineligible columns (a word cut by truncation runs into the forced </s>).  Selection is decided per group and
+ *    applies to the group's eligible columns.
+ *  - Hashes, mod 2^64, with mix64 the splitmix64 finaliser, GOLD = 0x9E3779B97F4A7C15, K = 0x6D6C6D5F6D61736B and key_r =
+ *    d_row_keys[r] (NULL: r):  R_r = mix64(mix64(seed ^ K) + key_r * GOLD).  Column j of row r is selected when it is eligible
+ *    and (mix64(R_r + (2 g(j) + 1) * GOLD) >> 32) < T_sel.  A selected column draws v = mix64(R_r + (2 j + 2) * GOLD), u = v >> 32:
+ *    u < T_mask gives the mask id, else u < T_mask_rand gives repl[((v & 0xFFFFFFFF) * M) >> 32], else the id is kept.  With
+ *    p = mlm_probability, a = mask_replace_prob, b = random_replace_prob (HF's names; 0.15, 0.8, 0.1 are HF's defaults):
+ *    T_sel = floor(p * 2^32), T_mask = floor(a * 2^32), T_mask_rand = floor((a + b) * 2^32), computed in double, so p = 1 selects
+ *    every eligible column and p = 0 none.  repl is the ascending list of the M ids that are in the decoder and not special.
+ * Differences from HF: selection is a Bernoulli draw per group (HF's whole-word collator draws an exact count per row); random
+ * replacements exclude the special ids (HF's randint(len(tokenizer)) includes them); the result is a pure function of (seed,
+ * key, row contents), independent of batch composition, sharding and any other RNG -- dynamic masking takes a new seed per
+ * epoch.  Windows that overlap draw independent decisions for the tokens they share (their rows and keys differ).
+ * Checks: the probabilities finite and in [0, 1], a + b <= 1, n >= 0, width >= 1, non-NULL pointers when n > 0, d_masked_ids
+ * != d_ids, and b > 0 only with M > 0 (GENZTOK_E_INVALID), all before the device slot.  Asynchronous on `stream`, one launch
+ * per call (none when n == 0), bit-identical from run to run.  The first call on a device uploads the continuation bitset
+ * (n_ids / 8 bytes) and repl (4 M bytes). */
+int genztok_mlm_mask_device(genztok_t *h, int dev, const int32_t *d_ids, int64_t n, int32_t width,
+                            const int64_t *d_row_keys /* NULL: row index */, uint64_t seed,
+                            double mlm_probability, double mask_replace_prob, double random_replace_prob,
+                            int whole_word, int32_t *d_masked_ids, int64_t *d_labels, void *stream);
+
 /* ---- measurement plumbing (not part of the reference's surface; used by bench.py and the tests) ------------------- */
 /* The synthetic workload of SURVEY.md 8 d2 produced on the device: the counter-based generator that
  * genz_tokenize_b200/workload.py::generate_hashed defines (same bytes).  genztok_synth_init uploads the word list
