@@ -9,6 +9,7 @@ SO_PATH = os.environ.get("GENZTOK_LIB") or os.path.join(_HERE, "libgenztok.so") 
 
 MAX_LEN_NONE = -(2 ** 31)
 WANT_TOKEN_TYPE, WANT_SEQUENCE_ID, WANT_SPANS, WANT_OFFSETS = 1, 2, 4, 8
+LONGEST_FIRST, ONLY_FIRST, ONLY_SECOND = 16, 32, 64         # pair truncation strategies (at most one)
 NONE, EOS_MARK, PAD_MARK = -1, -3, -4
 
 E_INVALID, E_IO, E_UTF8, E_CUDA, E_NOMEM, E_NODEVICE, E_LIMIT = -1, -2, -3, -4, -5, -6, -7

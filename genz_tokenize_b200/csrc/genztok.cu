@@ -11,6 +11,8 @@
 //   -> k_rows<RAGGED> -> k_post_rows.
 // Long documents as windows (window.cuh): the ragged steps up to k_rows<RAGGED> per side -> k_window_count -> k_scan_i64
 //   -> k_window_rows -> k_post_rows (row list).
+// Pair truncation strategies (window.cuh): the ragged steps up to k_rows<RAGGED> per side -> k_window_rows<KEEP> (k_pair_rows)
+//   -> k_post_rows<KEEP2> (row list).
 // Decode is k_decode_len (lengths, trailing pad runs) -> k_scan_i64 -> k_decode_write.
 // Extractive QA over the windows' offsets (qa.cuh): [k_qa_char_to_byte ->] k_qa_labels; k_qa_spans -> k_qa_spans_docs.
 // MLM inputs and labels from an id plane (mlm.cuh): k_mlm_mask<WHOLE_WORD>.
@@ -816,8 +818,9 @@ WinArgs window_args(DeviceCtx* d, bool pair, int64_t n, int32_t W, int32_t s) {
 
 // Step 1: both token streams, the windows of every document, d_win_off[n+1] and their total (synchronises).  The caller has
 // sized the word cache for the chunk (ensure_cache) and n >= 1.  offs: the streams carry token offsets too (offset_mapping).
-int windows_layout(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& a, const Side* b, int64_t n, int32_t W, int32_t s, bool offs,
-                   int64_t* d_win_off, int64_t* n_win) {
+// strategy (a pair truncation strategy, PAIR_*): the streams only; one row per document, *n_win = n, d_win_off is not used.
+int windows_layout(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& a, const Side* b, int64_t n, int32_t W, int32_t s, int32_t strategy,
+                   bool offs, int64_t* d_win_off, int64_t* n_win) {
     d->win.n_win = -1;                                               // the streams are about to change
     int rc = offs ? ensure_piece_lens(h, d, st) : GENZTOK_OK;
     if (rc) return rc;
@@ -827,6 +830,7 @@ int windows_layout(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& a, c
     if (!rc && b) rc = token_stream(h, d, st, *b, n, d->win.ids[1], d->win.off[1], offs ? &d->win.offs[1] : nullptr);
     if (rc) return rc;
     d->cache_empty = false;
+    if (strategy) { *n_win = n; return GENZTOK_OK; }
     CU(d->win.count.ensure((size_t)n * 8));
     WinArgs A = window_args(d, b != nullptr, n, W, s);
     A.count = d->win.count.as<int64_t>();
@@ -841,14 +845,15 @@ int windows_layout(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& a, c
 
 // Step 2: the K windows' planes and maps from the streams step 1 left (does not synchronise).  win_doc = doc_base + document.
 // With GENZTOK_WANT_OFFSETS in flags, P.offsets receives [K, W, 2] token offsets (step 1 must have run with offsets).
-int windows_write(genztok_t* h, DeviceCtx* d, cudaStream_t st, bool pair, int64_t n, int32_t W, int32_t s, uint32_t flags, const int64_t* d_win_off,
-                  int64_t K, const genztok_dev_planes_t& P, int64_t* win_doc, int32_t* win_start, int64_t doc_base) {
+// strategy: the K = n rows of a pair truncation strategy (k_pair_rows); d_win_off, win_doc and win_start are not used.
+int windows_write(genztok_t* h, DeviceCtx* d, cudaStream_t st, bool pair, int64_t n, int32_t W, int32_t s, int32_t strategy, uint32_t flags,
+                  const int64_t* d_win_off, int64_t K, const genztok_dev_planes_t& P, int64_t* win_doc, int32_t* win_start, int64_t doc_base) {
     if (K <= 0) return GENZTOK_OK;
     if (K >= (1ll << 32)) return fail(h, GENZTOK_E_LIMIT, "%lld windows in one chunk", (long long)K);
     CU(d->win.fix.ensure((size_t)K * 4));
     { LaunchScope ls(h, d, "k_reset_lists"); k_reset_lists<<<1, 1, 0, st>>>(d->C); }
     WinArgs A = window_args(d, pair, n, W, s);
-    A.win_off = d_win_off; A.n_win = K; A.doc_base = doc_base;
+    A.win_off = d_win_off; A.n_win = K; A.doc_base = doc_base; A.strategy = strategy;
     A.ids = P.input_ids; A.mask = P.attention_mask; A.row_len = P.row_len;
     if (pair) {
         A.tt = (flags & GENZTOK_WANT_TOKEN_TYPE) ? P.token_type_ids : nullptr;
@@ -864,8 +869,11 @@ int windows_write(genztok_t* h, DeviceCtx* d, cudaStream_t st, bool pair, int64_
     {
         // algorithmic bytes: the planes and per-window values written (the windows' tokens are read from the streams, mostly in L2)
         const int64_t alg = K * (int64_t)W * (5 + (A.tt ? 1 : 0) + (A.seq ? 1 : 0) + (offs ? 8 : 0)) + K * (4 + 8 + 4 + (pair ? 5 : 0));
-        LaunchScope ls(h, d, offs ? "k_window_rows_offsets" : "k_window_rows", alg);
-        if (offs) {
+        LaunchScope ls(h, d, strategy ? (offs ? "k_pair_rows_offsets" : "k_pair_rows") : offs ? "k_window_rows_offsets" : "k_window_rows", alg);
+        if (strategy) {
+            if (offs) { if (quad) k_window_rows<true, true, true, true><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, true, true, true><<<grid, 256, 0, st>>>(d->T, A); }
+            else { if (quad) k_window_rows<true, true, false, true><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, true, false, true><<<grid, 256, 0, st>>>(d->T, A); }
+        } else if (offs) {
             if (pair) { if (quad) k_window_rows<true, true, true><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, true, true><<<grid, 256, 0, st>>>(d->T, A); }
             else { if (quad) k_window_rows<true, false, true><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, false, true><<<grid, 256, 0, st>>>(d->T, A); }
         } else {
@@ -879,8 +887,9 @@ int windows_write(genztok_t* h, DeviceCtx* d, cudaStream_t st, bool pair, int64_
         Q.ids = P.input_ids; Q.W = W; Q.n_rows = K; Q.row_list = A.fix_list;
         Q.has_pair = 1; Q.tt = A.tt; Q.seq = A.seq; Q.seq_len = A.seq_len; Q.status = A.status;
         Q.has_max_len = 1; Q.max_len = W; Q.padding = 1; Q.truncation = 1; Q.eos_i8 = A.eos_i8; Q.pad_i8 = A.pad_i8;
-        LaunchScope ls(h, d, "k_post_rows_windows");
-        k_post_rows<<<d->sm_count, 256, 0, st>>>(d->T, Q, d->C.ctr + C_FIX);
+        LaunchScope ls(h, d, strategy ? "k_post_rows_pairs" : "k_post_rows_windows");
+        if (strategy) k_post_rows<true><<<d->sm_count, 256, 0, st>>>(d->T, Q, d->C.ctr + C_FIX);
+        else k_post_rows<<<d->sm_count, 256, 0, st>>>(d->T, Q, d->C.ctr + C_FIX);
         CU(cudaGetLastError());
     }
     return GENZTOK_OK;
@@ -982,7 +991,7 @@ void free_result(genztok_t* h, Out* out) {
 // ================================================================================================
 extern "C" {
 
-const char* genztok_version(void) { return "genztok-b200 0.4 (sm_100a)"; }
+const char* genztok_version(void) { return "genztok-b200 0.5 (sm_100a)"; }
 
 const char* genztok_last_error(const genztok_t* h) { return h ? h->err.c_str() : g_create_err.c_str(); }
 
@@ -1206,10 +1215,37 @@ int64_t genztok_profile_report(genztok_t* h, char* buf, int64_t cap, int reset) 
 }
 
 // ---- encode -----------------------------------------------------------------------------------------
+}  // extern "C"
+
+namespace {
+
+// The truncation strategy of flags (PAIR_*, or 0 for the reference cut) into *strategy, after the checks both encode forms share:
+// at most one strategy bit, and the fixed layout (max_len >= 4; the host form also padding and truncation, and no spans).
+int pair_strategy(genztok_t* h, uint32_t flags, int32_t max_len, bool fixed, int32_t* strategy) {
+    const uint32_t bits = flags & (GENZTOK_LONGEST_FIRST | GENZTOK_ONLY_FIRST | GENZTOK_ONLY_SECOND);
+    *strategy = bits == GENZTOK_LONGEST_FIRST ? PAIR_LONGEST_FIRST : bits == GENZTOK_ONLY_FIRST ? PAIR_ONLY_FIRST : bits == GENZTOK_ONLY_SECOND ? PAIR_ONLY_SECOND : 0;
+    if (!bits) return GENZTOK_OK;
+    if (!*strategy) return fail(h, GENZTOK_E_INVALID, "at most one truncation strategy (GENZTOK_LONGEST_FIRST, GENZTOK_ONLY_FIRST, GENZTOK_ONLY_SECOND)");
+    if (max_len < 4) return fail(h, GENZTOK_E_INVALID, "a truncation strategy needs max_len >= 4 (got %s)", max_len == GENZTOK_MAX_LEN_NONE ? "None" : std::to_string(max_len).c_str());
+    if (!fixed) return fail(h, GENZTOK_E_INVALID, "a truncation strategy needs the fixed layout: padding and truncation, without return_offset spans");
+    return GENZTOK_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
 int genztok_encode_device(genztok_t* h, int dev, const uint8_t* d_text, const int64_t* d_text_off, int64_t text_bytes, const uint8_t* d_pair,
                           const int64_t* d_pair_off, int64_t pair_bytes, int64_t n, int32_t max_len, uint32_t flags,
                           const genztok_dev_planes_t* planes, void* stream) {
     if (!h) return GENZTOK_E_INVALID;
+    int32_t strategy = 0;
+    int rc = pair_strategy(h, flags, max_len, true, &strategy);
+    if (rc) return rc;
+    if (strategy && (flags & (GENZTOK_WANT_OFFSETS | GENZTOK_WANT_SPANS)))
+        return fail(h, GENZTOK_E_INVALID, "genztok_encode_device: offsets and spans are not available with a truncation strategy");
+    if (strategy && (!planes || !planes->input_ids || !planes->attention_mask || !planes->row_len))
+        return fail(h, GENZTOK_E_INVALID, "genztok_encode_device: a truncation strategy needs input_ids, attention_mask and row_len");
     if (flags & GENZTOK_WANT_OFFSETS) return fail(h, GENZTOK_E_INVALID, "offsets are not available in the fixed device layout; use genztok_encode_windows_device");
     if (dev < 0 || dev >= (int)h->devs.size()) return fail(h, GENZTOK_E_NODEVICE, "no such device slot %d (handle has %d)", dev, (int)h->devs.size());
     if (!planes || !planes->input_ids || n < 0 || !d_text_off || (text_bytes > 0 && !d_text)) return fail(h, GENZTOK_E_INVALID, "genztok_encode_device: bad arguments");
@@ -1219,9 +1255,25 @@ int genztok_encode_device(genztok_t* h, int dev, const uint8_t* d_text, const in
     std::lock_guard<std::mutex> lk(h->mu);
     DeviceCtx* d = h->devs[(size_t)dev];
     CU(cudaSetDevice(d->device));
-    if (!fixed_fits(d, max_len)) return fail(h, GENZTOK_E_LIMIT, "max_len=%d does not fit the fixed-layout kernel; use genztok_encode", max_len);
     Side a{d_text, d_text_off, text_bytes}, b{d_pair, d_pair_off, pair_bytes};
     cudaStream_t st = stream ? (cudaStream_t)stream : d->stream;
+    if (strategy && d_pair_off) {
+        // the rows of a truncation strategy: both token streams (sized by a read-back: synchronises), then one k_pair_rows launch
+        LaunchScope::cur_stream = st;
+        const int64_t bytes = text_bytes + pair_bytes;
+        if (bytes > h->max_chunk_bytes) return fail(h, GENZTOK_E_LIMIT, "chunk of %lld bytes exceeds max_chunk_bytes=%lld", (long long)bytes, (long long)h->max_chunk_bytes);
+        rc = stream_enter(h, d, st);
+        if (rc) return rc;
+        if (n > 0) {
+            int64_t K = 0;
+            rc = ensure_cache(h, d, st, bytes + 32);
+            if (!rc) rc = windows_layout(h, d, st, a, &b, n, max_len, 0, strategy, false, nullptr, &K);
+            if (!rc) rc = windows_write(h, d, st, true, n, max_len, 0, strategy, flags, nullptr, K, *planes, nullptr, nullptr, 0);
+            if (rc) return rc;
+        }
+        return stream_leave(h, d, st);
+    }
+    if (!fixed_fits(d, max_len)) return fail(h, GENZTOK_E_LIMIT, "max_len=%d does not fit the fixed-layout kernel; use genztok_encode", max_len);
     return encode_fixed_on_device(h, d, st, a, d_pair_off ? &b : nullptr, n, max_len, flags, *planes);
 }
 
@@ -1239,6 +1291,7 @@ struct EncodeJob {
     int32_t max_len; int padding, truncation; uint32_t flags;
     bool has_pair, has_max_len, want_spans, fixed, want_tt, want_seq;
     bool want_offs;                // offset_mapping: the ragged pipeline writes token offsets beside the ids
+    int32_t strategy;              // pairs: a truncation strategy (PAIR_*, window.cuh) or 0; its rows are written by windows_chunks
     genztok_encoded_t* out;
     int32_t old_dirty[4];          // fixed layout: columns of the result planes (ids, mask, token types, sequence ids) that may hold something
                                    // other than padding from the buffer's last use (the width: unknown / a fresh buffer)
@@ -1597,6 +1650,93 @@ void encode_ragged_chunks(genztok_t* h, DeviceCtx* d, const EncodeJob& J, const 
     }
 }
 
+// What one device collects for its documents [rb, re) of genztok_encode_windows (chunk after chunk, in document order).
+struct WindowPart {
+    PartStatus status;
+    int64_t n_win = 0, tokens = 0, d2h_bytes = 0;
+    PinnedVec<int32_t> ids, row_len, seq_len, start, tok_offs; PinnedVec<uint8_t> mask, row_status; PinnedVec<int8_t> tt, seq; PinnedVec<int64_t> doc, offs;
+    void bind(genztok_t* h) { for (auto* v : {&ids, &row_len, &seq_len, &start, &tok_offs}) v->h = h; mask.h = h; row_status.h = h; tt.h = h; seq.h = h; doc.h = h; offs.h = h; }
+};
+
+// Windows of one device's chunks: per chunk the text goes up, both steps run, the planes and maps come home.
+// win_off[r] for r in (rb, re] is written relative to the part's first window.
+// With J.strategy the chunk's rows (one per document) go straight into the fixed-layout planes of J.out at their rows, and win_off
+// is not used.
+void windows_chunks(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int32_t stride, int64_t* win_off, const std::vector<int64_t>& cuts, WindowPart* part) {
+    cudaStream_t st = d->stream;
+    const bool has_pair = J.has_pair, rows = J.strategy != 0;
+    const int32_t W = J.max_len;
+    const int64_t rb = cuts.front(), re = cuts.back();
+    for (size_t ci = 0; ci + 1 < cuts.size(); ci++) {
+        const int64_t r0 = cuts[ci], r1 = cuts[ci + 1], m = r1 - r0;
+        const int64_t tb = J.text_off[r1] - J.text_off[r0], pb = has_pair ? J.pair_off[r1] - J.pair_off[r0] : 0;
+        CUF(d->text.ensure((size_t)tb + 96)); CUF(d->toff.ensure((size_t)(m + 1) * 8));
+        if (has_pair) { CUF(d->pair.ensure((size_t)pb + 96)); CUF(d->poff.ensure((size_t)(m + 1) * 8)); }
+        Side a, b;
+        CUF(upload_chunk(J, r0, r1, d->text, d->toff, d->pair, d->poff, st, &a, &b));
+        CUF(d->win.woff.ensure((size_t)(m + 1) * 8));
+        int64_t K = 0;
+        FAIL_RC(windows_layout(h, d, st, a, has_pair ? &b : nullptr, m, W, stride, J.strategy, J.want_offs, d->win.woff.as<int64_t>(), &K));
+        const size_t tot = (size_t)K * (size_t)W;
+        CUF(d->ids.ensure(tot * 4 + 16)); CUF(d->mask.ensure(tot + 16)); CUF(d->row_len.ensure((size_t)K * 4 + 16));
+        CUF(d->win.doc.ensure((size_t)K * 8 + 16)); CUF(d->win.start.ensure((size_t)K * 4 + 16));
+        genztok_dev_planes_t P{};
+        P.input_ids = d->ids.as<int32_t>(); P.attention_mask = d->mask.as<uint8_t>(); P.row_len = d->row_len.as<int32_t>();
+        if (J.want_tt) { CUF(d->tt.ensure(tot + 16)); P.token_type_ids = d->tt.as<int8_t>(); }
+        if (J.want_seq) { CUF(d->seq.ensure(tot + 16)); P.sequence_id = d->seq.as<int8_t>(); }
+        if (has_pair) { CUF(d->seq_len.ensure((size_t)K * 4 + 16)); CUF(d->status.ensure((size_t)K + 16)); P.seq_len = d->seq_len.as<int32_t>(); P.row_status = d->status.as<uint8_t>(); }
+        if (J.want_offs) { CUF(d->win.plane_offs.ensure(tot * 8 + 16)); P.offsets = d->win.plane_offs.as<int32_t>(); }
+        FAIL_RC(windows_write(h, d, st, has_pair, m, W, stride, J.strategy, J.flags, d->win.woff.as<int64_t>(), K, P, d->win.doc.as<int64_t>(), d->win.start.as<int32_t>(), r0));
+        // where the chunk's rows go on the host: the result planes at rows r0.. (strategy), else the part's arrays behind its windows so far
+        genztok_dev_planes_t H{};
+        size_t o = (size_t)r0;
+        if (rows) {
+            const genztok_encoded_t* out = J.out;
+            H.input_ids = out->input_ids; H.attention_mask = out->attention_mask; H.token_type_ids = out->token_type_ids; H.sequence_id = out->sequence_id;
+            H.row_len = out->row_len; H.seq_len = out->seq_len; H.row_status = out->row_status; H.offsets = out->offsets;
+        } else {
+            o = (size_t)part->n_win;
+            const size_t n1 = o + (size_t)K;
+            // first chunk of several: room for the part at this chunk's windows per document (+ 12 %)
+            const size_t est = (ci == 0 && r1 < re) ? (size_t)((double)K * (double)(re - rb) / (double)m * 1.125) + 64 : 0;
+            bool grown = grow(part->ids, n1 * W, est * W) && grow(part->mask, n1 * W, est * W) && grow(part->row_len, n1, est) && grow(part->doc, n1, est) &&
+                         grow(part->start, n1, est) && part->offs.resize((size_t)m + 1);
+            if (J.want_tt) grown = grown && grow(part->tt, n1 * W, est * W);
+            if (J.want_seq) grown = grown && grow(part->seq, n1 * W, est * W);
+            if (J.want_offs) grown = grown && grow(part->tok_offs, 2 * n1 * W, 2 * est * W);
+            if (has_pair) grown = grown && grow(part->seq_len, n1, est) && grow(part->row_status, n1, est);
+            if (!grown) PFAIL(GENZTOK_E_NOMEM, "pinned host allocation failed")
+            H.input_ids = part->ids.data(); H.attention_mask = part->mask.data(); H.token_type_ids = part->tt.data(); H.sequence_id = part->seq.data();
+            H.row_len = part->row_len.data(); H.seq_len = part->seq_len.data(); H.row_status = part->row_status.data(); H.offsets = part->tok_offs.data();
+        }
+        if (K) {
+            CUF(cudaMemcpyAsync(H.input_ids + o * W, P.input_ids, tot * 4, cudaMemcpyDeviceToHost, st));
+            CUF(cudaMemcpyAsync(H.attention_mask + o * W, P.attention_mask, tot, cudaMemcpyDeviceToHost, st));
+            if (J.want_tt) CUF(cudaMemcpyAsync(H.token_type_ids + o * W, P.token_type_ids, tot, cudaMemcpyDeviceToHost, st));
+            if (J.want_seq) CUF(cudaMemcpyAsync(H.sequence_id + o * W, P.sequence_id, tot, cudaMemcpyDeviceToHost, st));
+            if (J.want_offs) CUF(cudaMemcpyAsync(H.offsets + 2 * o * W, P.offsets, tot * 8, cudaMemcpyDeviceToHost, st));
+            CUF(cudaMemcpyAsync(H.row_len + o, P.row_len, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
+            if (!rows) {
+                CUF(cudaMemcpyAsync(part->doc.data() + o, d->win.doc.p, (size_t)K * 8, cudaMemcpyDeviceToHost, st));
+                CUF(cudaMemcpyAsync(part->start.data() + o, d->win.start.p, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
+            }
+            if (has_pair) {
+                CUF(cudaMemcpyAsync(H.seq_len + o, P.seq_len, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
+                CUF(cudaMemcpyAsync(H.row_status + o, P.row_status, (size_t)K, cudaMemcpyDeviceToHost, st));
+            }
+        }
+        if (!rows) CUF(cudaMemcpyAsync(part->offs.data(), d->win.woff.p, (size_t)(m + 1) * 8, cudaMemcpyDeviceToHost, st));
+        CUF(cudaStreamSynchronize(st));
+        part->d2h_bytes += (int64_t)tot * (5 + (J.want_tt ? 1 : 0) + (J.want_seq ? 1 : 0) + (J.want_offs ? 8 : 0)) + K * (4 + (has_pair ? 5 : 0)) +
+                           (rows ? 0 : K * 12 + (m + 1) * 8);
+        if (!rows) {
+            const int64_t* offs = part->offs.data();
+            for (int64_t i = 1; i <= m; i++) win_off[r0 + i] = part->n_win + offs[i];
+        }
+        part->n_win += K;
+    }
+}
+
 }  // namespace
 
 extern "C" {
@@ -1605,6 +1745,8 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
                    int32_t max_len, int padding, int truncation, uint32_t flags, genztok_encoded_t* out) {
     if (!h) return GENZTOK_E_INVALID;
     if (!out || n < 0 || !text_off) return fail(h, GENZTOK_E_INVALID, "genztok_encode: bad arguments");
+    int32_t strategy = 0;
+    { const int rc = pair_strategy(h, flags, max_len, padding && truncation && !(flags & GENZTOK_WANT_SPANS), &strategy); if (rc) return rc; }
     if (h->devs.empty()) return fail(h, GENZTOK_E_NODEVICE, "this handle was created without a CUDA device; there is no CPU path");
     memset(out, 0, sizeof *out);
     std::lock_guard<std::mutex> lk(h->mu);
@@ -1612,10 +1754,11 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
     J.padding = padding; J.truncation = truncation; J.out = out;
     J.has_max_len = max_len != GENZTOK_MAX_LEN_NONE;
     J.want_spans = (flags & GENZTOK_WANT_SPANS) != 0;       // return_offset: produced by the ragged pipeline
+    J.strategy = J.has_pair ? strategy : 0;                 // (without second texts every strategy is the reference cut)
     // the fixed regime; with offsets (offset_mapping) it is computed by the ragged pipeline, whose rows then all hold max_len
-    // entries, and presented in the fixed layout
-    const bool fixed_layout = J.has_max_len && max_len >= 1 && padding && truncation && fixed_fits(h->devs[0], max_len) && !J.want_spans;
-    J.fixed = fixed_layout && !J.want_offs;
+    // entries, and presented in the fixed layout; the rows of a truncation strategy are written by windows_chunks
+    const bool fixed_layout = J.has_max_len && max_len >= 1 && padding && truncation && (J.strategy || fixed_fits(h->devs[0], max_len)) && !J.want_spans;
+    J.fixed = fixed_layout && !J.want_offs && !J.strategy;
     const bool has_pair = J.has_pair, fixed = J.fixed;
     OutBlock* ob = new OutBlock();
     out->_owner = ob;
@@ -1634,7 +1777,7 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
     };
 #define OOM_CHECK(p) if (!(p)) { free_nolock(); return fail(h, GENZTOK_E_NOMEM, "pinned host allocation failed"); }
     if (J.want_spans) { out->span_off = out_alloc<int64_t>(h, ob, (size_t)n + 1); OOM_CHECK(out->span_off); out->span_off[0] = 0; }
-    if (fixed) {
+    if (fixed || J.strategy) {
         const size_t tot = (size_t)n * (size_t)max_len;
         out->width = max_len; out->total = (int64_t)tot;
         out->input_ids = out_alloc<int32_t>(h, ob, tot); OOM_CHECK(out->input_ids);
@@ -1643,6 +1786,10 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
         if (J.want_tt) { out->token_type_ids = out_alloc<int8_t>(h, ob, tot); OOM_CHECK(out->token_type_ids); out->tt_len = out_alloc<int32_t>(h, ob, (size_t)n); OOM_CHECK(out->tt_len); }
         if (J.want_seq) { out->sequence_id = out_alloc<int8_t>(h, ob, tot); OOM_CHECK(out->sequence_id); }
         if (has_pair) { out->seq_len = out_alloc<int32_t>(h, ob, (size_t)n); OOM_CHECK(out->seq_len); out->row_status = out_alloc<uint8_t>(h, ob, (size_t)n); OOM_CHECK(out->row_status); }
+        if (J.strategy) {
+            if (J.want_offs) { out->offsets = out_alloc<int32_t>(h, ob, 2 * tot); OOM_CHECK(out->offsets); }
+            for (auto& pr : ob->pinned) h->plane_meta.erase(pr.first);   // (these planes are written whole; no record describes them)
+        }
     } else {
         out->width = 0;
         out->row_off = out_alloc<int64_t>(h, ob, (size_t)n + 1); OOM_CHECK(out->row_off);
@@ -1668,6 +1815,15 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
     // every device writes its own rows of the result; the documents are balanced by bytes
     const int G = (int)h->devs.size();
     const std::vector<int64_t> dcut = shard_rows(G, n, [&](int64_t r) { return text_off[r] + (has_pair ? pair_off[r] : 0) + 64 * r; });
+    if (J.strategy) {
+        std::vector<WindowPart> parts((size_t)G);
+        run_parts(h, J, dcut, parts, [&](DeviceCtx* d, const std::vector<int64_t>& cuts, WindowPart* pt) { windows_chunks(h, d, J, 0, nullptr, cuts, pt); });
+        for (auto& pt : parts)
+            if (pt.status.rc) { free_nolock(); return pt.status.report(h); }
+        for (auto& pt : parts) { out->real_tokens += pt.tokens; out->d2h_bytes += pt.d2h_bytes; }
+        if (J.want_tt) for (int64_t r = 0; r < n; r++) out->tt_len[r] = max_len;
+        return GENZTOK_OK;
+    }
     std::vector<EncodePart> parts((size_t)G);
     run_parts(h, J, dcut, parts, [&](DeviceCtx* d, const std::vector<int64_t>& cuts, EncodePart* pt) {
         if (fixed) encode_fixed_chunks(h, d, J, cuts, pt); else encode_ragged_chunks(h, d, J, cuts, pt);
@@ -1741,74 +1897,6 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
 }  // extern "C"
 
 namespace {
-
-// What one device collects for its documents [rb, re) of genztok_encode_windows (chunk after chunk, in document order).
-struct WindowPart {
-    PartStatus status;
-    int64_t n_win = 0, tokens = 0, d2h_bytes = 0;
-    PinnedVec<int32_t> ids, row_len, seq_len, start, tok_offs; PinnedVec<uint8_t> mask, row_status; PinnedVec<int8_t> tt, seq; PinnedVec<int64_t> doc, offs;
-    void bind(genztok_t* h) { for (auto* v : {&ids, &row_len, &seq_len, &start, &tok_offs}) v->h = h; mask.h = h; row_status.h = h; tt.h = h; seq.h = h; doc.h = h; offs.h = h; }
-};
-
-// Windows of one device's chunks: per chunk the text goes up, both steps run, the planes and maps come home.
-// win_off[r] for r in (rb, re] is written relative to the part's first window.
-void windows_chunks(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int32_t stride, int64_t* win_off, const std::vector<int64_t>& cuts, WindowPart* part) {
-    cudaStream_t st = d->stream;
-    const bool has_pair = J.has_pair;
-    const int32_t W = J.max_len;
-    const int64_t rb = cuts.front(), re = cuts.back();
-    for (size_t ci = 0; ci + 1 < cuts.size(); ci++) {
-        const int64_t r0 = cuts[ci], r1 = cuts[ci + 1], m = r1 - r0;
-        const int64_t tb = J.text_off[r1] - J.text_off[r0], pb = has_pair ? J.pair_off[r1] - J.pair_off[r0] : 0;
-        CUF(d->text.ensure((size_t)tb + 96)); CUF(d->toff.ensure((size_t)(m + 1) * 8));
-        if (has_pair) { CUF(d->pair.ensure((size_t)pb + 96)); CUF(d->poff.ensure((size_t)(m + 1) * 8)); }
-        Side a, b;
-        CUF(upload_chunk(J, r0, r1, d->text, d->toff, d->pair, d->poff, st, &a, &b));
-        CUF(d->win.woff.ensure((size_t)(m + 1) * 8));
-        int64_t K = 0;
-        FAIL_RC(windows_layout(h, d, st, a, has_pair ? &b : nullptr, m, W, stride, J.want_offs, d->win.woff.as<int64_t>(), &K));
-        const size_t tot = (size_t)K * (size_t)W;
-        CUF(d->ids.ensure(tot * 4 + 16)); CUF(d->mask.ensure(tot + 16)); CUF(d->row_len.ensure((size_t)K * 4 + 16));
-        CUF(d->win.doc.ensure((size_t)K * 8 + 16)); CUF(d->win.start.ensure((size_t)K * 4 + 16));
-        genztok_dev_planes_t P{};
-        P.input_ids = d->ids.as<int32_t>(); P.attention_mask = d->mask.as<uint8_t>(); P.row_len = d->row_len.as<int32_t>();
-        if (J.want_tt) { CUF(d->tt.ensure(tot + 16)); P.token_type_ids = d->tt.as<int8_t>(); }
-        if (J.want_seq) { CUF(d->seq.ensure(tot + 16)); P.sequence_id = d->seq.as<int8_t>(); }
-        if (has_pair) { CUF(d->seq_len.ensure((size_t)K * 4 + 16)); CUF(d->status.ensure((size_t)K + 16)); P.seq_len = d->seq_len.as<int32_t>(); P.row_status = d->status.as<uint8_t>(); }
-        if (J.want_offs) { CUF(d->win.plane_offs.ensure(tot * 8 + 16)); P.offsets = d->win.plane_offs.as<int32_t>(); }
-        FAIL_RC(windows_write(h, d, st, has_pair, m, W, stride, J.flags, d->win.woff.as<int64_t>(), K, P, d->win.doc.as<int64_t>(), d->win.start.as<int32_t>(), r0));
-        const size_t o = (size_t)part->n_win, n1 = o + (size_t)K;
-        // first chunk of several: room for the part at this chunk's windows per document (+ 12 %)
-        const size_t est = (ci == 0 && r1 < re) ? (size_t)((double)K * (double)(re - rb) / (double)m * 1.125) + 64 : 0;
-        bool grown = grow(part->ids, n1 * W, est * W) && grow(part->mask, n1 * W, est * W) && grow(part->row_len, n1, est) && grow(part->doc, n1, est) &&
-                     grow(part->start, n1, est) && part->offs.resize((size_t)m + 1);
-        if (J.want_tt) grown = grown && grow(part->tt, n1 * W, est * W);
-        if (J.want_seq) grown = grown && grow(part->seq, n1 * W, est * W);
-        if (J.want_offs) grown = grown && grow(part->tok_offs, 2 * n1 * W, 2 * est * W);
-        if (has_pair) grown = grown && grow(part->seq_len, n1, est) && grow(part->row_status, n1, est);
-        if (!grown) PFAIL(GENZTOK_E_NOMEM, "pinned host allocation failed")
-        if (K) {
-            CUF(cudaMemcpyAsync(part->ids.data() + o * W, P.input_ids, tot * 4, cudaMemcpyDeviceToHost, st));
-            CUF(cudaMemcpyAsync(part->mask.data() + o * W, P.attention_mask, tot, cudaMemcpyDeviceToHost, st));
-            if (J.want_tt) CUF(cudaMemcpyAsync(part->tt.data() + o * W, P.token_type_ids, tot, cudaMemcpyDeviceToHost, st));
-            if (J.want_seq) CUF(cudaMemcpyAsync(part->seq.data() + o * W, P.sequence_id, tot, cudaMemcpyDeviceToHost, st));
-            if (J.want_offs) CUF(cudaMemcpyAsync(part->tok_offs.data() + 2 * o * W, P.offsets, tot * 8, cudaMemcpyDeviceToHost, st));
-            CUF(cudaMemcpyAsync(part->row_len.data() + o, P.row_len, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
-            CUF(cudaMemcpyAsync(part->doc.data() + o, d->win.doc.p, (size_t)K * 8, cudaMemcpyDeviceToHost, st));
-            CUF(cudaMemcpyAsync(part->start.data() + o, d->win.start.p, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
-            if (has_pair) {
-                CUF(cudaMemcpyAsync(part->seq_len.data() + o, P.seq_len, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
-                CUF(cudaMemcpyAsync(part->row_status.data() + o, P.row_status, (size_t)K, cudaMemcpyDeviceToHost, st));
-            }
-        }
-        CUF(cudaMemcpyAsync(part->offs.data(), d->win.woff.p, (size_t)(m + 1) * 8, cudaMemcpyDeviceToHost, st));
-        CUF(cudaStreamSynchronize(st));
-        part->d2h_bytes += (int64_t)tot * (5 + (J.want_tt ? 1 : 0) + (J.want_seq ? 1 : 0) + (J.want_offs ? 8 : 0)) + K * (16 + (has_pair ? 5 : 0)) + (m + 1) * 8;
-        const int64_t* offs = part->offs.data();
-        for (int64_t i = 1; i <= m; i++) win_off[r0 + i] = part->n_win + offs[i];
-        part->n_win += K;
-    }
-}
 
 int check_window_args(genztok_t* h, int32_t max_len, int32_t stride, uint32_t flags) {
     if (max_len < 3) return fail(h, GENZTOK_E_INVALID, "windows need max_len >= 3 (got %d)", max_len);
@@ -1928,7 +2016,7 @@ int genztok_encode_windows_device(genztok_t* h, int dev, const uint8_t* d_text, 
             rc = ensure_cache(h, d, st, bytes + 32);
             if (rc) return rc;
             Side a{d_text, d_text_off, text_bytes}, b{d_pair, d_pair_off, pair_bytes};
-            rc = windows_layout(h, d, st, a, has_pair ? &b : nullptr, n, max_len, stride, offs, d_win_off, &K);
+            rc = windows_layout(h, d, st, a, has_pair ? &b : nullptr, n, max_len, stride, 0, offs, d_win_off, &K);
             if (rc) return rc;
         }
         S.n_win = K;
@@ -1940,7 +2028,7 @@ int genztok_encode_windows_device(genztok_t* h, int dev, const uint8_t* d_text, 
         if (S.n_win > 0 && (!planes->input_ids || !planes->attention_mask || !planes->row_len || !d_win_doc || !d_win_start))
             return fail(h, GENZTOK_E_INVALID, "genztok_encode_windows_device: step 2 needs input_ids, attention_mask, row_len and the two maps");
         if (S.n_win > 0 && offs && !planes->offsets) return fail(h, GENZTOK_E_INVALID, "genztok_encode_windows_device: GENZTOK_WANT_OFFSETS needs planes->offsets");
-        rc = windows_write(h, d, st, has_pair, n, max_len, stride, flags, d_win_off, S.n_win, *planes, d_win_doc, d_win_start, 0);
+        rc = windows_write(h, d, st, has_pair, n, max_len, stride, 0, flags, d_win_off, S.n_win, *planes, d_win_doc, d_win_start, 0);
         if (rc) return rc;
     }
     return stream_leave(h, d, st);

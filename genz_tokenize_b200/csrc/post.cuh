@@ -119,6 +119,9 @@ struct PostArgs {
     unsigned long long* tokens_ctr;   // += sum(mask)
 };
 
+// KEEP2: a row whose status is already 2 (a pair truncation strategy that could not apply, written by k_window_rows<..., KEEP>)
+// keeps it.
+template <bool KEEP2 = false>
 __global__ void __launch_bounds__(256) k_post_rows(DevTables T, PostArgs A, const unsigned long long* list_count) {
     const int lane = threadIdx.x & 31;
     const uint64_t warp = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
@@ -202,7 +205,7 @@ __global__ void __launch_bounds__(256) k_post_rows(DevTables T, PostArgs A, cons
         if (lane == 0) {
             if (A.seq_len) A.seq_len[r] = m_len;
             if (A.tt_len) A.tt_len[r] = tt_len;
-            if (A.status) A.status[r] = err ? 1 : 0;
+            if (A.status) A.status[r] = (KEEP2 && A.status[r] == 2) ? 2 : err ? 1 : 0;
         }
     }
     if (A.tokens_ctr && lane == 0 && tok_total) atomicAdd(A.tokens_ctr, tok_total);

@@ -9,6 +9,10 @@
 // Window k of a single holds [bos] + T[k(C-s) : k(C-s)+C] + [eos] with C = W - 2.  A pair keeps its first text whole:
 // [bos] + A + [eos, eos] + B_k + [eos] with C = W - len(A) - 4; when C - s < 1 the document has one window, its truncated
 // pair row.  Every window is then padded to W as tokenize.py:141-182,247-258 pad a row (window 0 is the encode_batch row).
+//
+// Pair truncation strategies (k_window_rows<..., KEEP>, launched as k_pair_rows): one row per document from the same streams,
+// [bos] + A[:la'] + [eos, eos] + B[:lb'] + [eos] with (la', lb') = pair_keep(la, lb, W - 4, strategy), padded the same way.  A row
+// whose strategy cannot apply (row_status 2) is the whole pair row, truncated like encode_batch's.
 #pragma once
 #include "device_common.cuh"
 #include "encode.cuh"
@@ -34,7 +38,23 @@ struct WinArgs {
     // [n_win, W, 2] plane they are cut into
     const int2* offs_a; const int2* offs_b;
     int32_t* offs;
+    int32_t strategy;                             // k_window_rows<..., KEEP>: PAIR_LONGEST_FIRST / PAIR_ONLY_FIRST / PAIR_ONLY_SECOND
 };
+
+enum { PAIR_LONGEST_FIRST = 1, PAIR_ONLY_FIRST = 2, PAIR_ONLY_SECOND = 3 };
+
+// Tokens kept of each text of a pair by a truncation strategy (include/genztok.h states the rule): la, lb untruncated token counts,
+// C = max_len - 4.  x = la', y = lb'; z = 1 when only_first / only_second cannot remove enough (HF's SequenceTooShort: row_status 2,
+// x, y = la, lb).  Rows that fit keep everything under every strategy.  longest_first is the Rust tokenizers' LongestFirst: the
+// shorter text (the first on a tie) stays whole when it is at most floor(C/2), else the two keep floor(C/2) (shorter) and ceil(C/2).
+__host__ __device__ __forceinline__ int3 pair_keep(int32_t la, int32_t lb, int32_t C, int32_t strategy) {
+    if (la + lb <= C) return make_int3(la, lb, 0);
+    if (strategy == PAIR_ONLY_SECOND) return la < C ? make_int3(la, C - la, 0) : make_int3(la, lb, 1);
+    if (strategy == PAIR_ONLY_FIRST) return lb < C ? make_int3(C - lb, lb, 0) : make_int3(la, lb, 1);
+    const int32_t s = min(la, lb), h = C / 2;
+    const int32_t ks = s <= h ? s : h, kl = C - ks;
+    return la <= lb ? make_int3(ks, kl, 0) : make_int3(kl, ks, 0);
+}
 
 // Windows of one document.  L: tokens of the windowed text, LA: tokens of the first text (pairs).
 __host__ __device__ __forceinline__ int64_t window_count(int64_t L, int64_t LA, bool pair, int32_t W, int32_t s) {
@@ -57,26 +77,31 @@ __global__ void __launch_bounds__(256) k_window_count(WinArgs A) {
 // 16-byte store of ids and one 4-byte store per byte plane; the pad run needs no loads.  Otherwise a lane owns one column.
 // OFFS: the offsets plane too, taken from the streams where the ids are (first text, windowed slice) and (0, 0) elsewhere;
 // QUAD writes a lane's 4 columns (32 bytes) with two 16-byte stores.
-template <bool QUAD, bool PAIR, bool OFFS = false>
+// KEEP (pairs): row r is document r cut by pair_keep (win_off, stride, win_doc and win_start are not used); a row_status 2 row is
+// the `whole` row.
+template <bool QUAD, bool PAIR, bool OFFS = false, bool KEEP = false>
 __global__ void __launch_bounds__(256) k_window_rows(DevTables T, WinArgs A) {
+    static_assert(PAIR || !KEEP, "truncation strategies are for pairs");
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     const int32_t W = A.W;
     uint32_t tok_total = 0;
     for (int64_t r = warp; r < A.n_win; r += nwarps) {
-        int64_t lo = 0, hi = A.n_docs - 1;                            // the document: last d with win_off[d] <= r
-        while (lo < hi) { const int64_t mid = (lo + hi + 1) >> 1; if (A.win_off[mid] <= r) lo = mid; else hi = mid - 1; }
-        const int64_t d = lo, k = r - A.win_off[d];
+        int64_t lo = KEEP ? r : 0, hi = A.n_docs - 1;                // the document: last d with win_off[d] <= r
+        if (!KEEP) while (lo < hi) { const int64_t mid = (lo + hi + 1) >> 1; if (A.win_off[mid] <= r) lo = mid; else hi = mid - 1; }
+        const int64_t d = lo, k = KEEP ? 0 : r - A.win_off[d];
         const int64_t oa = A.off_a[d];
-        const int32_t LA = (int32_t)(A.off_a[d + 1] - oa - 2);
+        const int32_t LA0 = (int32_t)(A.off_a[d + 1] - oa - 2);
         const int64_t ox = PAIR ? A.off_b[d] : oa;
-        const int32_t L = PAIR ? (int32_t)(A.off_b[d + 1] - ox - 2) : LA;
+        const int32_t L = PAIR ? (int32_t)(A.off_b[d + 1] - ox - 2) : LA0;
+        const int3 keep = KEEP ? pair_keep(LA0, L, W - 4, A.strategy) : make_int3(LA0, L, 0);
+        const int32_t LA = keep.x;                                    // tokens of the first text in the row
         const int32_t C = PAIR ? W - LA - 4 : W - 2;
-        const bool whole = PAIR && C - A.stride < 1;                  // one window: the pair row, truncated like encode_batch's
+        const bool whole = KEEP ? keep.z != 0 : PAIR && C - A.stride < 1;   // one window: the pair row, truncated like encode_batch's
         const int64_t st64 = whole ? 0 : k * (int64_t)(C - A.stride);
         const int32_t st = (int32_t)st64;
-        const int32_t len = whole ? L : min(C, L - st);
-        if (LA < 0 || L < 0 || k < 0 || k >= window_count(L, LA, PAIR, W, A.stride) || len < 0) {   // win_off does not fit the streams
+        const int32_t len = whole ? L : KEEP ? keep.y : min(C, L - st);
+        if (LA0 < 0 || L < 0 || k < 0 || (!KEEP && k >= window_count(L, LA, PAIR, W, A.stride)) || len < 0) {   // win_off does not fit the streams
             if (lane == 0) atomicAdd(&A.ctr[C_ERR], 1ULL);
             continue;
         }
@@ -155,11 +180,13 @@ __global__ void __launch_bounds__(256) k_window_rows(DevTables T, WinArgs A) {
         special = __any_sync(FULL_MASK, special);
         if (lane == 0) {
             A.row_len[r] = Lr;
-            A.win_doc[r] = A.doc_base + d;
-            A.win_start[r] = st;
+            if (!KEEP) {
+                A.win_doc[r] = A.doc_base + d;
+                A.win_start[r] = st;
+            }
             if (PAIR) {
                 if (A.seq_len) A.seq_len[r] = sd.m;
-                if (A.status) A.status[r] = (uint8_t)sd.err;
+                if (A.status) A.status[r] = (uint8_t)(KEEP && whole ? 2 : sd.err);
                 if (special || !T.specials_distinct) { const unsigned long long j = atomicAdd(&A.ctr[C_FIX], 1ULL); A.fix_list[j] = (uint32_t)r; }
             }
         }

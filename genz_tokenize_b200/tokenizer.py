@@ -9,6 +9,7 @@ Extensions over the reference (which is one string per call): `encode_batch` / `
 `encode_windows_device` (long documents as overlapping max_len windows, every token kept).  Every encode
 form but encode_device can also return `offset_mapping` (HF's return_offsets_mapping): each token's
 (start, end) byte range in its own document's UTF-8 text, (0, 0) for tokens that are not from the text.
+`truncation=` also takes HF's pair strategies "longest_first", "only_first" and "only_second" (fixed layout).
 `qa_labels` / `qa_best_spans` turn those planes into extractive-QA training labels and read a QA model's
 start / end logits back into answer spans, on the GPU.  `mlm_mask` turns any fixed-layout id plane into masked-language-model
 inputs and labels (token or whole-word masking), on the GPU.
@@ -25,6 +26,25 @@ from .data import bundled_paths
 
 class GenztokError(RuntimeError):
     pass
+
+
+# truncation= names of the pair truncation strategies (include/genztok.h states the rule)
+_STRATEGIES = {"longest_first": L.LONGEST_FIRST, "only_first": L.ONLY_FIRST, "only_second": L.ONLY_SECOND}
+
+
+def _strategy_flag(truncation, max_len, padding=True, return_offset=False):
+    """The flag of a strategy name, after the checks of the fixed layout it needs; 0 for anything that is not a str."""
+    if not isinstance(truncation, str):
+        return 0
+    if truncation not in _STRATEGIES:
+        raise ValueError("truncation must be True, False or one of %s (got %r)" % (", ".join(map(repr, _STRATEGIES)), truncation))
+    if max_len is None or max_len < 4:
+        raise ValueError("truncation=%r needs max_len >= 4 (got %r)" % (truncation, max_len))
+    if not padding:
+        raise ValueError("truncation=%r needs padding=True (the fixed layout)" % truncation)
+    if return_offset:
+        raise ValueError("truncation=%r is not available with return_offset=True" % truncation)
+    return _STRATEGIES[truncation]
 
 
 def pack_strings(strs):
@@ -336,7 +356,8 @@ class Tokenize(object):
 
     def __call__(self, text, pair_text=None, max_len=None, padding=True, truncation=True, return_offset=False, return_offsets_mapping=False, **kw):
         """tokenize.py:184-259.  `text_pair=` is accepted as an alias of `pair_text`.  return_offsets_mapping: also
-        'offset_mapping', a (start, end) byte range per token (see encode_batch)."""
+        'offset_mapping', a (start, end) byte range per token (see encode_batch).  truncation: as encode_batch (a pair that
+        a strategy cannot truncate raises ValueError)."""
         if "text_pair" in kw:
             if pair_text is not None:
                 raise TypeError("pass pair_text or text_pair, not both")
@@ -372,6 +393,9 @@ class Tokenize(object):
         if r._offsets is not None:
             result['offset_mapping'] = [tuple(p) for p in r._offsets[s:e].tolist()]
         if r._has_pair:
+            if r._status[i] == 2:
+                raise ValueError("truncation=%r cannot truncate row %d to max_len: the text it may cut is too short (HF's "
+                                 "SequenceTooShort)" % (r._strategy, i))
             if r._status[i]:
                 raise ValueError("None is not in list")                   # tokenize.py:157-159
             pad, _, eos = self._special_ids()[:3]
@@ -399,6 +423,7 @@ class Tokenize(object):
             pbp = pop = None
         if return_offset:
             flags |= L.WANT_SPANS
+        strategy = _strategy_flag(truncation, max_len, padding, return_offset)
         enc = L.Encoded()
         ml = L.MAX_LEN_NONE if max_len is None else int(max_len)
         if max_len is not None and not -(2 ** 31) < ml < 2 ** 31:
@@ -406,16 +431,19 @@ class Tokenize(object):
         tb = np.ascontiguousarray(tb, dtype=np.uint8)
         to = np.ascontiguousarray(to, dtype=np.int64)
         rc = self._lib.genztok_encode(self._h, tb.ctypes.data, to.ctypes.data, pbp, pop, n, ml, int(bool(padding)), int(bool(truncation)),
-                                      flags, C.byref(enc))
+                                      flags | strategy, C.byref(enc))
         if rc:
             self._err(rc, "genztok_encode")
-        return self._wrap(enc, n, max_len is not None and bool(padding), _EncodedOwner(self, enc))
+        r = self._wrap(enc, n, max_len is not None and bool(padding), _EncodedOwner(self, enc))
+        r._strategy = truncation if strategy else None
+        return r
 
     def _wrap(self, enc, n, pad_mode, owner):
         """BatchEncoding of numpy views over the n rows of a genztok_encoded_t."""
         r = BatchEncoding()
         r._tok, r._n, r._width, r._has_pair = self, n, int(enc.width), bool(enc.has_pair)
         r._pad_mode = pad_mode
+        r._strategy = None
         tot = int(enc.total)
         r._ids = _view(enc.input_ids, tot, C.c_int32, np.int32, owner)
         r._mask = _view(enc.attention_mask, tot, C.c_uint8, np.uint8, owner)
@@ -460,7 +488,12 @@ class Tokenize(object):
         return_offsets_mapping: also 'offset_mapping', int32 [n, max_len, 2] (fixed layout) or [total, 2] (ragged): the
         [start, end) byte range of each token in the UTF-8 ('surrogatepass') bytes of its own document -- `texts[i]`, or
         `pair_texts[i]` for tokens of the second text -- and (0, 0) for <s>, </s>, pads and the </s> truncation adds.
-        It changes no other output."""
+        It changes no other output.
+        truncation: True / False as the reference (True cuts the concatenation <s> A </s></s> B </s> to max_len), or for pairs
+        HF's "longest_first" (the Rust tokenizers' rule), "only_first" or "only_second": each text keeps a prefix so that the
+        row fits max_len.  A pair that only_first / only_second cannot truncate gets row_status 2 and the True row on every
+        plane; row(i) raises ValueError for it.  The strategies need max_len >= 4, padding=True and return_offset=False;
+        include/genztok.h states the rule."""
         flags = L.WANT_OFFSETS if return_offsets_mapping else 0
         if pair_texts is not None:
             flags |= (L.WANT_TOKEN_TYPE if token_type_ids else 0) | (L.WANT_SEQUENCE_ID if sequence_id else 0)
@@ -592,11 +625,16 @@ class Tokenize(object):
         return [raw[off[i]:off[i + 1]].decode("utf-8", "surrogatepass") for i in range(n)]
 
     def encode_device(self, d_text, d_text_off, d_pair=None, d_pair_off=None, max_len=128, token_type_ids=True, sequence_id=False,
-                      out=None, text_bytes=None, pair_bytes=None):
+                      out=None, text_bytes=None, pair_bytes=None, truncation=True):
         """Fixed-layout encode with everything resident on the GPU.  Inputs are torch CUDA tensors (uint8 bytes whose
         storage is 16-byte aligned and int64 offsets[n+1]); outputs are torch tensors (DLPack-exportable) on the same
-        device, written on torch's current stream.  Nothing crosses PCIe and the call does not synchronise."""
+        device, written on torch's current stream.  Nothing crosses PCIe and the call does not synchronise.
+        truncation: True (the reference cut) or a pair strategy as in encode_batch; with a strategy and pairs the call
+        synchronises once per text to size the token streams, and row_status 2 marks the rows the strategy cannot truncate."""
         import torch
+        if not isinstance(truncation, str) and not truncation:
+            raise ValueError("encode_device always truncates (the fixed layout): truncation must be True or a strategy name")
+        strategy = _strategy_flag(truncation, max_len)
         n = d_text_off.numel() - 1
         dev = d_text.device
         has_pair = d_pair_off is not None
@@ -614,9 +652,9 @@ class Tokenize(object):
         P = L.DevPlanes()
         for k in ("input_ids", "attention_mask", "token_type_ids", "sequence_id", "row_len", "seq_len", "row_status"):
             setattr(P, k, out[k].data_ptr() if k in out else None)
-        flags = 0
+        flags = strategy
         if has_pair:
-            flags = (L.WANT_TOKEN_TYPE if "token_type_ids" in out else 0) | (L.WANT_SEQUENCE_ID if "sequence_id" in out else 0)
+            flags |= (L.WANT_TOKEN_TYPE if "token_type_ids" in out else 0) | (L.WANT_SEQUENCE_ID if "sequence_id" in out else 0)
         tbytes = d_text.numel() if text_bytes is None else text_bytes
         pbytes = (d_pair.numel() if pair_bytes is None else pair_bytes) if has_pair else 0
         slot = 0

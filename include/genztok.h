@@ -51,6 +51,26 @@ extern "C" {
  * least one byte.  Asking for offsets changes no other output.  (Documents are limited to max_chunk_bytes <= 512 MiB, so every
  * byte offset fits an int32.) */
 #define GENZTOK_WANT_OFFSETS 8u
+/* Pair truncation strategies (HF's truncation="longest_first" / "only_first" / "only_second"), for genztok_encode and
+ * genztok_encode_device; at most one.  Without them, truncation cuts the concatenation [bos] A [eos eos] B [eos] to max_len and
+ * forces a final </s> (tokenize.py:141-146), which can drop all of B.  With la, lb the untruncated token counts of the two texts
+ * (len(encode(x)) - 2) and C = max_len - 4:
+ *  - la + lb <= C: every strategy gives the row of the reference cut, on every plane.
+ *  - LONGEST_FIRST, the rule of the Rust `tokenizers` library (HF's fast tokenizers, truncate_encodings / LongestFirst): the
+ *    shorter text (the first when la == lb) stays whole when it has at most floor(C/2) tokens and the longer keeps C - shorter;
+ *    otherwise the shorter keeps floor(C/2) and the longer ceil(C/2).  At C = 9: (3, 20) -> (3, 6), (20, 3) -> (6, 3),
+ *    (10, 10) -> (4, 5), (20, 10) -> (5, 4).  (HF's Python "slow" tokenizers break the tie the other way: (10, 10) -> (5, 4).)
+ *  - ONLY_SECOND: A stays whole and B keeps C - la tokens, when la < C.  ONLY_FIRST: B stays whole and A keeps C - lb, when
+ *    lb < C.  Otherwise (HF raises SequenceTooShort) the row's row_status is 2 and its planes hold the reference cut's row.
+ * The kept tokens form [bos] + A[:la'] + [eos, eos] + B[:lb'] + [eos] (at most max_len entries), which then goes through the
+ * reference's padding, attention mask, get_sequence_id and get_token_type unchanged: a row of exactly max_len entries gets the
+ * </s>-id last token type, and row_status 1 happens only where those rules raise on that list (a literal <s> / </s> word in a
+ * text).  With GENZTOK_WANT_OFFSETS (host form) a kept token has its untruncated offsets, everything else (0, 0).  Requires
+ * max_len >= 4 and, for genztok_encode, padding, truncation and no GENZTOK_WANT_SPANS; otherwise GENZTOK_E_INVALID, reported
+ * before the device is looked at.  A batch without second texts ignores the strategy. */
+#define GENZTOK_LONGEST_FIRST 16u
+#define GENZTOK_ONLY_FIRST 32u
+#define GENZTOK_ONLY_SECOND 64u
 
 /* Entries of the int8 planes */
 #define GENZTOK_NONE (-1)      /* Python None */
@@ -77,7 +97,8 @@ typedef struct genztok_encoded {
     int8_t *sequence_id;     /* [total] or NULL */
     int32_t *tt_len;         /* [n] or NULL */
     int32_t *seq_len;        /* [n] or NULL */
-    uint8_t *row_status;     /* [n] or NULL; 1 = the reference raises ValueError (tokenize.py:157-159) */
+    uint8_t *row_status;     /* [n] or NULL; 1 = the reference raises ValueError (tokenize.py:157-159); 2 = the pair truncation
+                              * strategy of the call cannot apply (HF's SequenceTooShort; takes precedence over 1) */
     int64_t *span_off;       /* [n+1] entries of `spans` per row, or NULL */
     int32_t *spans;          /* [span_off[n]][2] (first,last) token index pairs, or NULL */
     int64_t real_tokens;     /* sum over rows of attention_mask */
@@ -145,7 +166,10 @@ void genztok_free_encoded(genztok_t *h, genztok_encoded_t *out);
  * stream) of device slot `dev` (index into device_ids).  Fixed layout only: requires
  * max_len >= 1, padding and truncation.  Asynchronous: returns after enqueueing.
  * GENZTOK_WANT_SPANS and GENZTOK_WANT_OFFSETS are rejected (GENZTOK_E_INVALID).  For offsets on the device use
- * genztok_encode_windows_device: window 0 of each document (rows d_win_off[:-1]) is its genztok_encode row. */
+ * genztok_encode_windows_device: window 0 of each document (rows d_win_off[:-1]) is its genztok_encode row.
+ * A pair truncation strategy (GENZTOK_LONGEST_FIRST / _ONLY_FIRST / _ONLY_SECOND, with pairs) needs input_ids, attention_mask and
+ * row_len, and synchronises: the token streams of the two texts are sized by reading their length back from the device, once per
+ * text, before the rows are written. */
 int genztok_encode_device(genztok_t *h, int dev, const uint8_t *d_text, const int64_t *d_text_off,
                           int64_t text_bytes, const uint8_t *d_pair, const int64_t *d_pair_off,
                           int64_t pair_bytes, int64_t n, int32_t max_len, uint32_t flags,
