@@ -94,6 +94,12 @@ SIGNATURES = {
                                               C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "genztok_mlm_mask_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_double,
                                          C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "genztok_encode_dropout": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_uint32, C.c_double, C.c_uint64,
+                                         C.c_void_p, C.POINTER(Encoded)]),
+    "genztok_encode_dropout_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int32,
+                                                C.c_uint32, C.c_double, C.c_uint64, C.c_void_p, C.POINTER(DevPlanes), C.c_void_p]),
+    "genztok_bpe_word_dropout": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int64, C.c_double, C.c_uint64, C.c_int64, C.POINTER(C.c_int32), C.c_int64,
+                                           C.POINTER(C.c_int64)]),
     "genztok_digest_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p]),
 }
 

@@ -45,8 +45,20 @@ __device__ __forceinline__ uint32_t bpe_symbols(const DevTables& T, const uint8_
     return n;
 }
 
+// BPE-dropout (dropout.cuh, include/genztok.h states the rule): drop(t, i) says whether the pair at position i of round t's
+// sequence is left out of that round -- it neither competes for the lowest rank nor is merged.  NoDrop is the reference's loop and
+// compiles to it; BpeDrop is the hash draw of one word: w = W_j, thr = floor(p * 2^32).
+struct NoDrop {
+    __device__ __forceinline__ bool operator()(uint32_t, uint32_t) const { return false; }
+};
+struct BpeDrop {
+    uint64_t w, thr;
+    __device__ __forceinline__ bool operator()(uint32_t t, uint32_t i) const { return (mix64(w + (((uint64_t)t << 32) | i)) >> 32) < thr; }
+};
+
 // The merge rounds (tokenize.py:69-98) on S[0..n). Returns the new length.
-__device__ __forceinline__ uint32_t bpe_rounds(const DevTables& T, uint32_t* S, uint32_t n, int lane) {
+template <class Drop = NoDrop>
+__device__ __forceinline__ uint32_t bpe_rounds(const DevTables& T, uint32_t* S, uint32_t n, int lane, const Drop& drop = Drop()) {
     for (uint32_t round = 0, n0 = n; n > 1 && round <= n0; round++) {   // every round removes >= 1 symbol
         // ---- bigram = min(pairs, key=rank)  (:70-71)
         uint32_t best = 0xFFFFFFFFu, ba = 0, bb = 0, bm = 0;
@@ -55,7 +67,7 @@ __device__ __forceinline__ uint32_t bpe_rounds(const DevTables& T, uint32_t* S, 
             if (i + 1 < n) {
                 uint32_t a = S[i], b = S[i + 1], mg;
                 uint32_t r = pair_rank(T, a, b, &mg);
-                if (r < best) { best = r; ba = a; bb = b; bm = mg; }
+                if (r < best && !drop(round, i)) { best = r; ba = a; bb = b; bm = mg; }
             }
         }
         uint32_t gbest = __reduce_min_sync(FULL_MASK, best);
@@ -70,7 +82,7 @@ __device__ __forceinline__ uint32_t bpe_rounds(const DevTables& T, uint32_t* S, 
             uint32_t i = base + lane;
             uint32_t a = i < n ? S[i] : SYM_NONE;
             uint32_t b = i + 1 < n ? S[i + 1] : SYM_NONE;
-            bool match = (i + 1 < n) && a == ba && b == bb;
+            bool match = (i + 1 < n) && a == ba && b == bb && !drop(round, i);   // (a dropped occurrence breaks a run of equal pairs)
             uint32_t m = __ballot_sync(FULL_MASK, match);
             uint32_t sel;
             if (ba == bb) {
@@ -103,13 +115,16 @@ __device__ __forceinline__ uint32_t bpe_rounds(const DevTables& T, uint32_t* S, 
 // merge site instead of one per symbol.  A 1,200-byte token costs ~40 look-up round trips per round the plain loop above; here ~2.
 // R needs n entries; dlist is a 64-entry scratch list in shared memory.  (tokenize.py:69-98: the same rounds, the same result.)
 static const uint32_t RANK_NONE = 0xFFFFFFFFu, RANK_DIRTY = 0xFFFFFFFEu;
-__device__ __forceinline__ uint32_t bpe_rounds_cached(const DevTables& T, uint32_t* S, uint32_t* R, uint32_t n, int lane, uint32_t* dlist) {
+// Under dropout R keeps the ranks: a round only masks which of them compete and merge.
+template <class Drop = NoDrop>
+__device__ __forceinline__ uint32_t bpe_rounds_cached(const DevTables& T, uint32_t* S, uint32_t* R, uint32_t n, int lane, uint32_t* dlist,
+                                                      const Drop& drop = Drop()) {
     for (uint32_t i = lane; i < n; i += 32) { uint32_t mg; R[i] = i + 1 < n ? pair_rank(T, S[i], S[i + 1], &mg) : RANK_NONE; }
     __syncwarp();
     for (uint32_t round = 0, n0 = n; n > 1 && round <= n0; round++) {
         // ---- bigram = min(pairs, key=rank)  (:70-71)
         uint32_t best = RANK_NONE, bi = 0;
-        for (uint32_t i = lane; i + 1 < n; i += 32) { const uint32_t r = R[i]; if (r < best) { best = r; bi = i; } }
+        for (uint32_t i = lane; i + 1 < n; i += 32) { const uint32_t r = R[i]; if (r < best && !drop(round, i)) { best = r; bi = i; } }
         const uint32_t gbest = __reduce_min_sync(FULL_MASK, best);
         if (gbest >= RANK_DIRTY) break;                          // `if bigram not in self.bpe_ranks: break` (:72-73)
         const int src = __ffs(__ballot_sync(FULL_MASK, best == gbest)) - 1;
@@ -125,7 +140,7 @@ __device__ __forceinline__ uint32_t bpe_rounds_cached(const DevTables& T, uint32
             const uint32_t i = base + lane;
             const uint32_t a = i < n ? S[i] : SYM_NONE;
             const uint32_t r = i < n ? R[i] : RANK_NONE;
-            const bool match = (i + 1 < n) && r == gbest;
+            const bool match = (i + 1 < n) && r == gbest && !drop(round, i);
             const uint32_t m = __ballot_sync(FULL_MASK, match);
             uint32_t sel;
             if (ba == bb) {                                      // runs of equal symbols: every second match from the run start (a a a -> aa a)
@@ -299,6 +314,15 @@ __global__ void k_bpe_single(DevTables T, const uint8_t* word, uint32_t len, uin
     const int lane = threadIdx.x & 31;
     uint32_t n = bpe_symbols(T, word, len, scratch, lane);
     n = bpe_rounds(T, scratch, n, lane);
+    for (uint32_t i = lane; i < n; i += 32) piece_ncp[i] = scratch[i] == SYM_NONE ? 1u : T.sym_ncp[scratch[i]] - ((i == n - 1) ? 4u : 0u);
+    if (lane == 0) *n_out = n;
+}
+
+// The same under BPE-dropout (genztok_bpe_word_dropout): D holds the draws of the word.
+__global__ void k_bpe_single_dropout(DevTables T, const uint8_t* word, uint32_t len, uint32_t* scratch, uint32_t* piece_ncp, uint32_t* n_out, BpeDrop D) {
+    const int lane = threadIdx.x & 31;
+    uint32_t n = bpe_symbols(T, word, len, scratch, lane);
+    n = bpe_rounds(T, scratch, n, lane, D);
     for (uint32_t i = lane; i < n; i += 32) piece_ncp[i] = scratch[i] == SYM_NONE ? 1u : T.sym_ncp[scratch[i]] - ((i == n - 1) ? 4u : 0u);
     if (lane == 0) *n_out = n;
 }

@@ -16,6 +16,7 @@
 // Decode is k_decode_len (lengths, trailing pad runs) -> k_scan_i64 -> k_decode_write.
 // Extractive QA over the windows' offsets (qa.cuh): [k_qa_char_to_byte ->] k_qa_labels; k_qa_spans -> k_qa_spans_docs.
 // MLM inputs and labels from an id plane (mlm.cuh): k_mlm_mask<WHOLE_WORD>.
+// BPE-dropout rows (dropout.cuh): k_dropout_stream -> k_dropout_rows -> k_post_rows (row list); no word cache, no read-back.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -34,6 +35,7 @@
 #include "../../include/genztok.h"
 #include "bpe.cuh"
 #include "device_common.cuh"
+#include "dropout.cuh"
 #include "encode.cuh"
 #include "flat.cuh"
 #include "gather.cuh"
@@ -125,6 +127,8 @@ struct DeviceCtx {
     struct WinState {
         DevBuf ids[2], off[2], count, woff, fix, doc, start;
         DevBuf offs[2], plane_offs;               // offset_mapping: the streams' token offsets, and the host form's [K, W, 2] plane
+        DevBuf len[2];                            // BPE-dropout: ids per slot of the capped streams (which live in ids[2])
+        DevBuf drop_scratch, drop_keys;           // BPE-dropout: symbols and ranks of long words; the host form's row keys of a chunk
         struct { const void *a = nullptr, *a_off = nullptr, *b = nullptr, *b_off = nullptr, *win_off = nullptr; int64_t n = -1, a_bytes = 0, b_bytes = 0;
                  int32_t W = 0, s = 0; bool offs = false; } sig;
         int64_t n_win = -1;                       // windows of that batch; -1: no step 1 to continue from
@@ -810,6 +814,7 @@ WinArgs window_args(DeviceCtx* d, bool pair, int64_t n, int32_t W, int32_t s) {
     A.ids_a = d->win.ids[0].as<int32_t>(); A.off_a = d->win.off[0].as<int64_t>();
     if (pair) { A.ids_b = d->win.ids[1].as<int32_t>(); A.off_b = d->win.off[1].as<int64_t>(); }
     A.offs_a = d->win.offs[0].as<int2>(); A.offs_b = pair ? d->win.offs[1].as<int2>() : nullptr;
+    A.len_a = d->win.len[0].as<int32_t>(); A.len_b = pair ? d->win.len[1].as<int32_t>() : nullptr;
     A.n_docs = n; A.W = W; A.stride = s;
     A.ctr = d->C.ctr;
     A.eos_i8 = eos_as_i8(d); A.pad_i8 = pad_as_i8(d);
@@ -845,7 +850,8 @@ int windows_layout(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& a, c
 
 // Step 2: the K windows' planes and maps from the streams step 1 left (does not synchronise).  win_doc = doc_base + document.
 // With GENZTOK_WANT_OFFSETS in flags, P.offsets receives [K, W, 2] token offsets (step 1 must have run with offsets).
-// strategy: the K = n rows of a pair truncation strategy (k_pair_rows); d_win_off, win_doc and win_start are not used.
+// strategy: the K = n rows of a pair truncation strategy (k_pair_rows), or with STREAMS_CAPPED the K = n reference rows of the capped
+// streams dropout_layout left (k_dropout_rows); d_win_off, win_doc and win_start are not used.
 int windows_write(genztok_t* h, DeviceCtx* d, cudaStream_t st, bool pair, int64_t n, int32_t W, int32_t s, int32_t strategy, uint32_t flags,
                   const int64_t* d_win_off, int64_t K, const genztok_dev_planes_t& P, int64_t* win_doc, int32_t* win_start, int64_t doc_base) {
     if (K <= 0) return GENZTOK_OK;
@@ -869,8 +875,12 @@ int windows_write(genztok_t* h, DeviceCtx* d, cudaStream_t st, bool pair, int64_
     {
         // algorithmic bytes: the planes and per-window values written (the windows' tokens are read from the streams, mostly in L2)
         const int64_t alg = K * (int64_t)W * (5 + (A.tt ? 1 : 0) + (A.seq ? 1 : 0) + (offs ? 8 : 0)) + K * (4 + 8 + 4 + (pair ? 5 : 0));
-        LaunchScope ls(h, d, strategy ? (offs ? "k_pair_rows_offsets" : "k_pair_rows") : offs ? "k_window_rows_offsets" : "k_window_rows", alg);
-        if (strategy) {
+        LaunchScope ls(h, d, strategy == STREAMS_CAPPED ? "k_dropout_rows" : strategy ? (offs ? "k_pair_rows_offsets" : "k_pair_rows")
+                                                                                : offs ? "k_window_rows_offsets" : "k_window_rows", alg);
+        if (strategy == STREAMS_CAPPED) {
+            if (pair) { if (quad) k_dropout_rows<true, true><<<grid, 256, 0, st>>>(d->T, A); else k_dropout_rows<false, true><<<grid, 256, 0, st>>>(d->T, A); }
+            else { if (quad) k_dropout_rows<true, false><<<grid, 256, 0, st>>>(d->T, A); else k_dropout_rows<false, false><<<grid, 256, 0, st>>>(d->T, A); }
+        } else if (strategy) {
             if (offs) { if (quad) k_window_rows<true, true, true, true><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, true, true, true><<<grid, 256, 0, st>>>(d->T, A); }
             else { if (quad) k_window_rows<true, true, false, true><<<grid, 256, 0, st>>>(d->T, A); else k_window_rows<false, true, false, true><<<grid, 256, 0, st>>>(d->T, A); }
         } else if (offs) {
@@ -887,11 +897,40 @@ int windows_write(genztok_t* h, DeviceCtx* d, cudaStream_t st, bool pair, int64_
         Q.ids = P.input_ids; Q.W = W; Q.n_rows = K; Q.row_list = A.fix_list;
         Q.has_pair = 1; Q.tt = A.tt; Q.seq = A.seq; Q.seq_len = A.seq_len; Q.status = A.status;
         Q.has_max_len = 1; Q.max_len = W; Q.padding = 1; Q.truncation = 1; Q.eos_i8 = A.eos_i8; Q.pad_i8 = A.pad_i8;
-        LaunchScope ls(h, d, strategy ? "k_post_rows_pairs" : "k_post_rows_windows");
-        if (strategy) k_post_rows<true><<<d->sm_count, 256, 0, st>>>(d->T, Q, d->C.ctr + C_FIX);
+        const bool keep2 = strategy && strategy != STREAMS_CAPPED;    // (status 2 exists only for the strategies)
+        LaunchScope ls(h, d, strategy == STREAMS_CAPPED ? "k_post_rows_dropout" : strategy ? "k_post_rows_pairs" : "k_post_rows_windows");
+        if (keep2) k_post_rows<true><<<d->sm_count, 256, 0, st>>>(d->T, Q, d->C.ctr + C_FIX);
         else k_post_rows<<<d->sm_count, 256, 0, st>>>(d->T, Q, d->C.ctr + C_FIX);
         CU(cudaGetLastError());
     }
+    return GENZTOK_OK;
+}
+
+// BPE-dropout, step 1: the two capped token streams of n documents (k_dropout_stream) into d->win.ids / d->win.len, for
+// windows_write(..., STREAMS_CAPPED, ...).  Row d's key is d_keys[d] (device memory), or key_base + d.  Does not synchronise; the
+// buffers grow (cudaMalloc) only when a call is larger than every earlier one on the device.  The word cache is not used.
+int dropout_layout(genztok_t* h, DeviceCtx* d, cudaStream_t st, const Side& a, const Side* b, int64_t n, int32_t W, double p, uint64_t seed,
+                   const int64_t* d_keys, int64_t key_base) {
+    d->win.n_win = -1;                                               // the window streams are about to change
+    const size_t slots = (size_t)n * (size_t)(W + 2);
+    const int64_t nbytes = a.nbytes + (b ? b->nbytes : 0);
+    for (int s = 0; s < (b ? 2 : 1); s++) { CU(d->win.ids[s].ensure(slots * 4 + 16)); CU(d->win.len[s].ensure((size_t)n * 4 + 16)); }
+    CU(d->win.drop_scratch.ensure((size_t)nbytes * 8 + 64));
+    DropArgs A{};
+    A.a = a; if (b) A.b = *b;
+    A.n = n; A.cap = W;
+    A.s0 = mix64(seed ^ DROP_K); A.thr = (uint64_t)std::floor(p * 4294967296.0);
+    A.row_keys = d_keys; A.key_base = key_base;
+    A.ids_a = d->win.ids[0].as<int32_t>(); A.len_a = d->win.len[0].as<int32_t>();
+    if (b) { A.ids_b = d->win.ids[1].as<int32_t>(); A.len_b = d->win.len[1].as<int32_t>(); }
+    A.scratch = d->win.drop_scratch.as<uint32_t>(); A.b_base = a.nbytes; A.nbytes = nbytes;
+    A.ctr = d->C.ctr;
+    const int64_t warps = b ? 2 * n : n;
+    {
+        LaunchScope ls(h, d, "k_dropout_stream", nbytes + (int64_t)slots * 4 * (b ? 2 : 1));
+        k_dropout_stream<<<(unsigned)std::max<int64_t>(1, std::min<int64_t>((warps + 7) / 8, (int64_t)d->sm_count * 64)), 256, 0, st>>>(d->T, A);
+    }
+    CU(cudaGetLastError());
     return GENZTOK_OK;
 }
 
@@ -991,7 +1030,7 @@ void free_result(genztok_t* h, Out* out) {
 // ================================================================================================
 extern "C" {
 
-const char* genztok_version(void) { return "genztok-b200 0.5 (sm_100a)"; }
+const char* genztok_version(void) { return "genztok-b200 0.6 (sm_100a)"; }
 
 const char* genztok_last_error(const genztok_t* h) { return h ? h->err.c_str() : g_create_err.c_str(); }
 
@@ -1043,7 +1082,9 @@ void genztok_destroy(genztok_t* h) {
         if (d->over32_ev) cudaEventDestroy(d->over32_ev);
         if (d->last_done) cudaEventDestroy(d->last_done);
         d->synth_len.release();
-        for (DevBuf* b : {&d->win.ids[0], &d->win.ids[1], &d->win.off[0], &d->win.off[1], &d->win.count, &d->win.woff, &d->win.fix, &d->win.doc, &d->win.start}) b->release();
+        for (DevBuf* b : {&d->win.ids[0], &d->win.ids[1], &d->win.off[0], &d->win.off[1], &d->win.count, &d->win.woff, &d->win.fix, &d->win.doc, &d->win.start,
+                          &d->win.offs[0], &d->win.offs[1], &d->win.plane_offs, &d->win.len[0], &d->win.len[1], &d->win.drop_scratch, &d->win.drop_keys})
+            b->release();
         for (auto& fb : d->flat) for (DevBuf* b : {&fb.dsb, &fb.st, &fb.tpref, &fb.cnt, &fb.wtok}) b->release();
         if (d->stream) cudaStreamDestroy(d->stream);
         delete d;
@@ -1292,6 +1333,8 @@ struct EncodeJob {
     bool has_pair, has_max_len, want_spans, fixed, want_tt, want_seq;
     bool want_offs;                // offset_mapping: the ragged pipeline writes token offsets beside the ids
     int32_t strategy;              // pairs: a truncation strategy (PAIR_*, window.cuh) or 0; its rows are written by windows_chunks
+    bool dropout;                  // BPE-dropout rows (dropout.cuh), written by windows_chunks: probability, seed, host row keys or NULL
+    double drop_p; uint64_t drop_seed; const int64_t* drop_keys;
     genztok_encoded_t* out;
     int32_t old_dirty[4];          // fixed layout: columns of the result planes (ids, mask, token types, sequence ids) that may hold something
                                    // other than padding from the buffer's last use (the width: unknown / a fresh buffer)
@@ -1660,11 +1703,11 @@ struct WindowPart {
 
 // Windows of one device's chunks: per chunk the text goes up, both steps run, the planes and maps come home.
 // win_off[r] for r in (rb, re] is written relative to the part's first window.
-// With J.strategy the chunk's rows (one per document) go straight into the fixed-layout planes of J.out at their rows, and win_off
-// is not used.
+// With J.strategy or J.dropout the chunk's rows (one per document) go straight into the fixed-layout planes of J.out at their rows,
+// and win_off is not used.
 void windows_chunks(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int32_t stride, int64_t* win_off, const std::vector<int64_t>& cuts, WindowPart* part) {
     cudaStream_t st = d->stream;
-    const bool has_pair = J.has_pair, rows = J.strategy != 0;
+    const bool has_pair = J.has_pair, rows = J.strategy != 0 || J.dropout;
     const int32_t W = J.max_len;
     const int64_t rb = cuts.front(), re = cuts.back();
     for (size_t ci = 0; ci + 1 < cuts.size(); ci++) {
@@ -1675,8 +1718,18 @@ void windows_chunks(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int32_t stri
         Side a, b;
         CUF(upload_chunk(J, r0, r1, d->text, d->toff, d->pair, d->poff, st, &a, &b));
         CUF(d->win.woff.ensure((size_t)(m + 1) * 8));
-        int64_t K = 0;
-        FAIL_RC(windows_layout(h, d, st, a, has_pair ? &b : nullptr, m, W, stride, J.strategy, J.want_offs, d->win.woff.as<int64_t>(), &K));
+        int64_t K = m;
+        if (J.dropout) {                                             // the row keys: the caller's, or the rows' indices in the whole call
+            const int64_t* keys = nullptr;
+            if (J.drop_keys) {
+                CUF(d->win.drop_keys.ensure((size_t)m * 8));
+                CUF(cudaMemcpyAsync(d->win.drop_keys.p, J.drop_keys + r0, (size_t)m * 8, cudaMemcpyHostToDevice, st));
+                keys = d->win.drop_keys.as<int64_t>();
+            }
+            FAIL_RC(dropout_layout(h, d, st, a, has_pair ? &b : nullptr, m, W, J.drop_p, J.drop_seed, keys, r0));
+        } else {
+            FAIL_RC(windows_layout(h, d, st, a, has_pair ? &b : nullptr, m, W, stride, J.strategy, J.want_offs, d->win.woff.as<int64_t>(), &K));
+        }
         const size_t tot = (size_t)K * (size_t)W;
         CUF(d->ids.ensure(tot * 4 + 16)); CUF(d->mask.ensure(tot + 16)); CUF(d->row_len.ensure((size_t)K * 4 + 16));
         CUF(d->win.doc.ensure((size_t)K * 8 + 16)); CUF(d->win.start.ensure((size_t)K * 4 + 16));
@@ -1686,7 +1739,8 @@ void windows_chunks(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int32_t stri
         if (J.want_seq) { CUF(d->seq.ensure(tot + 16)); P.sequence_id = d->seq.as<int8_t>(); }
         if (has_pair) { CUF(d->seq_len.ensure((size_t)K * 4 + 16)); CUF(d->status.ensure((size_t)K + 16)); P.seq_len = d->seq_len.as<int32_t>(); P.row_status = d->status.as<uint8_t>(); }
         if (J.want_offs) { CUF(d->win.plane_offs.ensure(tot * 8 + 16)); P.offsets = d->win.plane_offs.as<int32_t>(); }
-        FAIL_RC(windows_write(h, d, st, has_pair, m, W, stride, J.strategy, J.flags, d->win.woff.as<int64_t>(), K, P, d->win.doc.as<int64_t>(), d->win.start.as<int32_t>(), r0));
+        FAIL_RC(windows_write(h, d, st, has_pair, m, W, stride, J.dropout ? STREAMS_CAPPED : J.strategy, J.flags, d->win.woff.as<int64_t>(), K, P,
+                              d->win.doc.as<int64_t>(), d->win.start.as<int32_t>(), r0));
         // where the chunk's rows go on the host: the result planes at rows r0.. (strategy), else the part's arrays behind its windows so far
         genztok_dev_planes_t H{};
         size_t o = (size_t)r0;
@@ -1737,6 +1791,12 @@ void windows_chunks(genztok_t* h, DeviceCtx* d, const EncodeJob& J, int32_t stri
     }
 }
 
+// BPE-dropout of a host-buffer encode (genztok_encode_dropout): probability, seed, host row keys or NULL.
+struct DropSpec { double p; uint64_t seed; const int64_t* keys; };
+
+int encode_host(genztok_t* h, const uint8_t* text, const int64_t* text_off, const uint8_t* pair, const int64_t* pair_off, int64_t n, int32_t max_len,
+                int padding, int truncation, uint32_t flags, int32_t strategy, const DropSpec* drop, genztok_encoded_t* out);
+
 }  // namespace
 
 extern "C" {
@@ -1748,6 +1808,17 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
     int32_t strategy = 0;
     { const int rc = pair_strategy(h, flags, max_len, padding && truncation && !(flags & GENZTOK_WANT_SPANS), &strategy); if (rc) return rc; }
     if (h->devs.empty()) return fail(h, GENZTOK_E_NODEVICE, "this handle was created without a CUDA device; there is no CPU path");
+    return encode_host(h, text, text_off, pair, pair_off, n, max_len, padding, truncation, flags, strategy, nullptr, out);
+}
+
+}  // extern "C"
+
+namespace {
+
+// The host-buffer encode after its argument checks.  drop: the rows of BPE-dropout (the fixed layout, the reference cut), written by
+// windows_chunks like those of a truncation strategy.
+int encode_host(genztok_t* h, const uint8_t* text, const int64_t* text_off, const uint8_t* pair, const int64_t* pair_off, int64_t n, int32_t max_len,
+                int padding, int truncation, uint32_t flags, int32_t strategy, const DropSpec* drop, genztok_encoded_t* out) {
     memset(out, 0, sizeof *out);
     std::lock_guard<std::mutex> lk(h->mu);
     EncodeJob J = make_job(text, text_off, pair, pair_off, max_len, flags);
@@ -1755,10 +1826,12 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
     J.has_max_len = max_len != GENZTOK_MAX_LEN_NONE;
     J.want_spans = (flags & GENZTOK_WANT_SPANS) != 0;       // return_offset: produced by the ragged pipeline
     J.strategy = J.has_pair ? strategy : 0;                 // (without second texts every strategy is the reference cut)
+    if (drop) { J.dropout = true; J.drop_p = drop->p; J.drop_seed = drop->seed; J.drop_keys = drop->keys; }
+    const bool rows = J.strategy || J.dropout;              // one row per document from windows_chunks
     // the fixed regime; with offsets (offset_mapping) it is computed by the ragged pipeline, whose rows then all hold max_len
-    // entries, and presented in the fixed layout; the rows of a truncation strategy are written by windows_chunks
-    const bool fixed_layout = J.has_max_len && max_len >= 1 && padding && truncation && (J.strategy || fixed_fits(h->devs[0], max_len)) && !J.want_spans;
-    J.fixed = fixed_layout && !J.want_offs && !J.strategy;
+    // entries, and presented in the fixed layout; the rows of a truncation strategy or of BPE-dropout are written by windows_chunks
+    const bool fixed_layout = J.has_max_len && max_len >= 1 && padding && truncation && (rows || fixed_fits(h->devs[0], max_len)) && !J.want_spans;
+    J.fixed = fixed_layout && !J.want_offs && !rows;
     const bool has_pair = J.has_pair, fixed = J.fixed;
     OutBlock* ob = new OutBlock();
     out->_owner = ob;
@@ -1777,7 +1850,7 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
     };
 #define OOM_CHECK(p) if (!(p)) { free_nolock(); return fail(h, GENZTOK_E_NOMEM, "pinned host allocation failed"); }
     if (J.want_spans) { out->span_off = out_alloc<int64_t>(h, ob, (size_t)n + 1); OOM_CHECK(out->span_off); out->span_off[0] = 0; }
-    if (fixed || J.strategy) {
+    if (fixed || rows) {
         const size_t tot = (size_t)n * (size_t)max_len;
         out->width = max_len; out->total = (int64_t)tot;
         out->input_ids = out_alloc<int32_t>(h, ob, tot); OOM_CHECK(out->input_ids);
@@ -1786,7 +1859,7 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
         if (J.want_tt) { out->token_type_ids = out_alloc<int8_t>(h, ob, tot); OOM_CHECK(out->token_type_ids); out->tt_len = out_alloc<int32_t>(h, ob, (size_t)n); OOM_CHECK(out->tt_len); }
         if (J.want_seq) { out->sequence_id = out_alloc<int8_t>(h, ob, tot); OOM_CHECK(out->sequence_id); }
         if (has_pair) { out->seq_len = out_alloc<int32_t>(h, ob, (size_t)n); OOM_CHECK(out->seq_len); out->row_status = out_alloc<uint8_t>(h, ob, (size_t)n); OOM_CHECK(out->row_status); }
-        if (J.strategy) {
+        if (rows) {
             if (J.want_offs) { out->offsets = out_alloc<int32_t>(h, ob, 2 * tot); OOM_CHECK(out->offsets); }
             for (auto& pr : ob->pinned) h->plane_meta.erase(pr.first);   // (these planes are written whole; no record describes them)
         }
@@ -1815,7 +1888,7 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
     // every device writes its own rows of the result; the documents are balanced by bytes
     const int G = (int)h->devs.size();
     const std::vector<int64_t> dcut = shard_rows(G, n, [&](int64_t r) { return text_off[r] + (has_pair ? pair_off[r] : 0) + 64 * r; });
-    if (J.strategy) {
+    if (rows) {
         std::vector<WindowPart> parts((size_t)G);
         run_parts(h, J, dcut, parts, [&](DeviceCtx* d, const std::vector<int64_t>& cuts, WindowPart* pt) { windows_chunks(h, d, J, 0, nullptr, cuts, pt); });
         for (auto& pt : parts)
@@ -1892,6 +1965,63 @@ int genztok_encode(genztok_t* h, const uint8_t* text, const int64_t* text_off, c
         if (fixed_layout) return present_fixed();
     }
     return GENZTOK_OK;
+}
+
+// The argument checks both BPE-dropout encodes share (include/genztok.h).
+int check_dropout_args(genztok_t* h, const char* what, int64_t n, int32_t max_len, uint32_t flags, double p) {
+    if (n < 0) return fail(h, GENZTOK_E_INVALID, "%s: n >= 0 needed (got %lld)", what, (long long)n);
+    if (!(p >= 0.0 && p <= 1.0)) return fail(h, GENZTOK_E_INVALID, "%s: the dropout probability must be in [0, 1] (got %g)", what, p);
+    if (max_len < 4) return fail(h, GENZTOK_E_INVALID, "%s: BPE-dropout needs the fixed layout with max_len >= 4 (got %d)", what, max_len);
+    if (flags & ~(uint32_t)(GENZTOK_WANT_TOKEN_TYPE | GENZTOK_WANT_SEQUENCE_ID))
+        return fail(h, GENZTOK_E_INVALID, "%s: BPE-dropout takes only GENZTOK_WANT_TOKEN_TYPE and GENZTOK_WANT_SEQUENCE_ID (no offsets, spans or "
+                    "truncation strategy; got flags 0x%x)", what, flags);
+    return GENZTOK_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int genztok_encode_dropout(genztok_t* h, const uint8_t* text, const int64_t* text_off, const uint8_t* pair, const int64_t* pair_off, int64_t n,
+                           int32_t max_len, uint32_t flags, double p, uint64_t seed, const int64_t* row_keys, genztok_encoded_t* out) {
+    if (!h) return GENZTOK_E_INVALID;
+    if (!out || !text_off) return fail(h, GENZTOK_E_INVALID, "genztok_encode_dropout: bad arguments");
+    const int rc = check_dropout_args(h, "genztok_encode_dropout", n, max_len, flags, p);
+    if (rc) return rc;
+    if (h->devs.empty()) return fail(h, GENZTOK_E_NODEVICE, "this handle was created without a CUDA device; there is no CPU path");
+    const DropSpec drop{p, seed, row_keys};
+    return encode_host(h, text, text_off, pair, pair_off, n, max_len, 1, 1, flags, 0, &drop, out);
+}
+
+int genztok_encode_dropout_device(genztok_t* h, int dev, const uint8_t* d_text, const int64_t* d_text_off, int64_t text_bytes, const uint8_t* d_pair,
+                                  const int64_t* d_pair_off, int64_t pair_bytes, int64_t n, int32_t max_len, uint32_t flags, double p, uint64_t seed,
+                                  const int64_t* d_row_keys, const genztok_dev_planes_t* planes, void* stream) {
+    if (!h) return GENZTOK_E_INVALID;
+    int rc = check_dropout_args(h, "genztok_encode_dropout_device", n, max_len, flags, p);
+    if (rc) return rc;
+    if (!d_text_off || (text_bytes > 0 && !d_text) || (d_pair_off && pair_bytes > 0 && !d_pair) || !planes || !planes->input_ids ||
+        !planes->attention_mask || !planes->row_len)
+        return fail(h, GENZTOK_E_INVALID, "genztok_encode_dropout_device: bad arguments (input_ids, attention_mask and row_len are required)");
+    if (((uintptr_t)d_text & 15) || ((uintptr_t)d_pair & 15)) return fail(h, GENZTOK_E_INVALID, "device text buffers must be 16-byte aligned");
+    if (dev < 0 || dev >= (int)h->devs.size()) return fail(h, GENZTOK_E_NODEVICE, "no such device slot %d (handle has %d)", dev, (int)h->devs.size());
+    const bool has_pair = d_pair_off != nullptr;
+    const int64_t bytes = text_bytes + (has_pair ? pair_bytes : 0);
+    if (bytes > h->max_chunk_bytes) return fail(h, GENZTOK_E_LIMIT, "chunk of %lld bytes exceeds max_chunk_bytes=%lld", (long long)bytes, (long long)h->max_chunk_bytes);
+    std::lock_guard<std::mutex> lk(h->mu);
+    DeviceCtx* d = h->devs[(size_t)dev];
+    CU(cudaSetDevice(d->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : d->stream;
+    LaunchScope::cur_stream = st;
+    rc = stream_enter(h, d, st);
+    if (rc) return rc;
+    if (!d->cache_ready) { rc = ensure_cache(h, d, st, 0); if (rc) return rc; }   // (the counters; the word cache itself is not used)
+    if (n > 0) {
+        const Side a{d_text, d_text_off, text_bytes}, b{d_pair, d_pair_off, pair_bytes};
+        rc = dropout_layout(h, d, st, a, has_pair ? &b : nullptr, n, max_len, p, seed, d_row_keys, 0);
+        if (!rc) rc = windows_write(h, d, st, has_pair, n, max_len, 0, STREAMS_CAPPED, flags, nullptr, n, *planes, nullptr, nullptr, 0);
+        if (rc) return rc;
+    }
+    return stream_leave(h, d, st);
 }
 
 }  // extern "C"
@@ -2646,10 +2776,12 @@ int genztok_preprocess_device(genztok_t* h, int dev, int op, const uint8_t* d_te
     return stream_leave(h, d, st);
 }
 
-// ---- helpers ----------------------------------------------------------------------------------------------
-int genztok_bpe_word(genztok_t* h, const uint8_t* word, int64_t word_len, int32_t* piece_cp, int64_t cap, int64_t* n_pieces) {
-    if (!h || !n_pieces || word_len < 0) return GENZTOK_E_INVALID;
-    if (h->devs.empty()) return fail(h, GENZTOK_E_NODEVICE, "this handle was created without a CUDA device; there is no CPU path");
+}  // extern "C"
+
+namespace {
+
+// genztok_bpe_word and, with drop, genztok_bpe_word_dropout after their argument checks.
+int bpe_word(genztok_t* h, const uint8_t* word, int64_t word_len, int32_t* piece_cp, int64_t cap, int64_t* n_pieces, const BpeDrop* drop) {
     *n_pieces = 0;
     if (word_len == 0) return GENZTOK_OK;
     std::lock_guard<std::mutex> lk(h->mu);
@@ -2664,7 +2796,8 @@ int genztok_bpe_word(genztok_t* h, const uint8_t* word, int64_t word_len, int32_
     uint32_t* pieces = scratch + L;
     uint32_t* dn = pieces + L;
     CU(cudaMemcpyAsync(dw, word, L, cudaMemcpyHostToDevice, st));
-    { LaunchScope ls(h, d, "k_bpe_single"); k_bpe_single<<<1, 32, 0, st>>>(d->T, dw, (uint32_t)L, scratch, pieces, dn); }
+    if (drop) { LaunchScope ls(h, d, "k_bpe_single_dropout"); k_bpe_single_dropout<<<1, 32, 0, st>>>(d->T, dw, (uint32_t)L, scratch, pieces, dn, *drop); }
+    else { LaunchScope ls(h, d, "k_bpe_single"); k_bpe_single<<<1, 32, 0, st>>>(d->T, dw, (uint32_t)L, scratch, pieces, dn); }
     CU(cudaGetLastError());
     uint32_t nn = 0;
     CU(cudaMemcpyAsync(&nn, dn, 4, cudaMemcpyDeviceToHost, st));
@@ -2675,6 +2808,27 @@ int genztok_bpe_word(genztok_t* h, const uint8_t* word, int64_t word_len, int32_
         CU(cudaStreamSynchronize(st));
     }
     return GENZTOK_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+// ---- helpers ----------------------------------------------------------------------------------------------
+int genztok_bpe_word(genztok_t* h, const uint8_t* word, int64_t word_len, int32_t* piece_cp, int64_t cap, int64_t* n_pieces) {
+    if (!h || !n_pieces || word_len < 0) return GENZTOK_E_INVALID;
+    if (h->devs.empty()) return fail(h, GENZTOK_E_NODEVICE, "this handle was created without a CUDA device; there is no CPU path");
+    return bpe_word(h, word, word_len, piece_cp, cap, n_pieces, nullptr);
+}
+
+// Word 0 of side 0 of a row with key `key` (include/genztok.h): W_0 = mix64(mix64(mix64(seed ^ DROP_K) + key * GOLD) + GOLD).
+int genztok_bpe_word_dropout(genztok_t* h, const uint8_t* word, int64_t word_len, double p, uint64_t seed, int64_t key, int32_t* piece_cp, int64_t cap,
+                             int64_t* n_pieces) {
+    if (!h || !n_pieces || word_len < 0) return GENZTOK_E_INVALID;
+    if (!(p >= 0.0 && p <= 1.0)) return fail(h, GENZTOK_E_INVALID, "genztok_bpe_word_dropout: the dropout probability must be in [0, 1] (got %g)", p);
+    if (h->devs.empty()) return fail(h, GENZTOK_E_NODEVICE, "this handle was created without a CUDA device; there is no CPU path");
+    const BpeDrop drop{mix64(mix64(mix64(seed ^ DROP_K) + (uint64_t)key * GOLD) + GOLD), (uint64_t)std::floor(p * 4294967296.0)};
+    return bpe_word(h, word, word_len, piece_cp, cap, n_pieces, &drop);
 }
 
 int genztok_sequence_id(genztok_t* h, const int32_t* ids, int64_t n, int apply_token_type, int8_t* out, int64_t* out_len, int* status) {

@@ -13,6 +13,10 @@
 // Pair truncation strategies (k_window_rows<..., KEEP>, launched as k_pair_rows): one row per document from the same streams,
 // [bos] + A[:la'] + [eos, eos] + B[:lb'] + [eos] with (la', lb') = pair_keep(la, lb, W - 4, strategy), padded the same way.  A row
 // whose strategy cannot apply (row_status 2) is the whole pair row, truncated like encode_batch's.
+//
+// BPE-dropout rows (k_dropout_rows, dropout.cuh): one row per document, the reference cut (encode_batch's row), from streams capped
+// at W ids per text: slot d of a stream starts at d * (W + 2) and holds len[d] ids from its entry 1.  A text longer than W shows
+// at most W - 2 of its ids in the row, and the row's framing, token types and status are the same for any length >= W.
 #pragma once
 #include "device_common.cuh"
 #include "encode.cuh"
@@ -39,9 +43,11 @@ struct WinArgs {
     const int2* offs_a; const int2* offs_b;
     int32_t* offs;
     int32_t strategy;                             // k_window_rows<..., KEEP>: PAIR_LONGEST_FIRST / PAIR_ONLY_FIRST / PAIR_ONLY_SECOND
+    const int32_t* len_a; const int32_t* len_b;   // k_dropout_rows: ids per slot of the capped streams (off_a / off_b are not used)
 };
 
-enum { PAIR_LONGEST_FIRST = 1, PAIR_ONLY_FIRST = 2, PAIR_ONLY_SECOND = 3 };
+// STREAMS_CAPPED: not a strategy; tells the host's windows_write to assemble k_dropout_rows from capped streams
+enum { PAIR_LONGEST_FIRST = 1, PAIR_ONLY_FIRST = 2, PAIR_ONLY_SECOND = 3, STREAMS_CAPPED = 4 };
 
 // Tokens kept of each text of a pair by a truncation strategy (include/genztok.h states the rule): la, lb untruncated token counts,
 // C = max_len - 4.  x = la', y = lb'; z = 1 when only_first / only_second cannot remove enough (HF's SequenceTooShort: row_status 2,
@@ -79,29 +85,33 @@ __global__ void __launch_bounds__(256) k_window_count(WinArgs A) {
 // QUAD writes a lane's 4 columns (32 bytes) with two 16-byte stores.
 // KEEP (pairs): row r is document r cut by pair_keep (win_off, stride, win_doc and win_start are not used); a row_status 2 row is
 // the `whole` row.
-template <bool QUAD, bool PAIR, bool OFFS = false, bool KEEP = false>
-__global__ void __launch_bounds__(256) k_window_rows(DevTables T, WinArgs A) {
+// CAPPED (k_dropout_rows): row r is document r, always the `whole` row, from capped streams (len_a / len_b; win_off, stride,
+// win_doc and win_start are not used).
+template <bool QUAD, bool PAIR, bool OFFS, bool KEEP, bool CAPPED>
+__device__ __forceinline__ void window_rows(const DevTables& T, const WinArgs& A) {
     static_assert(PAIR || !KEEP, "truncation strategies are for pairs");
+    static_assert(!(KEEP && CAPPED) && !(OFFS && CAPPED), "capped streams hold the reference cut and no offsets");
+    constexpr bool ROWS = KEEP || CAPPED;                             // row r is document r
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     const int32_t W = A.W;
     uint32_t tok_total = 0;
     for (int64_t r = warp; r < A.n_win; r += nwarps) {
-        int64_t lo = KEEP ? r : 0, hi = A.n_docs - 1;                // the document: last d with win_off[d] <= r
-        if (!KEEP) while (lo < hi) { const int64_t mid = (lo + hi + 1) >> 1; if (A.win_off[mid] <= r) lo = mid; else hi = mid - 1; }
-        const int64_t d = lo, k = KEEP ? 0 : r - A.win_off[d];
-        const int64_t oa = A.off_a[d];
-        const int32_t LA0 = (int32_t)(A.off_a[d + 1] - oa - 2);
-        const int64_t ox = PAIR ? A.off_b[d] : oa;
-        const int32_t L = PAIR ? (int32_t)(A.off_b[d + 1] - ox - 2) : LA0;
+        int64_t lo = ROWS ? r : 0, hi = A.n_docs - 1;                // the document: last d with win_off[d] <= r
+        if (!ROWS) while (lo < hi) { const int64_t mid = (lo + hi + 1) >> 1; if (A.win_off[mid] <= r) lo = mid; else hi = mid - 1; }
+        const int64_t d = lo, k = ROWS ? 0 : r - A.win_off[d];
+        const int64_t oa = CAPPED ? d * (int64_t)(W + 2) : A.off_a[d];
+        const int32_t LA0 = CAPPED ? A.len_a[d] : (int32_t)(A.off_a[d + 1] - oa - 2);
+        const int64_t ox = PAIR && !CAPPED ? A.off_b[d] : oa;
+        const int32_t L = PAIR ? (CAPPED ? A.len_b[d] : (int32_t)(A.off_b[d + 1] - ox - 2)) : LA0;
         const int3 keep = KEEP ? pair_keep(LA0, L, W - 4, A.strategy) : make_int3(LA0, L, 0);
         const int32_t LA = keep.x;                                    // tokens of the first text in the row
         const int32_t C = PAIR ? W - LA - 4 : W - 2;
-        const bool whole = KEEP ? keep.z != 0 : PAIR && C - A.stride < 1;   // one window: the pair row, truncated like encode_batch's
+        const bool whole = CAPPED || (KEEP ? keep.z != 0 : PAIR && C - A.stride < 1);   // one window: the pair row, truncated like encode_batch's
         const int64_t st64 = whole ? 0 : k * (int64_t)(C - A.stride);
         const int32_t st = (int32_t)st64;
         const int32_t len = whole ? L : KEEP ? keep.y : min(C, L - st);
-        if (LA0 < 0 || L < 0 || k < 0 || (!KEEP && k >= window_count(L, LA, PAIR, W, A.stride)) || len < 0) {   // win_off does not fit the streams
+        if (LA0 < 0 || L < 0 || k < 0 || (!ROWS && k >= window_count(L, LA, PAIR, W, A.stride)) || len < 0) {   // win_off does not fit the streams
             if (lane == 0) atomicAdd(&A.ctr[C_ERR], 1ULL);
             continue;
         }
@@ -180,7 +190,7 @@ __global__ void __launch_bounds__(256) k_window_rows(DevTables T, WinArgs A) {
         special = __any_sync(FULL_MASK, special);
         if (lane == 0) {
             A.row_len[r] = Lr;
-            if (!KEEP) {
+            if (!ROWS) {
                 A.win_doc[r] = A.doc_base + d;
                 A.win_start[r] = st;
             }
@@ -194,5 +204,11 @@ __global__ void __launch_bounds__(256) k_window_rows(DevTables T, WinArgs A) {
     tok_total = __reduce_add_sync(FULL_MASK, tok_total);
     if (lane == 0 && tok_total) atomicAdd(&A.ctr[C_TOKENS], (unsigned long long)tok_total);
 }
+
+template <bool QUAD, bool PAIR, bool OFFS = false, bool KEEP = false>
+__global__ void __launch_bounds__(256) k_window_rows(DevTables T, WinArgs A) { window_rows<QUAD, PAIR, OFFS, KEEP, false>(T, A); }
+
+template <bool QUAD, bool PAIR>
+__global__ void __launch_bounds__(256) k_dropout_rows(DevTables T, WinArgs A) { window_rows<QUAD, PAIR, false, false, true>(T, A); }
 
 }  // namespace gzt

@@ -12,7 +12,8 @@ form but encode_device can also return `offset_mapping` (HF's return_offsets_map
 `truncation=` also takes HF's pair strategies "longest_first", "only_first" and "only_second" (fixed layout).
 `qa_labels` / `qa_best_spans` turn those planes into extractive-QA training labels and read a QA model's
 start / end logits back into answer spans, on the GPU.  `mlm_mask` turns any fixed-layout id plane into masked-language-model
-inputs and labels (token or whole-word masking), on the GPU.
+inputs and labels (token or whole-word masking), on the GPU.  `bpe_dropout=p` on encode_batch / encode_device (and `dropout=p` on
+`bpe`) skips every merge with probability p (BPE-dropout), a different segmentation per seed, on the GPU.
 """
 import ctypes as C
 import operator
@@ -45,6 +46,22 @@ def _strategy_flag(truncation, max_len, padding=True, return_offset=False):
     if return_offset:
         raise ValueError("truncation=%r is not available with return_offset=True" % truncation)
     return _STRATEGIES[truncation]
+
+
+def _dropout_args(bpe_dropout, seed, max_len, padding=True, truncation=True, return_offset=False, return_offsets_mapping=False):
+    """(p, seed as uint64) of a BPE-dropout encode, after the checks of the fixed layout it needs."""
+    p = float(bpe_dropout)
+    if not 0.0 <= p <= 1.0:
+        raise ValueError("bpe_dropout must be in [0, 1] (got %r)" % bpe_dropout)
+    if max_len is None or max_len < 4:
+        raise ValueError("bpe_dropout needs max_len >= 4 (got %r)" % (max_len,))
+    if not padding:
+        raise ValueError("bpe_dropout needs padding=True (the fixed layout)")
+    if truncation is not True:
+        raise ValueError("bpe_dropout needs truncation=True (the reference cut; got %r)" % (truncation,))
+    if return_offset or return_offsets_mapping:
+        raise ValueError("bpe_dropout is not available with return_offset / return_offsets_mapping")
+    return p, operator.index(seed) & (2 ** 64 - 1)
 
 
 def pack_strings(strs):
@@ -264,8 +281,9 @@ class Tokenize(object):
         self._open()
 
     # ---- single-call surface ---------------------------------------------------------------------------
-    def bpe(self, token):
-        """tokenize.py:62-101 -- the merge loop runs on the device; pieces are cut from `token` by code point."""
+    def bpe(self, token, dropout=None, seed=0, key=0):
+        """tokenize.py:62-101 -- the merge loop runs on the device; pieces are cut from `token` by code point.  dropout=p: the
+        BPE-dropout segmentation (include/genztok.h) of `token` as the first word of a row with row key `key`, encoded with `seed`."""
         if not isinstance(token, str):
             token = "".join(token)
         if len(token) == 0:
@@ -274,7 +292,13 @@ class Tokenize(object):
         cap = len(token) + 1
         pieces = (C.c_int32 * cap)()
         n = C.c_int64()
-        rc = self._lib.genztok_bpe_word(self._h, w, len(w), pieces, cap, C.byref(n))
+        if dropout is None:
+            rc = self._lib.genztok_bpe_word(self._h, w, len(w), pieces, cap, C.byref(n))
+        else:
+            p = float(dropout)
+            if not 0.0 <= p <= 1.0:
+                raise ValueError("dropout must be in [0, 1] (got %r)" % dropout)
+            rc = self._lib.genztok_bpe_word_dropout(self._h, w, len(w), p, operator.index(seed) & (2 ** 64 - 1), operator.index(key), pieces, cap, C.byref(n))
         if rc:
             self._err(rc, "genztok_bpe_word")
         out, pos = [], 0
@@ -482,7 +506,7 @@ class Tokenize(object):
 
     # ---- batch extensions -------------------------------------------------------------------------------
     def encode_batch(self, texts, pair_texts=None, max_len=None, padding=True, truncation=True, token_type_ids=True,
-                     sequence_id=True, return_offset=False, return_offsets_mapping=False):
+                     sequence_id=True, return_offset=False, return_offsets_mapping=False, bpe_dropout=None, seed=0, row_keys=None):
         """Encode n documents (or n pairs) in one call.  `texts` / `pair_texts`: list[str] or the packed
         form (uint8 bytes, int64 offsets[n+1]).  Returns a BatchEncoding of numpy arrays over pinned memory.
         return_offsets_mapping: also 'offset_mapping', int32 [n, max_len, 2] (fixed layout) or [total, 2] (ragged): the
@@ -493,13 +517,45 @@ class Tokenize(object):
         HF's "longest_first" (the Rust tokenizers' rule), "only_first" or "only_second": each text keeps a prefix so that the
         row fits max_len.  A pair that only_first / only_second cannot truncate gets row_status 2 and the True row on every
         plane; row(i) raises ValueError for it.  The strategies need max_len >= 4, padding=True and return_offset=False;
-        include/genztok.h states the rule."""
+        include/genztok.h states the rule.
+        bpe_dropout: None (the default) is the reference's BPE.  A probability p (0.0 included) takes the BPE-dropout path: every
+        merge is skipped with probability p, drawn from (seed, row key, word, round, position) as include/genztok.h states, with
+        row i's key row_keys[i] (int64 [n]) or i.  Same seed and keys, same rows; p = 0 gives the bpe_dropout=None rows.  It needs
+        the fixed layout: max_len >= 4, padding=True, truncation=True, no return_offset / return_offsets_mapping."""
         flags = L.WANT_OFFSETS if return_offsets_mapping else 0
         if pair_texts is not None:
             flags |= (L.WANT_TOKEN_TYPE if token_type_ids else 0) | (L.WANT_SEQUENCE_ID if sequence_id else 0)
         if max_len is not None:
             max_len = operator.index(max_len)
+        if bpe_dropout is not None:
+            p, seed = _dropout_args(bpe_dropout, seed, max_len, padding, truncation, return_offset, return_offsets_mapping)
+            return self._encode_dropout(texts, pair_texts, max_len, flags, p, seed, row_keys)
         return self._encode_raw(texts, pair_texts, max_len, padding, truncation, flags, return_offset)
+
+    def _encode_dropout(self, texts, pairs, max_len, flags, p, seed, row_keys):
+        tb, to = texts if isinstance(texts, tuple) else pack_strings(texts)
+        n = len(to) - 1
+        pbp = pop = None
+        if pairs is not None:
+            pb, po = pairs if isinstance(pairs, tuple) else pack_strings(pairs)
+            if len(po) - 1 != n:
+                raise ValueError("texts and pair_texts differ in length")
+            pb, po = np.ascontiguousarray(pb, dtype=np.uint8), np.ascontiguousarray(po, dtype=np.int64)
+            pbp, pop = pb.ctypes.data, po.ctypes.data
+        keys = None
+        if row_keys is not None:
+            keys = np.ascontiguousarray(np.asarray(row_keys, dtype=np.int64))
+            if keys.shape != (n,):
+                raise ValueError("row_keys must have shape (%d,) (got %s)" % (n, keys.shape))
+        if max_len >= 2 ** 31:
+            raise OverflowError("max_len out of range")
+        tb, to = np.ascontiguousarray(tb, dtype=np.uint8), np.ascontiguousarray(to, dtype=np.int64)
+        enc = L.Encoded()
+        rc = self._lib.genztok_encode_dropout(self._h, tb.ctypes.data, to.ctypes.data, pbp, pop, n, int(max_len), flags, p, seed,
+                                              keys.ctypes.data if keys is not None else None, C.byref(enc))
+        if rc:
+            self._err(rc, "genztok_encode_dropout")
+        return self._wrap(enc, n, True, _EncodedOwner(self, enc))
 
     @staticmethod
     def _window_args(max_len, stride):
@@ -625,18 +681,32 @@ class Tokenize(object):
         return [raw[off[i]:off[i + 1]].decode("utf-8", "surrogatepass") for i in range(n)]
 
     def encode_device(self, d_text, d_text_off, d_pair=None, d_pair_off=None, max_len=128, token_type_ids=True, sequence_id=False,
-                      out=None, text_bytes=None, pair_bytes=None, truncation=True):
+                      out=None, text_bytes=None, pair_bytes=None, truncation=True, bpe_dropout=None, seed=0, row_keys=None):
         """Fixed-layout encode with everything resident on the GPU.  Inputs are torch CUDA tensors (uint8 bytes whose
         storage is 16-byte aligned and int64 offsets[n+1]); outputs are torch tensors (DLPack-exportable) on the same
         device, written on torch's current stream.  Nothing crosses PCIe and the call does not synchronise.
         truncation: True (the reference cut) or a pair strategy as in encode_batch; with a strategy and pairs the call
-        synchronises once per text to size the token streams, and row_status 2 marks the rows the strategy cannot truncate."""
+        synchronises once per text to size the token streams, and row_status 2 marks the rows the strategy cannot truncate.
+        bpe_dropout, seed, row_keys: BPE-dropout as in encode_batch.  With row_keys None or an int64 CUDA tensor [n] on the input's
+        device the call does not synchronise; row_keys in host memory (a numpy array, a list, a CPU tensor) is first copied to the
+        device with a blocking copy."""
         import torch
         if not isinstance(truncation, str) and not truncation:
             raise ValueError("encode_device always truncates (the fixed layout): truncation must be True or a strategy name")
-        strategy = _strategy_flag(truncation, max_len)
+        drop = None
+        if bpe_dropout is not None:
+            drop = _dropout_args(bpe_dropout, seed, max_len, True, truncation)
+            strategy = 0
+        else:
+            strategy = _strategy_flag(truncation, max_len)
         n = d_text_off.numel() - 1
         dev = d_text.device
+        keys = None
+        if drop is not None and row_keys is not None:
+            keys = row_keys if isinstance(row_keys, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(np.asarray(row_keys, dtype=np.int64)))
+            if tuple(keys.shape) != (n,):
+                raise ValueError("row_keys must have shape (%d,) (got %s)" % (n, tuple(keys.shape)))
+            keys = keys.to(dev, torch.int64).contiguous()
         has_pair = d_pair_off is not None
         if out is None:
             out = {"input_ids": torch.empty((n, max_len), dtype=torch.int32, device=dev),
@@ -658,6 +728,14 @@ class Tokenize(object):
         tbytes = d_text.numel() if text_bytes is None else text_bytes
         pbytes = (d_pair.numel() if pair_bytes is None else pair_bytes) if has_pair else 0
         slot = 0
+        if drop is not None:
+            rc = self._lib.genztok_encode_dropout_device(self._h, slot, d_text.data_ptr(), d_text_off.data_ptr(), tbytes,
+                                                         d_pair.data_ptr() if has_pair else None, d_pair_off.data_ptr() if has_pair else None,
+                                                         pbytes, n, int(max_len), flags, drop[0], drop[1], keys.data_ptr() if keys is not None else None,
+                                                         C.byref(P), self._torch_stream(dev))
+            if rc:
+                self._err(rc, "genztok_encode_dropout_device")
+            return out
         rc = self._lib.genztok_encode_device(self._h, slot, d_text.data_ptr(), d_text_off.data_ptr(), tbytes,
                                              d_pair.data_ptr() if has_pair else None, d_pair_off.data_ptr() if has_pair else None, pbytes,
                                              n, int(max_len), flags, C.byref(P), self._torch_stream(dev))

@@ -360,6 +360,46 @@ int genztok_mlm_mask_device(genztok_t *h, int dev, const int32_t *d_ids, int64_t
                             double mlm_probability, double mask_replace_prob, double random_replace_prob,
                             int whole_word, int32_t *d_masked_ids, int64_t *d_labels, void *stream);
 
+/* ---- BPE-dropout (Provilkov et al., 2020): a different segmentation of the same text on every epoch --------------------
+ * Fixed-layout rows (padding, the reference cut, max_len >= 4) as genztok_encode gives them, except that every merge may be skipped.
+ * Words are split as always: the \S+\n? matches of tokenize.py:106 (the 29 whitespace code points of Python's \s), each starting
+ * from bpe()'s initial symbols (its code points, "</w>" on the last).  The merge loop is subword-nmt's encode() with dropout:
+ *  1. in round t (from 0), the pair at position i (from 0) of the current symbol sequence is dropped when its draw says so;
+ *  2. if no pair that is in bpe_ranks survives, the word is final (a round that drops every candidate ends the word; it is not
+ *     retried);
+ *  3. else the surviving pair with the lowest rank is merged at its surviving occurrences, left to right, an occurrence that overlaps
+ *     one merged before it in the round being skipped (x x x -> xx x); dropped occurrences of that pair stay unmerged;
+ *  4. until one symbol is left.  Pieces map to ids as always (S + "@@" / S[:-4], unk when the vocab lacks the piece).
+ * With p = 0 this is bpe(): the rows are bit-identical to genztok_encode's on every plane.  With p = 1 every word is its code points,
+ * which are unk unless the vocab holds each code point with and without "@@".  HF tokenizers' BPE(dropout=p) puts dropped merges
+ * back after the next successful merge and so gives other segmentations.
+ * Draws, mod 2^64, with mix64 the splitmix64 finaliser, GOLD = 0x9E3779B97F4A7C15 and K = 0x6270655F64726F70 ("bpe_drop"):
+ *    s0 = mix64(seed ^ K);  R = mix64(s0 + key * GOLD);  W_j = mix64(R + (2 j + side + 1) * GOLD);
+ *    pair (t, i) of word j is dropped  <=>  (mix64(W_j + (t << 32 | i)) >> 32) < floor(p * 2^32)  (computed in double; p = 1 drops all)
+ * with key = row_keys[r] (NULL: the row's index in the whole call), j the index of the word among its text's \S+\n? matches and
+ * side 0 for the text, 1 for the second text.  The rows are a pure function of (seed, key, text): they do not depend on chunking,
+ * sharding over the handle's devices, batch order (with keys that follow the documents) or the word cache, which is neither read
+ * nor written.  A text's words are merged only until it has max_len ids: the reference cut shows no more of it.
+ * Checks, before the device slot (GENZTOK_E_INVALID): n >= 0, p in [0, 1] (not NaN), max_len >= 4, and flags among
+ * GENZTOK_WANT_TOKEN_TYPE | GENZTOK_WANT_SEQUENCE_ID (offsets, spans and the pair truncation strategies are not available).
+ * genztok_encode_dropout: host buffers, results as genztok_encode's fixed layout (free with genztok_free_encoded), chunked and
+ * sharded as genztok_encode.  genztok_encode_dropout_device: everything on device `dev`, asynchronous on `stream` with no host read
+ * (planes: input_ids, attention_mask and row_len required; pairs also write seq_len / row_status when given); its work buffers grow
+ * (cudaMalloc / cudaFree) only on a call larger than every earlier one on the device.  Both use n * (max_len + 2) * 4 bytes per side
+ * of device memory for the capped token streams and 8 bytes per text byte of scratch for long words (released by genztok_destroy).
+ * A document whose offsets do not lie inside its side's bytes is counted by genztok_check_errors (the host form fails with
+ * GENZTOK_E_CUDA) and gets no ids.
+ * genztok_bpe_word_dropout: genztok_bpe_word under dropout, the segmentation of word 0, side 0 of a row with key `key`. */
+int genztok_encode_dropout(genztok_t *h, const uint8_t *text, const int64_t *text_off, const uint8_t *pair, const int64_t *pair_off, int64_t n,
+                           int32_t max_len, uint32_t flags, double p, uint64_t seed, const int64_t *row_keys /* [n] or NULL */,
+                           genztok_encoded_t *out);
+int genztok_encode_dropout_device(genztok_t *h, int dev, const uint8_t *d_text, const int64_t *d_text_off, int64_t text_bytes,
+                                  const uint8_t *d_pair, const int64_t *d_pair_off, int64_t pair_bytes, int64_t n, int32_t max_len,
+                                  uint32_t flags, double p, uint64_t seed, const int64_t *d_row_keys /* [n] or NULL */,
+                                  const genztok_dev_planes_t *planes, void *stream);
+int genztok_bpe_word_dropout(genztok_t *h, const uint8_t *word, int64_t word_len, double p, uint64_t seed, int64_t key,
+                             int32_t *piece_cp, int64_t cap, int64_t *n_pieces);
+
 /* ---- measurement plumbing (not part of the reference's surface; used by bench.py and the tests) ------------------- */
 /* The synthetic workload of SURVEY.md 8 d2 produced on the device: the counter-based generator that
  * genz_tokenize_b200/workload.py::generate_hashed defines (same bytes).  genztok_synth_init uploads the word list
